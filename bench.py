@@ -19,6 +19,10 @@ streams far more than the 126 MB L2.
 
 ``--impl reference`` times only that CPU implementation (all host threads) and prints the same line
 with "impl": "reference".
+
+``--dump-outputs DIR`` writes what the last timed step computed (rank 0's results for a seeded sample of
+its streams, and the lock/bit counters) as float32 / float64 .npy files, so that two builds run with the
+same arguments can be compared output for output (see dump_outputs).
 """
 from __future__ import annotations
 
@@ -242,6 +246,35 @@ def run_reference_arm(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+DUMP_RESULT_BUDGET = 48 << 20             # bytes of sampled per-call results; the whole dump stays under 64 MB
+DUMP_MAX_STREAMS = 16384
+
+
+def dump_outputs(out_dir, d_res, counters, n_frames, seed):
+    """The timed step's outputs as .npy: for a fixed sample of streams (chosen by --seed; every stream when the
+    bank is small enough) each field of the sc_frame_result records the step returned, plus the 16 lock/bit
+    counters.  Integer fields are stored as float32 (all exact); the 62 packed bits as two float64 halves
+    (bits 0-31 and 32-61) so that they stay exact; the counters as float64."""
+    import singlecarrier_b200 as sc
+    import torch
+    streams = d_res.shape[0]
+    per_stream = n_frames * (7 * 4 + 2 * 8)
+    k = max(1, min(streams, DUMP_MAX_STREAMS, DUMP_RESULT_BUDGET // per_stream))
+    idx = np.sort(np.random.default_rng(seed).choice(streams, k, replace=False))
+    rows = d_res[torch.from_numpy(idx).to(d_res.device)].cpu().numpy()
+    res = np.ascontiguousarray(rows).view(sc.RESULT_DTYPE).reshape(k, n_frames)
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"results_stream_index": idx.astype(np.float64)}
+    for name in ("valid", "max_index", "matches", "rx_timing", "call_index", "max_value", "cost"):
+        out["results_" + name] = res[name].astype(np.float32)
+    bits = res["bits"].astype(np.uint64)
+    out["results_bits_lo32"] = (bits & np.uint64(0xFFFFFFFF)).astype(np.float64)
+    out["results_bits_hi32"] = (bits >> np.uint64(32)).astype(np.float64)
+    out["lock_stats"] = counters.cpu().numpy().astype(np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def workload_config(args, streams_override=None):
     return {
         "workload": "BASELINE.json configs[3] per-GPU shard: 131072 streams/GPU x 10 s (1M streams on 8 GPUs), "
@@ -268,7 +301,12 @@ def main():
     ap.add_argument("--slab-parts", type=int, default=0, help="override the library's slab split (0 = default)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR as .npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     if args.slab_parts > 0:
@@ -347,6 +385,8 @@ def main():
     sym_per_step = world * streams * n_frames * SYM_PER_FRAME
     value = sym_per_step * args.steps / (ms_total * 1e-3) / 1e6
     stats = counters.cpu().numpy().tolist()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_res, counters, n_frames, args.seed)      # before the passes below reuse d_res
 
     # ---- roofline: per-kernel durations with events on the launching stream, one slab ----------------
     hbm_peak, sm_max, peak_src = peaks()
@@ -453,7 +493,7 @@ def run_small_bank(args, sc, torch, dev, n_frames, streams=1024):
     library's default for this size (the even and the odd calls as two overlapped chains, lane-cooperative training
     kernel) beside the serial call-by-call chain the large bank uses.  Same results either way (tests)."""
     from singlecarrier_b200.modem import OPT_OVERLAP, OPT_TRACKER, OVERLAP_OFF, TRACKER_THREAD
-    out = {"streams": streams, "unit": UNIT, "calls_per_step": n_frames,
+    out = {"streams": streams, "unit": UNIT, "calls_per_step": n_frames, "steps": args.steps,
            "workload": "BASELINE.json configs[1]: 1,024 loop-back streams, random offset/phase, one bank on one GPU"}
     res = torch.empty((streams, n_frames * 32), dtype=torch.uint8, device=dev)
     for name, serial in (("value", False), ("serial_chain_value", True)):
@@ -462,18 +502,18 @@ def run_small_bank(args, sc, torch, dev, n_frames, streams=1024):
             bank.set_option(OPT_OVERLAP, OVERLAP_OFF)
             bank.set_option(OPT_TRACKER, TRACKER_THREAD)
         d_in = synth_input(sc, torch, bank, streams, args.seconds * 8000, args.seed + 1, 0)
-        for _ in range(3):
+        for _ in range(args.warmup):
             bank.reset()
             bank.rx_frames_dev(d_in, n_frames, res)
         torch.cuda.synchronize(dev)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(10):
+        for _ in range(args.steps):
             bank.reset()
             bank.rx_frames_dev(d_in, n_frames, res)
         e1.record()
         torch.cuda.synchronize(dev)
-        ms = e0.elapsed_time(e1) / 10
+        ms = e0.elapsed_time(e1) / args.steps
         out[name] = streams * n_frames * SYM_PER_FRAME / (ms * 1e-3) / 1e6
         out["us_per_call" if not serial else "serial_chain_us_per_call"] = 1e3 * ms / n_frames
         bank.close()
@@ -545,7 +585,7 @@ def run_e2e(args, sc, torch, dist, bank, d_in, streams, n_frames, world, rank, d
         trial[mode] = timed(2)
     best = min(trial, key=lambda m: trial[m])
     ebank.set_option(OPT_H2D_MODE, best)
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     h0, o0 = ebank.transfer_bytes()
     dt = timed(steps)
     h1, o1 = ebank.transfer_bytes()

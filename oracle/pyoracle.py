@@ -13,6 +13,7 @@ Two libraries:
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
 import os
 import subprocess
 
@@ -305,6 +306,101 @@ class Reference:
 
     def global_f32(self, name: str) -> C.c_float:
         return C.c_float.in_dll(self.lib, name)
+
+
+REF_REPLAY = os.path.join(os.path.dirname(HERE), "tests", "golden", "ref_replay.npz")
+
+
+def _digest(a) -> str:
+    return hashlib.sha1(np.ascontiguousarray(a).tobytes()).hexdigest()[:16]
+
+
+class RecordingReference:
+    """Wraps an engine with the Reference interface and records every output under a key made of the call and a
+    digest of its input (the key RecordedReference looks up); ``save()`` writes them (tools/make_golden.py)."""
+
+    def __init__(self, engine):
+        self.engine, self.out, self.n = engine, {}, 0
+
+    def _put(self, key, **arrays):
+        for k, v in arrays.items():
+            self.out[f"{key}/{k}"] = np.asarray(v)
+
+    def reset(self, wide: bool = False):
+        self.engine.reset(wide)
+        self.n = 0
+
+    def run_stream(self, samples, wide: bool = False):
+        bits, st = self.engine.run_stream(samples, wide)
+        self._put(f"run_stream/{_digest(samples)}/{int(wide)}", bits=bits, stats=st)
+        return bits, st
+
+    def rx_frame(self, frame):
+        bits, st = self.engine.rx_frame(frame)
+        self._put(f"rx_frame/{self.n}/{_digest(frame)}", bits=bits, stats=st, filtered=self.engine.filtered(),
+                  decimated=self.engine.decimated())
+        self.n += 1
+        return bits, st
+
+    def tx_preamble(self):
+        out = self.engine.tx_preamble()
+        self._put(f"tx_preamble/{self.n}", out=out)
+        self.n += 1
+        return out
+
+    def tx_data(self, bits):
+        out = self.engine.tx_data(bits)
+        self._put(f"tx_data/{self.n}/{_digest(np.ascontiguousarray(bits, np.uint8))}", out=out)
+        self.n += 1
+        return out
+
+    def save(self, path: str = REF_REPLAY, **meta):
+        np.savez_compressed(path, **self.out, **{f"meta/{k}": np.asarray(v) for k, v in meta.items()})
+
+
+class RecordedReference:
+    """The reference's outputs replayed from tests/golden/ref_replay.npz, for machines without oracle/_ref: the same
+    calls as Reference, answered from what the reference returned for the same input (and, for the stateful
+    calls, the same position since reset()).  An input that was not recorded is an error, never a skip."""
+
+    def __init__(self, path: str = REF_REPLAY):
+        self.g = dict(np.load(path))
+        self.n = 0
+        self._last = None
+
+    def _get(self, key):
+        if f"{key}/bits" not in self.g and f"{key}/out" not in self.g:
+            raise KeyError(f"no recorded reference output for {key} in {os.path.basename(REF_REPLAY)} "
+                           "(inputs changed? re-record with tools/make_golden.py)")
+        return key
+
+    def reset(self, wide: bool = False):
+        self.n = 0
+
+    def run_stream(self, samples, wide: bool = False):
+        k = self._get(f"run_stream/{_digest(samples)}/{int(wide)}")
+        return self.g[k + "/bits"].copy(), self.g[k + "/stats"].copy()
+
+    def rx_frame(self, frame):
+        k = self._last = self._get(f"rx_frame/{self.n}/{_digest(frame)}")
+        self.n += 1
+        return self.g[k + "/bits"].copy(), self.g[k + "/stats"].copy()
+
+    def filtered(self, n: int = FRAME_SIZE) -> np.ndarray:
+        return self.g[self._last + "/filtered"][:n].copy()
+
+    def decimated(self, n: int = 752) -> np.ndarray:
+        return self.g[self._last + "/decimated"][:n].copy()
+
+    def tx_preamble(self) -> np.ndarray:
+        k = self._get(f"tx_preamble/{self.n}")
+        self.n += 1
+        return self.g[k + "/out"].copy()
+
+    def tx_data(self, bits: np.ndarray) -> np.ndarray:
+        k = self._get(f"tx_data/{self.n}/{_digest(np.ascontiguousarray(bits, np.uint8))}")
+        self.n += 1
+        return self.g[k + "/out"].copy()
 
 
 def synth_bench_stream(oracle, seed: int, stream_id: int, n_samples: int) -> np.ndarray:

@@ -4,6 +4,7 @@ import ctypes as C
 import os
 import re
 import subprocess
+import sys
 
 import pytest
 
@@ -51,10 +52,9 @@ def test_compat_headers_compile_as_c_and_cxx(tmp_path):
                     "-o", str(tmp_path / "t2.o")], check=True)
 
 
-def test_fails_loudly_without_a_gpu():
+def fails_loudly_without_a_gpu():
     import torch
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
+    assert not torch.cuda.is_available()
     import singlecarrier_b200 as sc
     assert sc.lib.sc_device_count() == 0
     with pytest.raises(sc.SingleCarrierError) as e:
@@ -64,8 +64,18 @@ def test_fails_loudly_without_a_gpu():
     assert sc.lib.sc_fir_batch_dev(0, 1, 0, 1, 1, 1, 1, None) == -2
     code = ("import ctypes,singlecarrier_b200 as sc; m=(ctypes.c_float*98)(); x=(ctypes.c_float*16)();"
             "sc.lib.fir(m, False, x, 8)")
-    r = subprocess.run(["python", "-c", code], cwd=ROOT, capture_output=True, text=True)
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, capture_output=True, text=True)
     assert r.returncode != 0 and "no CUDA device" in r.stderr
+
+
+def test_fails_loudly_without_a_gpu():
+    """The checks above in a child process that sees no device (CUDA_VISIBLE_DEVICES empty), so that they run on
+    machines with a GPU as well."""
+    code = (f"import sys; sys.path[:0] = [{ROOT!r}, {os.path.join(ROOT, 'tests')!r}]; "
+            "import test_abi; test_abi.fails_loudly_without_a_gpu()")
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-3000:]
 
 
 def test_host_helpers_need_no_gpu():

@@ -3,6 +3,7 @@ include/sc_compat and linked with libsinglecarrier_b200.so, must print what the 
 import ctypes as C
 import os
 import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -114,14 +115,18 @@ def test_interleaved_globals_match_reference(ref):
     """qpsk_rx_frame() shares RXMemory with scramble()/scramble_init()/data_eq() and leaves eq_coeff,
     kalman_gain, kalman_y and the internal u/d behind (src/scramble.c:41-42, src/equalizer.c:87,
     src/kalman.c:19-35): a caller that interleaves them sees exactly what the reference's objects give."""
-    import sys
     from oracle import pyoracle as po
     raw = os.path.join(ROOT, "tests", "golden", "preamble_qpsk_8k.raw")
     drv = os.path.join(ROOT, "tests", "dropin_interleave.py")
     ours = os.path.join(ROOT, "singlecarrier_b200", "libsinglecarrier_b200.so")
-    a = subprocess.run([sys.executable, drv, po.REF_SO, raw, "ref"], check=True, capture_output=True, text=True, timeout=300)
+    if po.have_ref():
+        a = subprocess.run([sys.executable, drv, po.REF_SO, raw, "ref"], check=True, capture_output=True, text=True,
+                           timeout=300)
+        la = a.stdout.strip().splitlines()
+    else:                                                                    # the reference's lines, recorded
+        la = open(os.path.join(ROOT, "tests", "golden", "dropin_interleave_ref.jsonl")).read().strip().splitlines()
     b = subprocess.run([sys.executable, drv, ours, raw, "ours"], check=True, capture_output=True, text=True, timeout=300)
-    la, lb = a.stdout.strip().splitlines(), b.stdout.strip().splitlines()
+    lb = b.stdout.strip().splitlines()
     assert len(la) == len(lb) == 14 + 4
     for x, y in zip(la, lb):
         assert x == y
@@ -150,7 +155,7 @@ def test_legacy_tx_frame_arbitrary_symbols(oracle):
         "np.concatenate(out).tofile(sys.argv[1])" % ROOT)
     import tempfile
     path = tempfile.mktemp(suffix=".i16")
-    subprocess.run(["python", "-c", code, path], check=True, cwd=ROOT, timeout=300)
+    subprocess.run([sys.executable, "-c", code, path], check=True, cwd=ROOT, timeout=300)
     got = np.fromfile(path, np.int16)
     os.unlink(path)
     want = []

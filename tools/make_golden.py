@@ -1,9 +1,9 @@
 #!/usr/bin/env python
 """Generate the committed golden vectors under tests/golden/ from the REFERENCE's own object code.
 
-Runs only in the build container (needs /root/reference, compiled by oracle/Makefile into
-oracle/_ref/libsc_ref.so).  The fixtures let the oracle restatement -- and through it the CUDA path
--- be pinned on boxes where the reference does not exist.  Re-run: ``python tools/make_golden.py``.
+Needs the reference's sources, compiled by oracle/Makefile into oracle/_ref/libsc_ref.so.  The fixtures let
+the oracle restatement -- and through it the CUDA path -- be pinned on machines where the reference does not
+exist.  Re-run: ``python tools/make_golden.py``.
 
 Fixtures
   preamble_qpsk_8k.raw   the reference's shipped sample file (data, copied verbatim; SURVEY section 2)
@@ -12,10 +12,22 @@ Fixtures
   tx_golden.npz          reference TX output for seeded bits (3 packets)
   stage_golden.npz       fir(), train_eq()/data_eq() trajectories, scrambler keystream
   fft_golden.npz         fft()/encode_fftr()/encode_fftri() outputs of src/fft.c
+  ref_replay.npz         what the reference returned to the tests that compare with it directly
+                         (tests/test_oracle_vs_ref.py, test_round2_gpu.py::test_cuda_path_vs_reference_objects_directly),
+                         keyed by call and input digest; replayed by pyoracle.RecordedReference where oracle/_ref is absent
+  dropin_interleave_ref.jsonl  tests/dropin_interleave.py's lines on the reference's objects
+
+``python tools/make_golden.py --replay-from-restatement`` writes only the last two where the reference is not
+available: ref_replay.npz from the oracle restatement (bit-identical to the reference on these inputs wherever
+both ran, tests/test_oracle_vs_ref.py) and the drop-in lines from libsinglecarrier_b200.so (equal to the
+reference's line for line, test_dropin_gpu.py::test_interleaved_globals_match_reference; needs a GPU).  The
+committed files were made this way; ref_replay.npz names its source in "meta/source".  A run with the
+reference overwrites both.
 """
 import ctypes as C
 import os
 import shutil
+import subprocess
 import sys
 
 import numpy as np
@@ -53,9 +65,91 @@ def synth_stream(R, rng, n_packets, lead, gap, noise, total):
     return x, np.array(allbits)
 
 
+class RestatementAsReference:
+    """The oracle restatement behind the Reference interface (stats with the reference's "mean" field)."""
+
+    def __init__(self):
+        self.o = po.Oracle()
+        self.reset()
+
+    def reset(self, wide=False):
+        self.st = self.o.new_state(wide)
+
+    def _stats(self, s):
+        out = np.zeros(s.shape, po.REF_STATS_DTYPE)
+        for f in ("valid", "max_index", "matches", "rx_timing", "max_value", "eq_coeff"):
+            out[f] = s[f]
+        out["mean"] = s["cost"]
+        return out
+
+    def run_stream(self, x, wide=False):
+        bits, s = self.o.run_stream(x, wide=wide)
+        return bits, self._stats(s)
+
+    def rx_frame(self, frame):
+        bits, s = self.o.rx_frame(self.st, frame)
+        return bits, self._stats(np.array([s]))[0]
+
+    def filtered(self, n=po.FRAME_SIZE):
+        return np.frombuffer(self.st, np.float32, count=2 * 3760).view(np.complex64)[:n].copy()
+
+    def decimated(self, n=752):
+        return np.frombuffer(self.st, np.float32, count=2 * 752, offset=3760 * 8).view(np.complex64)[:n].copy()
+
+    def tx_preamble(self):
+        return self.o.tx_preamble(self.st)
+
+    def tx_data(self, bits):
+        return self.o.tx_data(self.st, bits)
+
+
+def record_ref_replay(engine, source):
+    """The reference calls of the tests that compare with it directly, on their seeded inputs (kept in step with
+    the tests: an input that differs is not found at replay and fails the test)."""
+    o = po.Oracle()
+    R = po.RecordingReference(engine)
+    rng = np.random.default_rng(99)                                # test_oracle_vs_ref.py::test_rx_random_streams
+    samples = po.synth_streams(o, rng, 24, 10)
+    noise = [rng.integers(-a, a + 1, 1880 * 8).astype(np.int16) for a in (3, 100, 3000, 32767)]
+    for x in list(samples) + noise:
+        R.run_stream(x)
+    x = po.synth_streams(o, np.random.default_rng(5), 3, 8)        # ::test_wide_filter
+    for s in range(3):
+        R.run_stream(x[s], wide=True)
+    x = po.synth_streams(o, np.random.default_rng(6), 1, 6)[0]     # ::test_stage_taps_filtered_and_decimated
+    R.reset()
+    for n in range(6):
+        R.rx_frame(x[n * 1880:(n + 1) * 1880])
+    rng = np.random.default_rng(7)                                 # ::test_tx_random
+    R.reset()
+    for _ in range(5):
+        R.tx_preamble()
+        for _ in range(8):
+            R.tx_data(rng.integers(0, 2, 62).astype(np.uint8))
+    shipped = np.fromfile(os.path.join(GOLD, "preamble_qpsk_8k.raw"), dtype="<i2")[: 14 * 1880]
+    noisy = po.synth_streams(o, np.random.default_rng(2024), 64, 14)   # test_round2_gpu.py::test_cuda_path_vs_...
+    for x in [shipped] + list(noisy):
+        R.run_stream(x)
+    R.save(source=source)
+
+
+def interleave_lines(lib, kind):
+    raw = os.path.join(GOLD, "preamble_qpsk_8k.raw")
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "dropin_interleave.py"), lib, raw, kind],
+                         check=True, capture_output=True, text=True).stdout
+    with open(os.path.join(GOLD, "dropin_interleave_ref.jsonl"), "w") as f:
+        f.write(out)
+
+
+def replay_from_restatement():
+    po.build(quiet=False)
+    record_ref_replay(RestatementAsReference(), "oracle restatement (oracle/sc_oracle.c)")
+    interleave_lines(os.path.join(ROOT, "singlecarrier_b200", "libsinglecarrier_b200.so"), "ours")
+
+
 def main():
     po.build(quiet=False)
-    assert po.have_ref(), "needs /root/reference"
+    assert po.have_ref(), "needs the reference's objects (oracle/_ref/libsc_ref.so)"
     R = po.Reference()
     os.makedirs(GOLD, exist_ok=True)
     shutil.copyfile(REF_RAW, os.path.join(GOLD, "preamble_qpsk_8k.raw"))
@@ -147,9 +241,11 @@ def main():
         L.encode_fftri(ci, spec.ctypes.data, back.ctypes.data)
         f[f"r{n}_in"], f[f"r{n}_spec"], f[f"r{n}_back"] = xr, spec, back
     np.savez_compressed(os.path.join(GOLD, "fft_golden.npz"), **f)
+    record_ref_replay(R, "reference objects (oracle/_ref/libsc_ref.so)")
+    interleave_lines(po.REF_SO, "ref")
     for fn in sorted(os.listdir(GOLD)):
         print(fn, os.path.getsize(os.path.join(GOLD, fn)))
 
 
 if __name__ == "__main__":
-    main()
+    replay_from_restatement() if "--replay-from-restatement" in sys.argv[1:] else main()
