@@ -219,11 +219,18 @@ int sc_tx_packets_dev(sc_modem *m, const uint8_t *bits, uint8_t *bits_out, uint6
 
 /*
  * Channel for synthetic loop-back (BASELINE.json configs 2-5; no counterpart in the reference
- * beyond FOFFSET): same synthesis as sc_tx_packets_dev, but the analytic TX signal of stream s
- * is rotated by exp(j(2*pi*(df[s] + 0.5*drift[s]*t)*t + phi[s])) (t in seconds), optionally passed
- * through a 2-tap channel h = [1, a[s]*exp(j*theta[s])] at delay d[s] samples, and real AWGN of
- * standard deviation sigma[s] (in int16 LSB) is added before saturating to int16.  Any of the
- * per-stream parameter arrays (device pointers) may be NULL (= 0).
+ * beyond FOFFSET): same synthesis as sc_tx_packets_dev, then, in this order, on the analytic TX
+ * signal z[p] of stream s (p = output sample index, 0 at the stream's first sample, lead-in
+ * included; z = 0 in the lead-in, the dead air and the tail):
+ *   1. 2-tap channel h = [1, a[s]*exp(j*theta[s])] at delay d[s] samples:
+ *      e[p] = z[p] + a[s]*exp(j*theta[s])*z[p - d[s]];
+ *   2. rotation by exp(j(2*pi*(df[s] + 0.5*drift[s]*t)*t + phi[s])), t = p / 8000 s, i.e. the
+ *      offset is that of the receiver's oscillator and applies to both paths alike;
+ *   3. real part + real AWGN of standard deviation sigma[s] (int16 LSB), drawn from a counter-based
+ *      generator keyed by (seed, s, p), s counted over the whole bank;
+ *   4. saturation to +-32767 and rounding to nearest (ties to even).
+ * Any of the per-stream parameter arrays (device pointers) may be NULL: echo_delay then means 1,
+ * every other array 0.
  */
 typedef struct {
     const float   *df_hz;       /* frequency offset                  */
@@ -317,12 +324,14 @@ int sc_selftest_rcp_dev(int device, uint32_t lo_bits, uint32_t hi_bits, uint64_t
  * counter is preamble_frames_detected, qpsk.c:70,193).  results must hold calls 0..n_frames-1 of a cold
  * started bank.  A valid call n >= 2 found its preamble at decimated index max_index of the window taken
  * from frame n-2 with the rx_timing in force after call n-2, i.e. at sample
- * (n-2)*1880 + 5*max_index + rx_timing - 48 (two 24-sample RRC delays) of the stream; it is "aligned" when
- * that lies within 10 samples of the start of packet j = round((pos - lead_in[s]) / (1880 + gap)).  Its 62
- * decided bits are the first data frame of packet j (SURVEY F5); TX does not scramble (qpsk.c:397) and RX
- * descrambles, so bits ^ keystream(n) ^ tx_bits is the error pattern.
+ * pos = (n-2)*1880 + 5*max_index + rx_timing - 48 (two 24-sample RRC delays) of the stream; it is "aligned"
+ * when pos - lead_in[s] (lead_in NULL = 0) lies within 10 samples (inclusive) of the start
+ * j*(1880 + gap) of a transmitted packet j, 0 <= j < n_packets.  Its 62 decided bits are the first data
+ * frame of packet j (SURVEY F5); TX does not scramble (qpsk.c:397) and RX descrambles, so the low 62 bits
+ * of bits ^ keystream(n) ^ tx_bits are the error pattern.
  *   tx_bits : device, [n_streams][n_packets][8][62] bytes of 0/1 (sc_tx_*_dev's bits_out)
- *   group   : device int32[n_streams] or NULL (all streams in group 0), values 0..n_groups-1
+ *   group   : device int32[n_streams] or NULL (all streams in group 0), values 0..n_groups-1; a stream
+ *             whose group lies outside that range is not counted at all
  *   counters: device uint64[n_groups][8], ACCUMULATED into: 0 calls (n >= 2), 1 valid, 2 aligned, 3 bits
  *             compared (62 per aligned call), 4 bit errors, 5..7 reserved (0).  Plain sums. */
 int sc_ber_stats_dev(int device, const sc_frame_result *results, int64_t n_streams, int64_t result_stride,

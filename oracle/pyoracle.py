@@ -69,6 +69,8 @@ class Oracle:
         L.sco_tx_preamble.argtypes = [C.c_void_p, C.c_void_p]
         L.sco_tx_data.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
         L.sco_tx_frame.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int]
+        L.sco_tx_preamble_analytic.argtypes = [C.c_void_p, C.c_void_p]
+        L.sco_tx_data_analytic.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
         L.sco_fir.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int]
         L.sco_correlate.restype = C.c_float
         L.sco_correlate.argtypes = [C.c_void_p, C.c_int]
@@ -127,6 +129,20 @@ class Oracle:
         nsym = b.size // 2
         out = np.zeros(nsym * 5, "<i2")
         self.lib.sco_tx_data(_p(state), _p(out), _p(b), nsym)
+        return out
+
+    def tx_preamble_analytic(self, state) -> np.ndarray:
+        """tx_preamble() before the real part is taken: the scaled complex signal (complex64)."""
+        out = np.zeros(PREAMBLE_LENGTH * 5, np.complex64)
+        self.lib.sco_tx_preamble_analytic(_p(state), _p(out))
+        return out
+
+    def tx_data_analytic(self, state, bits: np.ndarray) -> np.ndarray:
+        """tx_data() before the real part is taken: the scaled complex signal (complex64)."""
+        b = np.ascontiguousarray(bits, np.uint8)
+        nsym = b.size // 2
+        out = np.zeros(nsym * 5, np.complex64)
+        self.lib.sco_tx_data_analytic(_p(state), _p(out), _p(b), nsym)
         return out
 
     # ---- stage primitives ----------------------------------------------------------------
@@ -433,6 +449,8 @@ def synth_bench_stream(oracle, seed: int, stream_id: int, n_samples: int) -> np.
     t = np.arange(n_samples) / 8000.0
     y = (xa * np.exp(1j * (2 * np.pi * df * t + phi))).real
     ebn0_db = float(stream_id % 13)
+    # bench.py's P_sig, kept so that both arms run the same workload.  The data section's true RMS is
+    # harness.DATA_RMS_LSB (7,207 LSB, not 16384 * 0.48 = 7,864), so the real Eb/N0 is the label minus 0.76 dB.
     p_sig = (16384.0 * 0.48) ** 2
     sigma = np.sqrt(p_sig * 8000.0 / (2.0 * 1600.0 * 2.0 * 10.0 ** (ebn0_db / 10.0)))
     y = y + rng.normal(0.0, sigma, n_samples)

@@ -301,46 +301,74 @@ int sco_rx_frame(sco_state *s, const int16_t in[SCO_FRAME_SIZE], uint8_t bits[SC
 }
 
 /* ------------------------------------------------------------- src/qpsk.c:278-322 */
-int sco_tx_frame(sco_state *s, int16_t samples[], const sco_c32 symbol[], int length, int preamble) {
+/* The transmitter up to the scaled complex signal, before qpsk_tx_frame() takes the real part and truncates it:
+ * out[i].r is exactly the float the reference converts to int16, out[i].i is the quadrature component. */
+int sco_tx_frame_analytic(sco_state *s, sco_c32 out[], const sco_c32 symbol[], int length, int preamble) {
     int n = length * SCO_CYCLES;
-    sco_c32 signal[n];
 
     for (int i = 0; i < length; i++) {                /* zero-stuff, :285-291 */
-        signal[i * SCO_CYCLES] = symbol[i];
-        for (int j = 1; j < SCO_CYCLES; j++) signal[i * SCO_CYCLES + j] = c32(0.0f, 0.0f);
+        out[i * SCO_CYCLES] = symbol[i];
+        for (int j = 1; j < SCO_CYCLES; j++) out[i * SCO_CYCLES + j] = c32(0.0f, 0.0f);
     }
 
-    sco_fir(s->tx_filter, s->wide, signal, n);        /* :296 */
+    sco_fir(s->tx_filter, s->wide, out, n);           /* :296 */
 
     for (int i = 0; i < n; i++) {                     /* :301-304 */
         s->tx_phase = cmul(s->tx_phase, s->tx_rect);
-        signal[i] = cmul(signal[i], s->tx_phase);
+        out[i] = cmul(out[i], s->tx_phase);
     }
     s->tx_phase = renorm(s->tx_phase);                /* :306 */
 
     float scale = preamble ? 8192.0f : 16384.0f;      /* :313-319 */
-    for (int i = 0; i < n; i++) samples[i] = (int16_t) (signal[i].r * scale);
+    for (int i = 0; i < n; i++) out[i] = c32(out[i].r * scale, out[i].i * scale);
 
     return n;
 }
 
-int sco_tx_preamble(sco_state *s, int16_t samples[]) {                    /* :327-329, :361-365 */
-    sco_c32 table[SCO_PREAMBLE_LENGTH];
+int sco_tx_frame(sco_state *s, int16_t samples[], const sco_c32 symbol[], int length, int preamble) {
+    sco_c32 signal[length * SCO_CYCLES];
+    int n = sco_tx_frame_analytic(s, signal, symbol, length, preamble);
+    for (int i = 0; i < n; i++) samples[i] = (int16_t) signal[i].r;             /* :319 */
+    return n;
+}
+
+static void preamble_symbols(sco_c32 table[SCO_PREAMBLE_LENGTH]) {               /* :361-365 */
     for (int i = 0; i < SCO_PREAMBLE_LENGTH; i++) {
         float v = (float) sco_preamblevalues[i];
         table[i] = c32(v, v);
     }
-    return sco_tx_frame(s, samples, table, SCO_PREAMBLE_LENGTH, 1);
 }
 
-int sco_tx_data(sco_state *s, int16_t samples[], const uint8_t bits[], int n_symbols) {   /* :334-342, :251-256 */
-    sco_c32 symbol[n_symbols];
+static void data_symbols(sco_c32 symbol[], const uint8_t bits[], int n_symbols) {   /* :251-256 */
     for (int i = 0; i < n_symbols; i++) {
         float vi = (bits[2 * i + 1] == 1) ? -1.0f : 1.0f;
         float vq = (bits[2 * i] == 1) ? -1.0f : 1.0f;
         symbol[i] = c32(vi, vq);
     }
+}
+
+int sco_tx_preamble(sco_state *s, int16_t samples[]) {                    /* :327-329 */
+    sco_c32 table[SCO_PREAMBLE_LENGTH];
+    preamble_symbols(table);
+    return sco_tx_frame(s, samples, table, SCO_PREAMBLE_LENGTH, 1);
+}
+
+int sco_tx_data(sco_state *s, int16_t samples[], const uint8_t bits[], int n_symbols) {   /* :334-342 */
+    sco_c32 symbol[n_symbols];
+    data_symbols(symbol, bits, n_symbols);
     return sco_tx_frame(s, samples, symbol, n_symbols, 0);
+}
+
+int sco_tx_preamble_analytic(sco_state *s, sco_c32 out[]) {
+    sco_c32 table[SCO_PREAMBLE_LENGTH];
+    preamble_symbols(table);
+    return sco_tx_frame_analytic(s, out, table, SCO_PREAMBLE_LENGTH, 1);
+}
+
+int sco_tx_data_analytic(sco_state *s, sco_c32 out[], const uint8_t bits[], int n_symbols) {
+    sco_c32 symbol[n_symbols];
+    data_symbols(symbol, bits, n_symbols);
+    return sco_tx_frame_analytic(s, out, symbol, n_symbols, 0);
 }
 
 /* ------------------------------------------------------------- src/qpsk.c:436-458 */

@@ -94,6 +94,11 @@ int  sco_rx_frame(sco_state *s, const int16_t in[SCO_FRAME_SIZE], uint8_t bits[S
 int  sco_tx_frame(sco_state *s, int16_t samples[], const sco_c32 symbol[], int length, int preamble); /* qpsk.c:278-322 */
 int  sco_tx_preamble(sco_state *s, int16_t samples[]);                    /* src/qpsk.c:327-329              */
 int  sco_tx_data(sco_state *s, int16_t samples[], const uint8_t bits[], int n_symbols);    /* qpsk.c:334-342 */
+/* the same transmitter stopped before the real part is taken: the scaled complex signal (sco_tx_frame() truncates
+ * its real part to int16, so these are pinned to the reference through the int16 outputs) */
+int  sco_tx_frame_analytic(sco_state *s, sco_c32 out[], const sco_c32 symbol[], int length, int preamble);
+int  sco_tx_preamble_analytic(sco_state *s, sco_c32 out[]);
+int  sco_tx_data_analytic(sco_state *s, sco_c32 out[], const uint8_t bits[], int n_symbols);
 
 /* whole-stream drivers (what main()'s loop does, qpsk.c:436-458) */
 void sco_run_stream(const int16_t in[], int n_frames, int wide, float foffset_hz,

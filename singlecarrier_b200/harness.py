@@ -15,10 +15,14 @@ from typing import Optional
 import numpy as np
 
 from .modem import FRAME_SIZE, REFERENCE_GAP, ModemBank, keystream_word
+from .taps import modem_taps
 
 PERIOD = FRAME_SIZE + REFERENCE_GAP          # 2783 samples: one packet + dead air (qpsk.c:384,405,410-412)
 GROUP_DELAY = 48                             # TX RRC (24) + RX RRC (24) samples
-DATA_RMS_LSB = 16384.0 * 0.48                # per-component RMS of the analytic data section (2.2 x tap energy)
+# RMS of the real TX signal over the data section, i.e. of each component of the analytic one: +-1 QPSK
+# symbols, one in five filter inputs, x 2.2 (fir.c:42) x 16384 (qpsk.c:319).  7,207 LSB for the default
+# alpha = 0.35 taps; the alpha = 0.5 taps give 7,205.
+DATA_RMS_LSB = 16384.0 * 2.2 * math.sqrt(float((modem_taps(0.35).astype(np.float64) ** 2).sum()) / 5.0)
 
 
 @dataclass
