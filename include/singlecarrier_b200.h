@@ -123,7 +123,8 @@ uint64_t sc_launch_count(void);
 #define SC_OVERLAP_MAX       32768
 int  sc_set_option(sc_modem *m, int option, int64_t value);
 int  sc_profile_read(sc_modem *m, double out[4]);
-/* bytes queued host->device (out[0]) and device->host (out[1]) by sc_rx_frames_host since sc_create */
+/* bytes queued host->device (out[0]) and device->host (out[1]) by sc_rx_frames_host / sc_rx_frames_soft_host
+ * since sc_create */
 int  sc_transfer_bytes(const sc_modem *m, uint64_t out[2]);
 /* frees the process-wide device caches (FFT twiddle / permutation tables) */
 int  sc_release_caches(void);
@@ -158,6 +159,27 @@ int sc_rx_frames_dev(sc_modem *m, const int16_t *in, int64_t stream_stride, int 
                      sc_frame_result *results, int64_t result_stride, float *eq_dbg, void *stream);
 int sc_rx_frames_host(sc_modem *m, const int16_t *in, int64_t stream_stride, int n_frames,
                       sc_frame_result *results, int64_t result_stride, float *eq_dbg);
+
+/*
+ * Soft output: the same calls, and in addition the equalizer output of every data step -- the value each
+ * decision is sliced from (data_eq(), equalizer.c:64-80), before slicing and descrambling.  Data step i
+ * (0..SC_DATA_SYMBOLS-1) of a call reads the symbol at sync_pos + i in a valid call and at rx_timing + i in an
+ * invalid one; it is written for invalid calls too.  It is computed by the same float32 operations as the decision,
+ * so bit 2i of the raw decision is (Im < 0) and bit 2i+1 is (Re < 0), and results[].bits = raw decisions XOR
+ * sc_keystream_word(call_index) (valid calls).
+ *
+ * symbols: SC_DATA_SYMBOLS complex floats (re, im interleaved) per record, record (s, j) at
+ * (s*result_stride + j) * 2*SC_DATA_SYMBOLS floats -- the same record indexing as results.  Required (NULL:
+ * SC_EINVAL); a device pointer aligned to 8 bytes for _dev, a host pointer for _host (pinned gives asynchronous
+ * copies; sc_transfer_bytes counts the copied symbol bytes).  results and the bank's state afterwards are exactly
+ * what sc_rx_frames_* would have produced, on the same schedules (SC_OPT_OVERLAP included), so soft and plain
+ * batches may alternate on one handle.  There is no eq_dbg argument.  On SC_FLAG_PACKET banks these are ordinary
+ * calls (no sc_packet_result).
+ */
+int sc_rx_frames_soft_dev(sc_modem *m, const int16_t *in, int64_t stream_stride, int n_frames,
+                          sc_frame_result *results, int64_t result_stride, float *symbols, void *stream);
+int sc_rx_frames_soft_host(sc_modem *m, const int16_t *in, int64_t stream_stride, int n_frames,
+                           sc_frame_result *results, int64_t result_stride, float *symbols);
 
 /* ---- packet mode: an EXTENSION with no counterpart in the reference ----------------------------- */
 

@@ -7,8 +7,9 @@ fir / equalizer / kalman / scramble primitives underneath), processing thousands
 and ``bench.py``.  PyTorch is used only for device memory, streams and ``torch.distributed``.
 """
 from ._lib import LIB_PATH, SingleCarrierError, lib  # noqa: F401
-from .modem import (BITS_PER_CALL, FRAME_SIZE, PACKET_DTYPE, RESULT_DTYPE, SYMBOLS_PER_FRAME, ModemBank,  # noqa: F401
-                    NcclComm, PinnedBuffer, h2d_probe, keystream_word, launch_count, unpack_bits, unpack_packet_bits)
+from .modem import (BITS_PER_CALL, DATA_SYMBOLS, FRAME_SIZE, PACKET_DTYPE, RESULT_DTYPE, SYMBOLS_PER_FRAME,  # noqa: F401
+                    ModemBank, NcclComm, PinnedBuffer, h2d_probe, keystream_word, launch_count, soft_bits, unpack_bits,
+                    unpack_packet_bits)
 
 __all__ = ["ModemBank", "NcclComm", "PinnedBuffer", "h2d_probe", "RESULT_DTYPE", "PACKET_DTYPE", "unpack_packet_bits", "FRAME_SIZE", "BITS_PER_CALL",
-           "SYMBOLS_PER_FRAME", "unpack_bits", "keystream_word", "launch_count", "SingleCarrierError", "lib", "LIB_PATH"]
+           "SYMBOLS_PER_FRAME", "DATA_SYMBOLS", "unpack_bits", "soft_bits", "keystream_word", "launch_count", "SingleCarrierError", "lib", "LIB_PATH"]

@@ -55,6 +55,8 @@ def _load() -> C.CDLL:
     sig("sc_profile_read", i32, vp, C.POINTER(C.c_double))
     sig("sc_rx_frames_dev", i32, vp, vp, i64, i32, vp, i64, vp, vp)
     sig("sc_rx_frames_host", i32, vp, vp, i64, i32, vp, i64, vp)
+    sig("sc_rx_frames_soft_dev", i32, vp, vp, i64, i32, vp, i64, vp, vp)
+    sig("sc_rx_frames_soft_host", i32, vp, vp, i64, i32, vp, i64, vp)
     sig("sc_rx_packets_dev", i32, vp, vp, i64, i32, vp, i64, vp, i64, vp, vp)
     sig("sc_rx_packets_host", i32, vp, vp, i64, i32, vp, i64, vp, i64, C.POINTER(C.c_uint64))
     sig("sc_unpack_bits", None, vp, i64, vp)

@@ -34,14 +34,16 @@ cudaError_t launch_frontend(bool wide, const int16_t *in, long stream_stride, co
 cudaError_t launch_track(bool debug_eq, const float2 *win, const int *max_index, const float *max_value,
                          const int *timing_cur, int *timing_next, sc_frame_result *results, long result_stride,
                          float *eq_dbg, float *state_dbg, uint32_t call_index, unsigned long long keystream,
-                         int n_streams, cudaStream_t st, bool coop = false);
+                         int n_streams, cudaStream_t st, bool coop = false, float *sym = nullptr);
 cudaError_t launch_track_train(const float2 *win_ov, float *state, long state_stride, int n_streams, cudaStream_t st,
                                bool coop);
 cudaError_t launch_track_data(const float2 *win_ov, float *state, long state_stride, const int *max_index,
                               const float *max_value, const int *timing_cur, int *timing_next, sc_frame_result *results,
                               long result_stride, uint32_t call_index, unsigned long long keystream, int n_streams,
-                              cudaStream_t st, bool coop, const TimingSrc *ts = nullptr, int *timing_cur_out = nullptr);
-// timing_next / timing_cur_out may be nullptr (nothing stored)
+                              cudaStream_t st, bool coop, const TimingSrc *ts = nullptr, int *timing_cur_out = nullptr,
+                              float *sym = nullptr);
+// timing_next / timing_cur_out may be nullptr (nothing stored).  sym (launch_track, launch_track_data): nullptr, or
+// the equalizer outputs of the call's 31 data steps as NDATA float2 per record, records indexed like results
 constexpr int TRACK_STATE_FLOATS = 48;   // C[5], G[5], U[10] complex, D[5], KY, 2 pad: the drop-in shim's view
 
 // sc_stage_kernels.cu

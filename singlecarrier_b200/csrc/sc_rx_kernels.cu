@@ -287,19 +287,20 @@ struct TileLoaderOv {
 };
 __device__ __forceinline__ int ov_alt_row(int rx_timing) { return X_ROWS + min(max(rx_timing - PRE, 0), PRE - 1); }
 
-template <bool DEBUG_EQ>
+// SOFT: the 31 equalizer outputs of the call also go to sym, NDATA per record, records indexed like results.
+template <bool DEBUG_EQ, bool SOFT>
 __global__ void __launch_bounds__(TK_THREADS)
 track_kernel(const float2 *__restrict__ win, const int *__restrict__ max_index, const float *__restrict__ max_value,
              const int *__restrict__ timing_cur, int *__restrict__ timing_next, sc_frame_result *__restrict__ results,
              long result_stride, float *__restrict__ eq_dbg, float *__restrict__ state_dbg, uint32_t call_index,
-             unsigned long long keystream, int n_streams) {
+             unsigned long long keystream, int n_streams, float2 *__restrict__ sym) {
     const long s = (long) blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= n_streams) return;
 
     TileLoader ld;
     ld.X = win + ((s >> 5) * WIN_ROWS) * 32 + (s & 31);
     TrackOut o;
-    track_core(ld, o);
+    track_core<SOFT>(ld, o, SOFT ? sym + s * result_stride * NDATA : nullptr);
 
     const int t_in = timing_cur[s];
     const int mi = max_index[s];
@@ -369,12 +370,13 @@ track_train_kernel(const float2 *__restrict__ win, float *__restrict__ state, lo
     e[36 * stride] = mag;
 }
 
+template <bool SOFT>
 __global__ void __launch_bounds__(TK_THREADS)
 track_data_kernel(const float2 *__restrict__ win, const float *__restrict__ state, long stride,
                   const int *__restrict__ max_index, const float *__restrict__ max_value,
                   const int *__restrict__ timing_cur, int *__restrict__ timing_next, sc_frame_result *__restrict__ results,
                   long result_stride, uint32_t call_index, unsigned long long keystream, int n_streams, TimingSrc ts,
-                  int *__restrict__ timing_cur_out, bool coop_state) {
+                  int *__restrict__ timing_cur_out, bool coop_state, float2 *__restrict__ sym) {
     const long s = (long) blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= n_streams) return;
     const int t_in = resolve_timing(ts, timing_cur, s);
@@ -413,7 +415,7 @@ track_data_kernel(const float2 *__restrict__ win, const float *__restrict__ stat
     }
     o.valid = o.matches > MATCH_THRESHOLD;                          // qpsk.c:196
     float cost;
-    track_data(ld, o.tk, o.valid, o.word, cost);
+    track_data<SOFT>(ld, o.tk, o.valid, o.word, cost, SOFT ? sym + s * result_stride * NDATA : nullptr);
     o.cost = o.valid ? mag : cost;
 
     const int mi = max_index[s];
@@ -437,12 +439,12 @@ static_assert(TRK_STATE_WORDS >= 57, "cooperative tracker state");
 
 __device__ __forceinline__ void tc_barrier() { asm volatile("bar.sync 1, 64;" ::: "memory"); }
 
-template <int PHASE>
+template <int PHASE, bool SOFT>
 __global__ void __launch_bounds__(TC_THREADS)
 track_coop_kernel(const float2 *__restrict__ win, const int *__restrict__ max_index, const float *__restrict__ max_value,
                   const int *__restrict__ timing_cur, int *__restrict__ timing_next,
                   sc_frame_result *__restrict__ results, long result_stride, uint32_t call_index,
-                  unsigned long long keystream, int n_streams, float *__restrict__ state) {
+                  unsigned long long keystream, int n_streams, float *__restrict__ state, float2 *__restrict__ sym) {
     // The window is rows of 8 bytes in L2 (the front-end has just written it), ~700 clocks away; a step is ~250.
     // All of it is fetched at once into shared memory, then read from there.
     constexpr int ROWS = PHASE == TRK_ALL ? WIN_ROWS : PRE + EQ;
@@ -517,13 +519,13 @@ track_coop_kernel(const float2 *__restrict__ win, const int *__restrict__ max_in
     // equalize(), qpsk.c:111-123, and magnitude(), qpsk.c:101-109 (the sum over x[0] is the one lane 0 keeps)
     int matches = 0, bI, bQ;
     float mag = 0.0f;
-    c32 xi = from2(Xi[0]);
+    c32 xi = from2(Xi[0]), v;
 #pragma unroll 2
     for (int k = 0; k < PRE; k++) {
         const c32 ni = from2(Xi[k + 1]);
         const float ref = ((c_pre_neg[k >> 5] >> (k & 31)) & 1u) ? -1.0f : 1.0f;
         mag = __fadd_rn(mag, __fadd_rn(__fmul_rn(xi.r, xi.r), __fmul_rn(xi.i, xi.i)));
-        const c32 err = tp.error<false>(xi, ref, bI, bQ);
+        const c32 err = tp.error<false>(xi, ref, bI, bQ, v);
         if (__fmul_rn(err.r, ref) > 0.0f) matches++;
         tc_barrier();
         tp.update(err, &s_xa[k & 1][qs]);
@@ -549,10 +551,12 @@ track_coop_kernel(const float2 *__restrict__ win, const int *__restrict__ max_in
     xi = from2(Xi[0]);
     unsigned long long word = 0ull;
     float cost = 0.0f;
+    float2 *ssym = SOFT ? sym + s * result_stride * NDATA : nullptr;   // written by the storing lane only
 #pragma unroll 1
     for (int k = 0; k < NDATA; k++) {
         const c32 ni = from2(Xi[k + 1]);                           // at most row 197 + 1: inside the padded array
-        const c32 err = tp.error<true>(xi, 0.0f, bI, bQ);
+        const c32 err = tp.error<true>(xi, 0.0f, bI, bQ, v);
+        if (SOFT && store) ssym[k] = to2(v);
         cost = __fadd_rn(cost, err.r);                             // qpsk.c:228
         word |= ((unsigned long long) (unsigned) (bQ | (bI << 1))) << (2 * k);
         tc_barrier();
@@ -600,9 +604,11 @@ static cudaError_t rx_kernel_attributes() {
     SC_PREF((frontend_kernel<true, false, false, true>));
     SC_PREF((frontend_kernel<true, true, false, true>));
     SC_PREF(track_train_kernel);
-    SC_PREF(track_data_kernel);
-    SC_PREF(track_coop_kernel<TRK_ALL>);
-    SC_PREF(track_coop_kernel<TRK_TRAIN>);
+    SC_PREF(track_data_kernel<false>);
+    SC_PREF(track_data_kernel<true>);
+    SC_PREF((track_coop_kernel<TRK_ALL, false>));
+    SC_PREF((track_coop_kernel<TRK_ALL, true>));
+    SC_PREF((track_coop_kernel<TRK_TRAIN, false>));
 #undef SC_PREF
     if (dev < 64) done.fetch_or(1ull << dev);
     return cudaSuccess;
@@ -656,24 +662,37 @@ cudaError_t launch_frontend(bool wide, const int16_t *in, long stream_stride, co
 cudaError_t launch_track(bool debug_eq, const float2 *win, const int *max_index, const float *max_value,
                          const int *timing_cur, int *timing_next, sc_frame_result *results, long result_stride,
                          float *eq_dbg, float *state_dbg, uint32_t call_index, unsigned long long keystream,
-                         int n_streams, cudaStream_t st, bool coop) {
+                         int n_streams, cudaStream_t st, bool coop, float *sym) {
     cudaError_t ea = rx_kernel_attributes();
     if (ea != cudaSuccess) return ea;
+    float2 *sym2 = reinterpret_cast<float2 *>(sym);
     if (coop && !debug_eq) {
-        track_coop_kernel<TRK_ALL><<<(n_streams + TC_STREAMS - 1) / TC_STREAMS, TC_THREADS, 0, st>>>(
-            win, max_index, max_value, timing_cur, timing_next, results, result_stride, call_index, keystream, n_streams,
-            nullptr);
+        const int grid = (n_streams + TC_STREAMS - 1) / TC_STREAMS;
+        if (sym)
+            track_coop_kernel<TRK_ALL, true><<<grid, TC_THREADS, 0, st>>>(
+                win, max_index, max_value, timing_cur, timing_next, results, result_stride, call_index, keystream,
+                n_streams, nullptr, sym2);
+        else
+            track_coop_kernel<TRK_ALL, false><<<grid, TC_THREADS, 0, st>>>(
+                win, max_index, max_value, timing_cur, timing_next, results, result_stride, call_index, keystream,
+                n_streams, nullptr, nullptr);
         g_launch_count++;
         return cudaGetLastError();
     }
     const int thr = TK_THREADS;                 // 32 / 64 / 128 measured equal within 0.3 %
     const int grid = (n_streams + thr - 1) / thr;
     if (debug_eq)
-        track_kernel<true><<<grid, thr, 0, st>>>(win, max_index, max_value, timing_cur, timing_next, results,
-                                                        result_stride, eq_dbg, state_dbg, call_index, keystream, n_streams);
+        track_kernel<true, false><<<grid, thr, 0, st>>>(win, max_index, max_value, timing_cur, timing_next, results,
+                                                        result_stride, eq_dbg, state_dbg, call_index, keystream, n_streams,
+                                                        nullptr);
+    else if (sym)
+        track_kernel<false, true><<<grid, thr, 0, st>>>(win, max_index, max_value, timing_cur, timing_next, results,
+                                                        result_stride, nullptr, nullptr, call_index, keystream, n_streams,
+                                                        sym2);
     else
-        track_kernel<false><<<grid, thr, 0, st>>>(win, max_index, max_value, timing_cur, timing_next, results,
-                                                         result_stride, eq_dbg, state_dbg, call_index, keystream, n_streams);
+        track_kernel<false, false><<<grid, thr, 0, st>>>(win, max_index, max_value, timing_cur, timing_next, results,
+                                                         result_stride, eq_dbg, state_dbg, call_index, keystream, n_streams,
+                                                         nullptr);
     g_launch_count++;
     return cudaGetLastError();
 }
@@ -684,8 +703,8 @@ cudaError_t launch_track(bool debug_eq, const float2 *win, const int *max_index,
 cudaError_t launch_track_train(const float2 *win_ov, float *state, long state_stride, int n_streams, cudaStream_t st,
                                bool coop) {
     if (coop)
-        track_coop_kernel<TRK_TRAIN><<<(n_streams + TC_STREAMS - 1) / TC_STREAMS, TC_THREADS, 0, st>>>(
-            win_ov, nullptr, nullptr, nullptr, nullptr, nullptr, 0, 0u, 0ull, n_streams, state);
+        track_coop_kernel<TRK_TRAIN, false><<<(n_streams + TC_STREAMS - 1) / TC_STREAMS, TC_THREADS, 0, st>>>(
+            win_ov, nullptr, nullptr, nullptr, nullptr, nullptr, 0, 0u, 0ull, n_streams, state, nullptr);
     else
         track_train_kernel<<<(n_streams + TK_THREADS - 1) / TK_THREADS, TK_THREADS, 0, st>>>(win_ov, state, state_stride,
                                                                                             n_streams);
@@ -696,13 +715,19 @@ cudaError_t launch_track_train(const float2 *win_ov, float *state, long state_st
 cudaError_t launch_track_data(const float2 *win_ov, float *state, long state_stride, const int *max_index,
                               const float *max_value, const int *timing_cur, int *timing_next, sc_frame_result *results,
                               long result_stride, uint32_t call_index, unsigned long long keystream, int n_streams,
-                              cudaStream_t st, bool coop, const TimingSrc *tsp, int *timing_cur_out) {
+                              cudaStream_t st, bool coop, const TimingSrc *tsp, int *timing_cur_out, float *sym) {
     const TimingSrc ts = tsp ? *tsp : TimingSrc();
     // off the chains' critical path and sharing the SMs with their kernels: spread thin on small banks
     const int thr = n_streams <= 148 * 32 ? 32 : n_streams <= 148 * 64 ? 64 : TK_THREADS;
-    track_data_kernel<<<(n_streams + thr - 1) / thr, thr, 0, st>>>(
-        win_ov, state, state_stride, max_index, max_value, timing_cur, timing_next, results, result_stride, call_index,
-        keystream, n_streams, ts, timing_cur_out, coop);
+    const int grid = (n_streams + thr - 1) / thr;
+    if (sym)
+        track_data_kernel<true><<<grid, thr, 0, st>>>(
+            win_ov, state, state_stride, max_index, max_value, timing_cur, timing_next, results, result_stride, call_index,
+            keystream, n_streams, ts, timing_cur_out, coop, reinterpret_cast<float2 *>(sym));
+    else
+        track_data_kernel<false><<<grid, thr, 0, st>>>(
+            win_ov, state, state_stride, max_index, max_value, timing_cur, timing_next, results, result_stride, call_index,
+            keystream, n_streams, ts, timing_cur_out, coop, nullptr);
     g_launch_count++;
     return cudaGetLastError();
 }

@@ -51,10 +51,11 @@ __device__ __forceinline__ void track_train(const Loader &ld, Tracker &tk, int &
     mag_out = mag;
 }
 
-// the 31 data_eq() steps of qpsk.c:206-215 (valid) / :226-229 (invalid), continuing from the trained tracker
-template <class Loader>
+// the 31 data_eq() steps of qpsk.c:206-215 (valid) / :226-229 (invalid), continuing from the trained tracker.
+// SOFT: the equalizer output of step i also goes to sym[i] (one 8-byte store per step).
+template <bool SOFT = false, class Loader>
 __device__ __forceinline__ void track_data(const Loader &ld, Tracker &tk, bool valid, unsigned long long &word_out,
-                                           float &cost_out) {
+                                           float &cost_out, float2 *sym = nullptr) {
     // valid: data symbols follow the preamble; invalid: they start at rx_timing
     c32 x[EQ];
 #pragma unroll
@@ -69,7 +70,9 @@ __device__ __forceinline__ void track_data(const Loader &ld, Tracker &tk, bool v
         const int rn = min(i + EQ, Y_ROWS - 1);
         nxt = valid ? ld.x(PRE + rn) : ld.y(rn);
         int bI, bQ;
-        const float er = tk.data(x, bI, bQ);
+        c32 s;
+        const float er = tk.data(x, bI, bQ, s);
+        if (SOFT) sym[i] = to2(s);
         cost = __fadd_rn(cost, er);                                // qpsk.c:228
         word |= ((unsigned long long) (unsigned) (bQ | (bI << 1))) << (2 * i);   // bits[2i]=Q, bits[2i+1]=I
 #pragma unroll
@@ -79,13 +82,13 @@ __device__ __forceinline__ void track_data(const Loader &ld, Tracker &tk, bool v
     cost_out = cost;
 }
 
-template <class Loader>
-__device__ __forceinline__ void track_core(const Loader &ld, TrackOut &o) {
+template <bool SOFT = false, class Loader>
+__device__ __forceinline__ void track_core(const Loader &ld, TrackOut &o, float2 *sym = nullptr) {
     int matches;
     float mag, cost;
     track_train(ld, o.tk, matches, mag);
     const bool valid = matches > MATCH_THRESHOLD;                  // qpsk.c:196
-    track_data(ld, o.tk, valid, o.word, cost);
+    track_data<SOFT>(ld, o.tk, valid, o.word, cost, sym);
     o.cost = valid ? mag : cost;
     o.matches = matches;
     o.valid = valid;

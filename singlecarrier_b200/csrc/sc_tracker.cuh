@@ -108,9 +108,10 @@ struct Tracker {
     }
 
     // data_eq(&dibit, in, index) without the descrambler, src/equalizer.c:64-85 and
-    // qpsk_demod(), src/qpsk.c:268-271.  Returns crealf(error); bI/bQ are the raw decisions.
-    __device__ __forceinline__ float data(const c32 (&x)[EQ], int &bI, int &bQ) {
-        c32 s = mk(0.0f, 0.0f);
+    // qpsk_demod(), src/qpsk.c:268-271.  Returns crealf(error); bI/bQ are the raw decisions, s the equalizer output
+    // they are sliced from (`sym` of data_eq()).
+    __device__ __forceinline__ float data(const c32 (&x)[EQ], int &bI, int &bQ, c32 &s) {
+        s = mk(0.0f, 0.0f);
 #pragma unroll
         for (int i = 0; i < EQ; i++) s = cadd(s, cmulc(x[i], C[i]));
         bI = s.r < 0.0f;
@@ -120,6 +121,10 @@ struct Tracker {
         const c32 err = mk(__fmul_rn(__fsub_rn(ci, s.r), 0.1f), __fmul_rn(__fsub_rn(cq, s.i), 0.1f));
         update(x, err);
         return err.r;
+    }
+    __device__ __forceinline__ float data(const c32 (&x)[EQ], int &bI, int &bQ) {
+        c32 s;
+        return data(x, bI, bQ, s);
     }
 };
 

@@ -180,9 +180,9 @@ struct TapLanes {
     __device__ __forceinline__ void reset() { C = mk(0.0f, 0.0f); }
 
     // head of train_eq() (DATA = false, src/equalizer.c:45-52) or data_eq() (DATA = true, :64-80): the equalizer's
-    // output from the taps as they stand, decision, error.  xi = x[i].
+    // output from the taps as they stand (v, every lane of the group), decision, error.  xi = x[i].
     template <bool DATA>
-    __device__ __forceinline__ c32 error(c32 xi, float ref, int &bI, int &bQ) const {
+    __device__ __forceinline__ c32 error(c32 xi, float ref, int &bI, int &bQ, c32 &v) const {
         ex->v[slot] = to2(DATA ? cmulc(xi, C) : cmul(xi, C));
         __syncwarp();
         float2 p0, p1, p2, p3;
@@ -190,7 +190,7 @@ struct TapLanes {
         lds128(&ex->v[2], p2, p3);
         const float2 p4 = ex->v[4];
         __syncwarp();
-        c32 v = mk(0.0f, 0.0f);
+        v = mk(0.0f, 0.0f);
         v = cadd(v, from2(p0));
         v = cadd(v, from2(p1));
         v = cadd(v, from2(p2));

@@ -17,6 +17,7 @@ from ._lib import SC_FLAG_DEBUG_EQ, SC_FLAG_PACKET, SC_FLAG_WIDE, Channel, check
 FRAME_SIZE = 1880
 SYMBOLS_PER_FRAME = 376
 BITS_PER_CALL = 62
+DATA_SYMBOLS = 31          # data steps per call: bits 2i (Q) and 2i+1 (I) are sliced from symbol i
 PACKET_SAMPLES = 1880
 OPT_SLAB_PARTS, OPT_PROFILE, OPT_H2D_MODE, OPT_FE_SEARCH, OPT_TRACKER, OPT_OVERLAP = 1, 2, 3, 4, 5, 6
 OVERLAP_AUTO, OVERLAP_OFF, OVERLAP_ON, OVERLAP_MAX = 0, 1, 2, 32768
@@ -40,6 +41,25 @@ assert PACKET_DTYPE.itemsize == 96
 
 def keystream_word(call_index: int) -> int:
     return int(lib.sc_keystream_word(call_index))
+
+
+def soft_bits(results: np.ndarray, symbols: np.ndarray) -> np.ndarray:
+    """Soft decisions in the order of ``bits``: float32 [..., 62] with soft[2i] = +-Im and soft[2i+1] = +-Re of
+    symbol i, negated where the call's keystream bit is 1, so that bit k == (soft[k] < 0) wherever the component
+    is non-zero.  ``results`` RESULT_DTYPE [...], ``symbols`` complex64 [..., 31] from rx_frames_soft_*."""
+    r = np.asarray(results)
+    assert r.dtype == RESULT_DTYPE
+    sym = np.asarray(symbols, np.complex64)
+    assert sym.shape == r.shape + (DATA_SYMBOLS,)
+    soft = np.empty(r.shape + (BITS_PER_CALL,), np.float32)
+    soft[..., 0::2] = sym.imag
+    soft[..., 1::2] = sym.real
+    calls = r["call_index"].ravel()
+    uniq, inv = np.unique(calls, return_inverse=True)
+    words = np.array([keystream_word(int(c)) for c in uniq], np.uint64)[inv].reshape(r.shape)
+    flip = ((words[..., None] >> np.arange(BITS_PER_CALL, dtype=np.uint64)) & np.uint64(1)).astype(bool)
+    soft[flip] = -soft[flip]
+    return soft
 
 
 def launch_count() -> int:
@@ -235,6 +255,20 @@ class ModemBank:
                                     results.strides[0] // 32, _ptr(eq)))
         return results, eq
 
+    def rx_frames_soft_host(self, samples: np.ndarray, n_frames: Optional[int] = None):
+        """rx_frames_host plus the equalizer output of every data step (sc_rx_frames_soft_host).  Returns
+        (results[n_streams, n_frames], symbols complex64 [n_streams, n_frames, 31]); see soft_bits()."""
+        assert samples.dtype == np.int16 and samples.ndim == 2 and samples.shape[0] == self.n_streams
+        assert samples.strides[1] == 2
+        stride = samples.strides[0] // 2
+        if n_frames is None:
+            n_frames = samples.shape[1] // FRAME_SIZE
+        results = np.zeros((self.n_streams, n_frames), RESULT_DTYPE)
+        symbols = np.zeros((self.n_streams, n_frames, DATA_SYMBOLS), np.complex64)
+        check(lib.sc_rx_frames_soft_host(self._h, samples.ctypes.data, stride, n_frames, results.ctypes.data,
+                                         n_frames, symbols.ctypes.data))
+        return results, symbols
+
     def rx_packets_host(self, samples: np.ndarray, n_frames: Optional[int] = None, capacity: Optional[int] = None):
         """Packet mode (extension): the ordinary results plus one PACKET_DTYPE record per valid call n >= 2 with all
         8 x 62 bits of the packet, sorted by (stream, call).  Returns (results, packets, n_found)."""
@@ -264,6 +298,14 @@ class ModemBank:
         [n_streams, n_frames*32] (view as RESULT_DTYPE after copying back)."""
         check(lib.sc_rx_frames_dev(self._h, samples.data_ptr(), samples.stride(0), n_frames,
                                    results.data_ptr(), results.stride(0) // 32, _ptr(eq_dbg), stream))
+
+    def rx_frames_soft_dev(self, samples, n_frames: int, results, symbols, stream: int = 0) -> None:
+        """rx_frames_dev plus the equalizer outputs: symbols is a CUDA tensor with 62 floats (31 complex) per record,
+        records indexed like results (e.g. float32 [n_streams, n_frames*62] or complex64 [n_streams, n_frames, 31])."""
+        result_stride = results.stride(0) // 32
+        assert symbols.stride(0) * symbols.element_size() == result_stride * DATA_SYMBOLS * 8, "records' stride"
+        check(lib.sc_rx_frames_soft_dev(self._h, samples.data_ptr(), samples.stride(0), n_frames, results.data_ptr(),
+                                        result_stride, symbols.data_ptr(), stream))
 
     # ---- TX ------------------------------------------------------------------------------------
     def tx_packets_dev(self, out, n_packets: int, gap_samples: int = REFERENCE_GAP, bits=None, bits_out=None,
