@@ -124,7 +124,8 @@ uint64_t sc_launch_count(void);
 int  sc_set_option(sc_modem *m, int option, int64_t value);
 int  sc_profile_read(sc_modem *m, double out[4]);
 /* bytes queued host->device (out[0]) and device->host (out[1]) by sc_rx_frames_host / sc_rx_frames_soft_host
- * since sc_create */
+ * since sc_create (sc_rx_packets_host / sc_rx_packets_soft_host: the same for their ordinary calls; packet records
+ * and packet symbols are not counted) */
 int  sc_transfer_bytes(const sc_modem *m, uint64_t out[2]);
 /* frees the process-wide device caches (FFT twiddle / permutation tables) */
 int  sc_release_caches(void);
@@ -174,7 +175,7 @@ int sc_rx_frames_host(sc_modem *m, const int16_t *in, int64_t stream_stride, int
  * copies; sc_transfer_bytes counts the copied symbol bytes).  results and the bank's state afterwards are exactly
  * what sc_rx_frames_* would have produced, on the same schedules (SC_OPT_OVERLAP included), so soft and plain
  * batches may alternate on one handle.  There is no eq_dbg argument.  On SC_FLAG_PACKET banks these are ordinary
- * calls (no sc_packet_result).
+ * calls (no sc_packet_result); sc_rx_packets_soft_* below gives the soft output of the packets.
  */
 int sc_rx_frames_soft_dev(sc_modem *m, const int16_t *in, int64_t stream_stride, int n_frames,
                           sc_frame_result *results, int64_t result_stride, float *symbols, void *stream);
@@ -214,6 +215,38 @@ int sc_rx_packets_dev(sc_modem *m, const int16_t *in, int64_t stream_stride, int
 int sc_rx_packets_host(sc_modem *m, const int16_t *in, int64_t stream_stride, int n_frames,
                        sc_frame_result *results, int64_t result_stride, sc_packet_result *packets,
                        int64_t capacity, uint64_t *n_packets);
+
+/*
+ * Packet mode with soft output: sc_rx_packets_* and, in addition, the equalizer output of each of the 248 data
+ * steps of every packet record written -- the value its decision is sliced from, before slicing and descrambling.
+ * results, packets, capacity and n_packets mean exactly what they mean for sc_rx_packets_*; the records, results and
+ * the bank's state afterwards are the same, so soft and plain batches may alternate on one handle.  The records are
+ * appended in another order than sc_rx_packets_* appends them.
+ *
+ * packet_symbols: 8 x SC_DATA_SYMBOLS = 248 complex floats (re, im interleaved) per record; the block of packets[k]
+ *   starts at float k * 496, so record k and block k always belong to the same packet (for _dev also when
+ *   *n_packets does not start at 0).  Blocks of dropped records (beyond capacity) are not written.  Required (NULL:
+ *   SC_EINVAL before any work, the call index does not advance); for _dev a device pointer aligned to 8 bytes.
+ * symbols: NULL, or the per-call soft output with the layout and meaning of sc_rx_frames_soft_* (for _dev aligned to
+ *   8 bytes).
+ * Bit mapping: in data frame f (0..7) of a packet, with sym = the record's block, bit 2i of the raw decision is
+ * (Im(sym[31 f + i]) < 0) and bit 2i+1 is (Re(sym[31 f + i]) < 0), and packets[k].bits[f] = raw decision XOR
+ * sc_packet_keystream_word(f).  packets[k].cost is the float32 sequential sum over the 248 steps of
+ * (c - Re) * 0.1f, c = (Re < 0 ? -1 : 1), each operation rounded.
+ * sc_transfer_bytes counts what _host moves for the ordinary calls (results and per-call symbols) as for
+ * sc_rx_frames_soft_host; like sc_rx_packets_host it does not count packet records or packet symbols.
+ */
+int sc_rx_packets_soft_dev(sc_modem *m, const int16_t *in, int64_t stream_stride, int n_frames,
+                           sc_frame_result *results, int64_t result_stride, float *symbols,
+                           sc_packet_result *packets, int64_t capacity, uint64_t *n_packets,
+                           float *packet_symbols, void *stream);
+int sc_rx_packets_soft_host(sc_modem *m, const int16_t *in, int64_t stream_stride, int n_frames,
+                            sc_frame_result *results, int64_t result_stride, float *symbols,
+                            sc_packet_result *packets, int64_t capacity, uint64_t *n_packets,
+                            float *packet_symbols);
+/* descrambler keystream word of data frame `frame` (0..7) of every packet: the register is seeded with 0x4A80 per
+ * packet and advanced 62 steps per frame (0 for any other frame) */
+uint64_t sc_packet_keystream_word(int frame);
 
 /* Host helper: unpack results into the reference's on-disk format (qpsk.c:455-457): for every
  * VALID call, 62 bytes (0/1) are written to rows + (s*n_frames + j)*62; other rows untouched. */

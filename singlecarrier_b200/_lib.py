@@ -59,6 +59,9 @@ def _load() -> C.CDLL:
     sig("sc_rx_frames_soft_host", i32, vp, vp, i64, i32, vp, i64, vp)
     sig("sc_rx_packets_dev", i32, vp, vp, i64, i32, vp, i64, vp, i64, vp, vp)
     sig("sc_rx_packets_host", i32, vp, vp, i64, i32, vp, i64, vp, i64, C.POINTER(C.c_uint64))
+    sig("sc_rx_packets_soft_dev", i32, vp, vp, i64, i32, vp, i64, vp, vp, i64, vp, vp, vp)
+    sig("sc_rx_packets_soft_host", i32, vp, vp, i64, i32, vp, i64, vp, vp, i64, C.POINTER(C.c_uint64), vp)
+    sig("sc_packet_keystream_word", u64, i32)
     sig("sc_unpack_bits", None, vp, i64, vp)
     sig("sc_tx_packets_dev", i32, vp, vp, vp, u64, i32, i32, vp, vp, i64, i64, vp)
     sig("sc_tx_channel_dev", i32, vp, vp, vp, u64, i32, i32, vp, C.POINTER(Channel), vp, i64, i64, vp)

@@ -97,10 +97,14 @@ packet_fir_kernel(PacketSrc src, const int2 *__restrict__ list, const int *__res
 }
 
 // ---- the sequential loop over one packet ----------------------------------------------------------------
+// SOFT: the equalizer output of data step i also goes to psym[pos * PK_DATA + i], pos = the packet's record slot.  The
+// slot is claimed before the data loop (248 outputs cannot wait in registers), so a record and its symbol block always
+// belong to the same packet; both are dropped beyond packet_capacity.
+template <bool SOFT>
 __global__ void __launch_bounds__(128)
 packet_track_kernel(PacketSrc src, const int2 *__restrict__ list, const int *__restrict__ count, int cap,
                     const float2 *__restrict__ sym, PacketKey key, sc_packet_result *__restrict__ packets,
-                    long packet_capacity, unsigned long long *__restrict__ n_packets) {
+                    long packet_capacity, unsigned long long *__restrict__ n_packets, float2 *__restrict__ psym) {
     const int n_list = min(*count, cap);
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n_list) return;
@@ -127,12 +131,25 @@ packet_track_kernel(PacketSrc src, const int2 *__restrict__ list, const int *__r
     sc_packet_result r;
     float cost = 0.0f;
     unsigned long long word = 0ull;
+    unsigned long long pos = 0ull;
+    float2 *out = nullptr;
+    if (SOFT) {
+        pos = atomicAdd(n_packets, 1ull);
+        if ((long) pos < packet_capacity) out = psym + (long) pos * PK_DATA;
+    }
 #pragma unroll 1
     for (int i = 0; i < PK_DATA; i++) {                               // qpsk.c:206-215 over all NS x DATA_SYMBOLS symbols
         x[EQ - 1] = nxt;
         nxt = from2(X[min(PRE + i + EQ, PK_SYMS - 1) * 32]);
         int bI, bQ;
-        const float er = tk.data(x, bI, bQ);
+        float er;
+        if (SOFT) {
+            c32 s;
+            er = tk.data(x, bI, bQ, s);
+            if (out) out[i] = to2(s);
+        } else {
+            er = tk.data(x, bI, bQ);
+        }
         cost = __fadd_rn(cost, er);
         const int f = i / NDATA, k = i - f * NDATA;
         word |= ((unsigned long long) (unsigned) (bQ | (bI << 1))) << (2 * k);
@@ -152,13 +169,13 @@ packet_track_kernel(PacketSrc src, const int2 *__restrict__ list, const int *__r
     r.reserved0 = 0;
     r.reserved1 = 0;
     r.reserved2 = 0;
-    const unsigned long long pos = atomicAdd(n_packets, 1ull);
+    if (!SOFT) pos = atomicAdd(n_packets, 1ull);
     if ((long) pos < packet_capacity) packets[pos] = r;
 }
 
 cudaError_t launch_packet_pass(const PacketSrc &src, int n_streams, int j_lo, int j_hi, int cap, int2 *list, int *count,
                                float2 *sym, const PacketKey &key, sc_packet_result *packets, long packet_capacity,
-                               unsigned long long *n_packets, cudaStream_t st) {
+                               unsigned long long *n_packets, float2 *packet_sym, cudaStream_t st) {
     cudaError_t e = cudaMemsetAsync(count, 0, sizeof(int), st);
     if (e != cudaSuccess) return e;
     const long total = (long) n_streams * (j_hi - j_lo);
@@ -171,7 +188,12 @@ cudaError_t launch_packet_pass(const PacketSrc &src, int n_streams, int j_lo, in
     const int g2 = (int) std::min<long>((worst + PK_FIR_WARPS - 1) / PK_FIR_WARPS, 148L * 16);
     packet_fir_kernel<<<g2, PK_FIR_WARPS * 32, 0, st>>>(src, list, count, cap, sym);
     const int g3 = (int) ((worst + 127) / 128);
-    packet_track_kernel<<<g3, 128, 0, st>>>(src, list, count, cap, sym, key, packets, packet_capacity, n_packets);
+    if (packet_sym)
+        packet_track_kernel<true><<<g3, 128, 0, st>>>(src, list, count, cap, sym, key, packets, packet_capacity, n_packets,
+                                                      packet_sym);
+    else
+        packet_track_kernel<false><<<g3, 128, 0, st>>>(src, list, count, cap, sym, key, packets, packet_capacity,
+                                                       n_packets, nullptr);
     g_launch_count += 3;
     return cudaGetLastError();
 }

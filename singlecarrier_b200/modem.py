@@ -18,6 +18,8 @@ FRAME_SIZE = 1880
 SYMBOLS_PER_FRAME = 376
 BITS_PER_CALL = 62
 DATA_SYMBOLS = 31          # data steps per call: bits 2i (Q) and 2i+1 (I) are sliced from symbol i
+PACKET_FRAMES = 8          # data frames per packet (packet mode)
+PACKET_DATA_SYMBOLS = PACKET_FRAMES * DATA_SYMBOLS   # 248 data steps per packet record
 PACKET_SAMPLES = 1880
 OPT_SLAB_PARTS, OPT_PROFILE, OPT_H2D_MODE, OPT_FE_SEARCH, OPT_TRACKER, OPT_OVERLAP = 1, 2, 3, 4, 5, 6
 OVERLAP_AUTO, OVERLAP_OFF, OVERLAP_ON, OVERLAP_MAX = 0, 1, 2, 32768
@@ -59,6 +61,28 @@ def soft_bits(results: np.ndarray, symbols: np.ndarray) -> np.ndarray:
     words = np.array([keystream_word(int(c)) for c in uniq], np.uint64)[inv].reshape(r.shape)
     flip = ((words[..., None] >> np.arange(BITS_PER_CALL, dtype=np.uint64)) & np.uint64(1)).astype(bool)
     soft[flip] = -soft[flip]
+    return soft
+
+
+def packet_keystream_word(frame: int) -> int:
+    """Descrambler word of data frame ``frame`` (0..7) of every packet (the register is seeded per packet)."""
+    return int(lib.sc_packet_keystream_word(frame))
+
+
+def packet_soft_bits(packets: np.ndarray, packet_symbols: np.ndarray) -> np.ndarray:
+    """The packet counterpart of soft_bits: float32 [n, 8, 62] in the order of the packets' bits (frame f, bit k),
+    soft[f, 2i] = +-Im and soft[f, 2i+1] = +-Re of symbol 31 f + i, negated where the packet keystream bit is 1, so
+    that bit == (soft < 0) wherever the component is non-zero.  ``packets`` PACKET_DTYPE [n], ``packet_symbols``
+    complex64 [n, 248] from rx_packets_soft_*."""
+    p = np.asarray(packets)
+    assert p.dtype == PACKET_DTYPE and p.ndim == 1
+    sym = np.asarray(packet_symbols, np.complex64).reshape(p.shape[0], PACKET_FRAMES, DATA_SYMBOLS)
+    soft = np.empty((p.shape[0], PACKET_FRAMES, BITS_PER_CALL), np.float32)
+    soft[..., 0::2] = sym.imag
+    soft[..., 1::2] = sym.real
+    words = np.array([packet_keystream_word(f) for f in range(PACKET_FRAMES)], np.uint64)
+    flip = ((words[:, None] >> np.arange(BITS_PER_CALL, dtype=np.uint64)) & np.uint64(1)).astype(bool)
+    soft[:, flip] = -soft[:, flip]
     return soft
 
 
@@ -287,11 +311,50 @@ class ModemBank:
         got = got[np.lexsort((got["call_index"], got["stream"]))]
         return results, got, int(n.value)
 
+    def rx_packets_soft_host(self, samples: np.ndarray, n_frames: Optional[int] = None, capacity: Optional[int] = None,
+                             call_symbols: bool = False):
+        """rx_packets_host plus the equalizer output of the 248 data steps of every packet (sc_rx_packets_soft_host)
+        and, with call_symbols, of the 31 of every call.  Returns (results, call symbols complex64
+        [n_streams, n_frames, 31] or None, packets sorted by (stream, call), packet symbols complex64 [n, 248] in the
+        same order, n_found); see packet_soft_bits()."""
+        assert samples.dtype == np.int16 and samples.ndim == 2 and samples.shape[0] == self.n_streams
+        assert samples.strides[1] == 2
+        stride = samples.strides[0] // 2
+        if n_frames is None:
+            n_frames = samples.shape[1] // FRAME_SIZE
+        results = np.zeros((self.n_streams, n_frames), RESULT_DTYPE)
+        symbols = np.zeros((self.n_streams, n_frames, DATA_SYMBOLS), np.complex64) if call_symbols else None
+        if capacity is None:
+            capacity = self.n_streams * n_frames
+        packets = np.zeros(max(capacity, 1), PACKET_DTYPE)
+        psym = np.zeros((max(capacity, 1), PACKET_DATA_SYMBOLS), np.complex64)
+        n = C.c_uint64(0)
+        check(lib.sc_rx_packets_soft_host(self._h, samples.ctypes.data, stride, n_frames, results.ctypes.data, n_frames,
+                                          _ptr(symbols), packets.ctypes.data, capacity, C.byref(n), psym.ctypes.data))
+        kept = min(int(n.value), capacity)
+        got = packets[:kept]
+        order = np.lexsort((got["call_index"], got["stream"]))
+        return results, symbols, got[order], psym[:kept][order], int(n.value)
+
     def rx_packets_dev(self, samples, n_frames: int, results, packets, n_packets, stream: int = 0) -> None:
         """Device form: packets = CUDA uint8 [capacity * 96], n_packets = CUDA int64[1] (accumulated into)."""
         check(lib.sc_rx_packets_dev(self._h, samples.data_ptr(), samples.stride(0), n_frames, results.data_ptr(),
                                     results.stride(0) // 32, packets.data_ptr(), packets.numel() // 96,
                                     n_packets.data_ptr(), stream))
+
+    def rx_packets_soft_dev(self, samples, n_frames: int, results, packets, n_packets, packet_symbols,
+                            symbols=None, stream: int = 0) -> None:
+        """Device form of rx_packets_soft_host: as rx_packets_dev, plus packet_symbols, a CUDA tensor with 496 floats
+        (248 complex) per record of packets (e.g. complex64 [capacity, 248]), and symbols (None, or as for
+        rx_frames_soft_dev)."""
+        result_stride = results.stride(0) // 32
+        capacity = packets.numel() // 96
+        assert packet_symbols.numel() * packet_symbols.element_size() >= capacity * PACKET_DATA_SYMBOLS * 8, "capacity"
+        if symbols is not None:
+            assert symbols.stride(0) * symbols.element_size() == result_stride * DATA_SYMBOLS * 8, "records' stride"
+        check(lib.sc_rx_packets_soft_dev(self._h, samples.data_ptr(), samples.stride(0), n_frames, results.data_ptr(),
+                                         result_stride, _ptr(symbols), packets.data_ptr(), capacity,
+                                         n_packets.data_ptr(), packet_symbols.data_ptr(), stream))
 
     def rx_frames_dev(self, samples, n_frames: int, results, eq_dbg=None, stream: int = 0) -> None:
         """samples: CUDA int16 tensor [n_streams, stride]; results: CUDA uint8 tensor
