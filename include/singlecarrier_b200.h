@@ -393,6 +393,35 @@ int sc_ber_stats_dev(int device, const sc_frame_result *results, int64_t n_strea
                      int n_frames, const uint8_t *tx_bits, int n_packets, const int32_t *lead_in, int gap_samples,
                      const int32_t *group, int n_groups, uint64_t *counters, void *stream);
 
+#define SC_N_PACKET_BER_COUNTERS 32
+/* Bit errors of packet-mode records (SC_FLAG_PACKET) against the transmitted bits, on the device: the counter that
+ * goes with sc_rx_packets_dev / sc_rx_packets_soft_dev, so that a caller can queue the batch, this call and
+ * sc_reduce_stats on one CUDA stream without a host synchronisation.
+ *   packets, capacity, n_found: the buffers sc_rx_packets_dev filled; n_found is a DEVICE pointer, read by the kernel,
+ *             which counts records 0 .. min(*n_found, capacity) - 1 (records accumulated over several batches are all
+ *             counted).
+ *   results, n_streams, result_stride, n_frames, tx_bits, n_packets, lead_in, gap_samples, group, n_groups: as for
+ *             sc_ber_stats_dev (results: calls 0..n_frames-1 of a cold-started bank).
+ * Alignment, the rule of sc_ber_stats_dev applied to the record: with n = call_index and
+ * pos = (n-2)*1880 + 5*max_index + results[stream][n-2].rx_timing - 48 - lead_in[stream], the record is aligned to
+ * transmitted packet j when |pos - j*(1880 + gap_samples)| <= 10 and 0 <= j < n_packets.  TX scrambles and RX
+ * descrambles in packet mode, so the error pattern of data frame f (0..7) is (bits[f] ^ txword(f)) & (2^62 - 1), where
+ * txword(f) packs tx_bits[stream][j][f][0..61] & 1 (no keystream term).
+ * A record is not counted at all when its stream is outside 0..n_streams-1, its call_index outside 2..n_frames-1 or
+ * its stream's group outside 0..n_groups-1.
+ *   counters: device uint64[n_groups][32], ACCUMULATED into, plain sums: 0 records counted, 1 aligned records, 2 bits
+ *             compared (496 per aligned record), 3 bit errors, 4..7 reserved (0), 8+f bit errors in data frame f,
+ *             16+f aligned records with at least one error in data frame f, 24+b histogram of the bit errors of an
+ *             aligned record: b = 0 for none, b = 1..6 for 2^(b-1) .. 2^b - 1, b = 7 for 64 or more.  The packet
+ *             error rate is (counter 1 - counter 24) / counter 1.
+ * SC_EINVAL before any CUDA call: packets, n_found, results, tx_bits or counters NULL; capacity, n_streams or n_frames
+ * negative; result_stride < n_frames, n_packets < 1, gap_samples < 0 or n_groups < 1.  capacity == 0, n_streams == 0
+ * and n_frames < 3 launch nothing. */
+int sc_packet_ber_stats_dev(int device, const sc_packet_result *packets, int64_t capacity, const uint64_t *n_found,
+                            const sc_frame_result *results, int64_t n_streams, int64_t result_stride, int n_frames,
+                            const uint8_t *tx_bits, int n_packets, const int32_t *lead_in, int gap_samples,
+                            const int32_t *group, int n_groups, uint64_t *counters, void *stream);
+
 /* ---- multi-GPU reduction of the counters (SURVEY section 8e: the path's only collective) ------------------ */
 
 /* ncclAllReduce(sum) of n_counters uint64 in place on `stream`; nccl_comm is a ncclComm_t created by the

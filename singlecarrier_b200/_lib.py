@@ -83,6 +83,7 @@ def _load() -> C.CDLL:
     sig("sc_state_export", i32, vp, vp, i64)
     sig("sc_state_import", i32, vp, vp, i64)
     sig("sc_ber_stats_dev", i32, i32, vp, i64, i64, i32, vp, i32, vp, i32, vp, i32, vp, vp)
+    sig("sc_packet_ber_stats_dev", i32, i32, vp, i64, vp, vp, i64, i64, i32, vp, i32, vp, i32, vp, i32, vp, vp)
     sig("sc_reduce_stats", i32, vp, i32, vp, vp)
     sig("sc_comm_unique_id", i32, vp)
     sig("sc_comm_init_rank", i32, C.POINTER(vp), i32, i32, vp, i32)

@@ -99,6 +99,11 @@ cudaError_t launch_lock_stats(const sc_frame_result *results, long n_streams, lo
 cudaError_t launch_ber_stats(const sc_frame_result *results, long n_streams, long result_stride, int n_frames,
                              const uint8_t *tx_bits, int n_packets, const int *lead_in, int gap, const int *group,
                              int n_groups, unsigned long long *counters, cudaStream_t st);
+// capacity >= 1; n_found is read on the device
+cudaError_t launch_packet_ber_stats(const sc_packet_result *packets, long capacity, const unsigned long long *n_found,
+                                    const sc_frame_result *results, long n_streams, long result_stride, int n_frames,
+                                    const uint8_t *tx_bits, int n_packets, const int *lead_in, int gap,
+                                    const int *group, int n_groups, unsigned long long *counters, cudaStream_t st);
 
 // sc_packet_kernels.cu -- packet mode (extension)
 constexpr int PK_DATA = 8 * SC_DATA_SYMBOLS;                              // 248 data symbols per packet

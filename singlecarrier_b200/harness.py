@@ -14,7 +14,7 @@ from typing import Optional
 
 import numpy as np
 
-from .modem import FRAME_SIZE, REFERENCE_GAP, ModemBank, keystream_word
+from .modem import FRAME_SIZE, N_PACKET_BER_COUNTERS, REFERENCE_GAP, ModemBank, keystream_word
 from .taps import modem_taps
 
 PERIOD = FRAME_SIZE + REFERENCE_GAP          # 2783 samples: one packet + dead air (qpsk.c:384,405,410-412)
@@ -154,3 +154,28 @@ def ber_and_lock_dev(bank: ModemBank, res, n_frames: int, wl: Workload, group=No
     torch.cuda.synchronize(res.device)
     c = cnt.cpu().numpy()
     return {name: c[:, k].copy() for k, name in enumerate(("calls", "valid", "aligned", "bits", "errors"))}
+
+
+def packet_counters(c) -> dict:
+    """Named views of sc_packet_ber_stats_dev's counters (int64 [n_groups, 32])."""
+    c = np.asarray(c)
+    return {"records": c[:, 0].copy(), "aligned": c[:, 1].copy(), "bits": c[:, 2].copy(), "errors": c[:, 3].copy(),
+            "frame_errors": c[:, 8:16].copy(), "frames_in_error": c[:, 16:24].copy(),
+            "error_histogram": c[:, 24:32].copy()}
+
+
+def packet_ber_dev(bank: ModemBank, packets, n_found, res, n_frames: int, wl: Workload, group=None, n_groups: int = 1,
+                   comm=None):
+    """The packet counterpart of ber_and_lock_dev: bit errors of the packet records that rx_packets_dev left in
+    ``packets`` / ``n_found`` (sc_packet_ber_stats_dev), summed over all ranks with sc_reduce_stats when ``comm`` is
+    given.  Returns numpy arrays per group: records, aligned, bits, errors, frame_errors [n_groups, 8],
+    frames_in_error [n_groups, 8] and error_histogram [n_groups, 8] (bins 0 | 1 | 2-3 | ... | 32-63 | >= 64)."""
+    import torch
+    cnt = torch.zeros((n_groups, N_PACKET_BER_COUNTERS), dtype=torch.int64, device=res.device)
+    g = None if group is None else group.to(torch.int32).contiguous()
+    bank.packet_ber_stats(packets, n_found, res, n_frames, wl.tx_bits, wl.lead, wl.gap, cnt, group=g,
+                          n_groups=n_groups)
+    if comm is not None:
+        comm.all_reduce_counters(cnt)
+    torch.cuda.synchronize(res.device)
+    return packet_counters(cnt.cpu().numpy())

@@ -26,7 +26,7 @@ OVERLAP_AUTO, OVERLAP_OFF, OVERLAP_ON, OVERLAP_MAX = 0, 1, 2, 32768
 TRACKER_AUTO, TRACKER_THREAD, TRACKER_COOP, TRACKER_COOP_MAX = 0, 1, 2, 1024
 FE_SEARCH_DIRECT, FE_SEARCH_MMA, FE_SEARCH_TCGEN05 = 0, 1, 2
 H2D_COLUMNS, H2D_ROWS, H2D_FULL, H2D_COLUMNS_3D = 0, 1, 2, 3
-N_COUNTERS, N_BER_COUNTERS = 16, 8
+N_COUNTERS, N_BER_COUNTERS, N_PACKET_BER_COUNTERS = 16, 8, 32
 REFERENCE_GAP = 903         # dead air between packets in the reference's main(), qpsk.c:410-412
 
 # sc_frame_result, include/singlecarrier_b200.h
@@ -246,6 +246,16 @@ class ModemBank:
         check(lib.sc_ber_stats_dev(self.device, results.data_ptr(), self.n_streams, results.stride(0) // 32, n_frames,
                                    tx_bits.data_ptr(), n_packets, _ptr(lead_in), gap, _ptr(group), n_groups,
                                    counters.data_ptr(), stream))
+
+    def packet_ber_stats(self, packets, n_found, results, n_frames: int, tx_bits, lead_in, gap: int, counters,
+                         group=None, n_groups: int = 1, stream: int = 0) -> None:
+        """Accumulate the bit-error counters of packet records (sc_packet_ber_stats_dev) into counters (CUDA int64
+        [n_groups, 32]).  packets = CUDA uint8 [capacity * 96] and n_found = CUDA int64[1] as rx_packets_dev filled
+        them (n_found is read on the device); results, tx_bits, lead_in, gap, group as for ber_stats."""
+        check(lib.sc_packet_ber_stats_dev(self.device, packets.data_ptr(), packets.numel() // 96, n_found.data_ptr(),
+                                          results.data_ptr(), self.n_streams, results.stride(0) // 32, n_frames,
+                                          tx_bits.data_ptr(), tx_bits.shape[1], _ptr(lead_in), gap, _ptr(group),
+                                          n_groups, counters.data_ptr(), stream))
 
     def transfer_bytes(self):
         out = (C.c_uint64 * 2)()
