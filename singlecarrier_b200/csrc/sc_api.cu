@@ -46,13 +46,54 @@ static int fail(int code, const char *fmt, ...) {
     return code;
 }
 
+// A failed runtime call also sets the runtime's last error, which every launcher returns: clear it, so that a
+// refused allocation does not fail the next launch on this thread.
 #define CU(call)                                                                                   \
     do {                                                                                           \
         cudaError_t e_ = (call);                                                                   \
-        if (e_ != cudaSuccess)                                                                     \
+        if (e_ != cudaSuccess) {                                                                   \
+            cudaGetLastError();                                                                    \
             return fail(e_ == cudaErrorMemoryAllocation ? SC_ENOMEM : SC_ECUDA, "%s:%d %s: %s",    \
                         __FILE__, __LINE__, #call, cudaGetErrorString(e_));                        \
+        }                                                                                          \
     } while (0)
+
+// Device resources owned by the handle or a cache entry, released with their device current.
+template <typename T>
+struct DevBuf {
+    T *p = nullptr;
+    size_t cap = 0;                                 // elements
+    DevBuf() = default;
+    DevBuf(DevBuf &&o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr, o.cap = 0; }
+    DevBuf &operator=(DevBuf &&o) noexcept { std::swap(p, o.p), std::swap(cap, o.cap); return *this; }
+    ~DevBuf() { if (p) cudaFree(p); }
+    operator T *() const { return p; }
+    // room for n elements; the contents are discarded when n exceeds the capacity
+    cudaError_t reserve(size_t n) {
+        if (cap >= n) return cudaSuccess;
+        cudaError_t e = p ? cudaFree(p) : cudaSuccess;
+        p = nullptr, cap = 0;
+        if (e == cudaSuccess && (e = cudaMalloc(&p, n * sizeof(T))) == cudaSuccess) cap = n;
+        return e;
+    }
+};
+
+template <typename H, cudaError_t (*Destroy)(H)>
+struct Owned {
+    H h = nullptr;
+    Owned() = default;
+    Owned(Owned &&o) noexcept : h(o.h) { o.h = nullptr; }
+    Owned &operator=(Owned &&) = delete;
+    ~Owned() { if (h) Destroy(h); }
+    operator H() const { return h; }
+};
+// create() does nothing when the object exists, so lazily built scratch that failed part-way is completed later
+struct Stream : Owned<cudaStream_t, cudaStreamDestroy> {
+    cudaError_t create() { return h ? cudaSuccess : cudaStreamCreateWithFlags(&h, cudaStreamNonBlocking); }
+};
+struct Event : Owned<cudaEvent_t, cudaEventDestroy> {
+    cudaError_t create(unsigned flags = cudaEventDisableTiming) { return h ? cudaSuccess : cudaEventCreateWithFlags(&h, flags); }
+};
 
 static const int N_PIPE = 3;        // internal CUDA streams (slabs in flight)
 static const int TAB_HEAD = 2;      // phasor-table frames generated before the first call starts
@@ -74,53 +115,50 @@ struct sc_modem {
     float2 rx_rect, tx_rect;
 
     // per-stream device state (SURVEY appendix B)
-    int *timing[2] = {nullptr, nullptr};    // rx_timing at entry of call n in timing[n & 1]
-    int *timing_cold = nullptr;             // FINE_TIMING_OFFSET for every stream (source of resets)
-    float2 *win = nullptr;                  // tracker windows, tiles of 32 streams x WIN_ROWS
-    int *max_index = nullptr;
-    float *max_value = nullptr;
-    int16_t *hist = nullptr;                // last frame of the previous batch, [n][1880]
+    DevBuf<int> timing[2];                  // rx_timing at entry of call n in timing[n & 1]
+    DevBuf<int> timing_cold;                // FINE_TIMING_OFFSET for every stream (source of resets)
+    DevBuf<float2> win;                     // tracker windows, tiles of 32 streams x WIN_ROWS
+    DevBuf<int> max_index;
+    DevBuf<float> max_value;
+    DevBuf<int16_t> hist;                   // last frame of the previous batch, [n][1880]
 
     // shared tables
-    float2 *rx_phase = nullptr;             // fbb_rx_phase (device scalar)
-    float2 *mix_table = nullptr;            // slot 0 = frame of call-1, slots 1.. = this batch
-    int mix_cap = 0;                        // frames
-    float2 *unit_phase = nullptr;           // constant 1+0i: the cold phasor of a transmission (qpsk.c:375)
+    DevBuf<float2> rx_phase;                // fbb_rx_phase (device scalar)
+    DevBuf<float2> mix_table;               // slot 0 = frame of call-1, slots 1.. = this batch
+    DevBuf<float2> unit_phase;              // constant 1+0i: the cold phasor of a transmission (qpsk.c:375)
     float *state_dbg = nullptr;             // drop-in shim: full tracker state after the last call, [n][48] (not owned)
+    std::vector<uint64_t> kw;               // keystream words of the batch being queued
 
-    cudaStream_t pipe[N_PIPE] = {};
-    cudaEvent_t ev_start = nullptr, ev_done[N_PIPE] = {};
+    Stream pipe[N_PIPE];
+    Event ev_start, ev_done[N_PIPE];
     // the phasor table is generated by one thread (a sequential float recurrence): the first TAB_HEAD
     // frames on pipe[0], the rest on tab_stream while the first calls already run
-    cudaStream_t tab_stream = nullptr;
-    cudaEvent_t ev_tab1 = nullptr, ev_tab2 = nullptr;
+    Stream tab_stream;
+    Event ev_tab1, ev_tab2;
     int tab_split = 0;                      // table slots 1..tab_split are ready once pipe[0]'s part is done
-    std::vector<cudaEvent_t> ev_tabc;       // piece c (slots tab_split + 1 + TAB_CHUNK c ..) is ready at ev_tabc[c]
+    std::vector<Event> ev_tabc;             // piece c (slots tab_split + 1 + TAB_CHUNK c ..) is ready at ev_tabc[c]
 
     // staging for the host entry point
-    int16_t *stage_in[N_PIPE] = {};
-    sc_frame_result *stage_res[N_PIPE] = {};
-    float *stage_eq[N_PIPE] = {};
-    float *stage_sym[N_PIPE] = {};
-    size_t stage_in_cap = 0, stage_res_cap = 0, stage_eq_cap = 0, stage_sym_cap = 0;
+    DevBuf<int16_t> stage_in[N_PIPE];
+    DevBuf<sc_frame_result> stage_res[N_PIPE];
+    DevBuf<float> stage_eq[N_PIPE];
+    DevBuf<float> stage_sym[N_PIPE];
 
     // packet mode (SC_FLAG_PACKET, extension): the frame before the saved one, its phasor table, the rx_timing
     // snapshots and per-pipe scratch for the packet pass
     bool packet = false;
-    int16_t *pk_hist2 = nullptr;            // frame call-2, [n][1880]
-    float2 *pk_mix_hist2 = nullptr;         // phasor table of frame call-2
-    int *pk_t_before[N_PIPE] = {}, *pk_t_at[N_PIPE] = {};     // [slab] rx_timing at entry of calls call0-1 / call0
-    int2 *pk_list[N_PIPE] = {};
-    int *pk_count[N_PIPE] = {};
-    float2 *pk_sym[N_PIPE] = {};
-    cudaStream_t pk_stream[N_PIPE] = {};    // the packet passes run beside the call chain, not inside it
-    cudaEvent_t pk_ev_go[N_PIPE] = {}, pk_ev_done[N_PIPE] = {};
-    size_t pk_slab_cap = 0;
-    unsigned long long *pk_n_host_dev = nullptr;               // packet counter of the host entry point
-    sc_packet_result *pk_stage = nullptr;
-    size_t pk_stage_cap = 0;
-    float2 *pk_sym_stage = nullptr;         // packet symbols of the host entry point, PK_DATA per record
-    size_t pk_sym_stage_cap = 0;            // in records
+    DevBuf<int16_t> pk_hist2;               // frame call-2, [n][1880]
+    DevBuf<float2> pk_mix_hist2;            // phasor table of frame call-2
+    DevBuf<int> pk_t_before[N_PIPE], pk_t_at[N_PIPE];         // [slab] rx_timing at entry of calls call0-1 / call0
+    DevBuf<int2> pk_list[N_PIPE];
+    DevBuf<int> pk_count[N_PIPE];
+    DevBuf<float2> pk_sym[N_PIPE];
+    Stream pk_stream[N_PIPE];               // the packet passes run beside the call chain, not inside it
+    Event pk_ev_go[N_PIPE], pk_ev_done[N_PIPE];
+    bool pk_ready = false;
+    DevBuf<unsigned long long> pk_n_host_dev;                  // packet counter of the host entry point
+    DevBuf<sc_packet_result> pk_stage;
+    DevBuf<float2> pk_sym_stage;            // packet symbols of the host entry point, PK_DATA per record
     PacketKey pk_key;
 
     // A batch call that failed after its first launch leaves some streams advanced and others not:
@@ -142,16 +180,16 @@ struct sc_modem {
     // overlapped chains (SC_OPT_OVERLAP): tall windows, search results, the tracker hand-over and rx_timing in rings of
     // OV_RING calls; two chain streams (the pipe and a partner) and a stream for the data steps per pipe; event rings
     int overlap = SC_OVERLAP_AUTO;
-    float2 *ov_win[OV_RING] = {};
-    int *ov_max_index[OV_RING] = {};
-    float *ov_max_value[OV_RING] = {};
-    float *ov_state[OV_RING] = {};
-    int *ov_timing[OV_RING] = {};
-    cudaStream_t ov_stream[N_PIPE] = {}, ov_data[N_PIPE][2] = {};
-    cudaEvent_t ov_ev_fe[N_PIPE][OV_RING] = {}, ov_ev_train[N_PIPE][OV_RING] = {}, ov_ev_data[N_PIPE][OV_RING] = {};
-    cudaEvent_t ov_ev_first[N_PIPE] = {}, ov_join[N_PIPE][3] = {};
+    DevBuf<float2> ov_win[OV_RING];
+    DevBuf<int> ov_max_index[OV_RING];
+    DevBuf<float> ov_max_value[OV_RING];
+    DevBuf<float> ov_state[OV_RING];
+    DevBuf<int> ov_timing[OV_RING];
+    Stream ov_stream[N_PIPE], ov_data[N_PIPE][2];
+    Event ov_ev_fe[N_PIPE][OV_RING], ov_ev_train[N_PIPE][OV_RING], ov_ev_data[N_PIPE][OV_RING];
+    Event ov_ev_first[N_PIPE], ov_join[N_PIPE][3];
     bool ov_ready = false;
-    std::vector<cudaEvent_t> ev_fe, ev_tk;  // (start, stop) pairs
+    std::vector<Event> ev_fe, ev_tk;        // (start, stop) pairs
 };
 
 // ---- scrambler keystream (integer LFSR, src/scramble.c:57-69) ----------------------------------
@@ -255,27 +293,27 @@ extern "C" int sc_create(sc_modem **out, int device, int64_t n_streams, uint32_t
     auto body = [&]() -> int {
         CU(cudaSetDevice(device));
         const int64_t np = m->n_pad;
-        CU(cudaMalloc(&m->timing[0], np * sizeof(int)));
-        CU(cudaMalloc(&m->timing[1], np * sizeof(int)));
-        CU(cudaMalloc(&m->timing_cold, np * sizeof(int)));
+        CU(m->timing[0].reserve(np));
+        CU(m->timing[1].reserve(np));
+        CU(m->timing_cold.reserve(np));
         {
             std::vector<int> t(np, 3);
             CU(cudaMemcpy(m->timing_cold, t.data(), np * sizeof(int), cudaMemcpyHostToDevice));
         }
-        CU(cudaMalloc(&m->win, (size_t) (np / 32) * WIN_ROWS * 32 * sizeof(float2)));
-        CU(cudaMalloc(&m->max_index, np * sizeof(int)));
-        CU(cudaMalloc(&m->max_value, np * sizeof(float)));
-        CU(cudaMalloc(&m->hist, (size_t) m->n * FRAME * sizeof(int16_t)));
+        CU(m->win.reserve((size_t) (np / 32) * WIN_ROWS * 32));
+        CU(m->max_index.reserve(np));
+        CU(m->max_value.reserve(np));
+        CU(m->hist.reserve((size_t) m->n * FRAME));
         CU(cudaMemset(m->hist, 0, (size_t) m->n * FRAME * sizeof(int16_t)));
-        CU(cudaMalloc(&m->rx_phase, sizeof(float2)));
+        CU(m->rx_phase.reserve(1));
         if (m->packet) {
-            CU(cudaMalloc(&m->pk_hist2, (size_t) m->n * FRAME * sizeof(int16_t)));
+            CU(m->pk_hist2.reserve((size_t) m->n * FRAME));
             CU(cudaMemset(m->pk_hist2, 0, (size_t) m->n * FRAME * sizeof(int16_t)));
-            CU(cudaMalloc(&m->pk_mix_hist2, (size_t) FRAME * sizeof(float2)));
+            CU(m->pk_mix_hist2.reserve(FRAME));
             CU(cudaMemset(m->pk_mix_hist2, 0, (size_t) FRAME * sizeof(float2)));
-            CU(cudaMalloc(&m->pk_n_host_dev, sizeof(unsigned long long)));
+            CU(m->pk_n_host_dev.reserve(1));
         }
-        CU(cudaMalloc(&m->unit_phase, sizeof(float2)));
+        CU(m->unit_phase.reserve(1));
         {
             const float2 one = make_float2(1.0f, 0.0f);
             CU(cudaMemcpy(m->unit_phase, &one, sizeof one, cudaMemcpyHostToDevice));
@@ -286,13 +324,13 @@ extern "C" int sc_create(sc_modem **out, int device, int64_t n_streams, uint32_t
         }
         if (const char *e = getenv("SC_H2D_MODE")) m->h2d_mode = std::max(0, std::min(atoi(e), (int) SC_H2D_COLUMNS_3D));
         for (int i = 0; i < N_PIPE; i++) {
-            CU(cudaStreamCreateWithFlags(&m->pipe[i], cudaStreamNonBlocking));
-            CU(cudaEventCreateWithFlags(&m->ev_done[i], cudaEventDisableTiming));
+            CU(m->pipe[i].create());
+            CU(m->ev_done[i].create());
         }
-        CU(cudaEventCreateWithFlags(&m->ev_start, cudaEventDisableTiming));
-        CU(cudaStreamCreateWithFlags(&m->tab_stream, cudaStreamNonBlocking));
-        CU(cudaEventCreateWithFlags(&m->ev_tab1, cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&m->ev_tab2, cudaEventDisableTiming));
+        CU(m->ev_start.create());
+        CU(m->tab_stream.create());
+        CU(m->ev_tab1.create());
+        CU(m->ev_tab2.create());
         return modem_cold(m);
     };
     rc = body();
@@ -304,86 +342,35 @@ extern "C" int sc_create(sc_modem **out, int device, int64_t n_streams, uint32_t
     return SC_OK;
 }
 
+// The device-wide synchronisation also covers the caller's streams, on which a device-path batch queues work that
+// touches handle memory.
 extern "C" void sc_destroy(sc_modem *m) {
     if (!m) return;
     cudaSetDevice(m->device);
     cudaDeviceSynchronize();
-    cudaFree(m->timing[0]);
-    cudaFree(m->timing[1]);
-    cudaFree(m->timing_cold);
-    for (cudaEvent_t e : m->ev_fe) cudaEventDestroy(e);
-    for (cudaEvent_t e : m->ev_tk) cudaEventDestroy(e);
-    cudaFree(m->win);
-    cudaFree(m->max_index);
-    cudaFree(m->max_value);
-    cudaFree(m->hist);
-    cudaFree(m->rx_phase);
-    cudaFree(m->mix_table);
-    cudaFree(m->unit_phase);
-    cudaFree(m->pk_hist2);
-    cudaFree(m->pk_mix_hist2);
-    cudaFree(m->pk_n_host_dev);
-    cudaFree(m->pk_stage);
-    cudaFree(m->pk_sym_stage);
-    for (int i = 0; i < N_PIPE; i++) {
-        cudaFree(m->pk_t_before[i]);
-        cudaFree(m->pk_t_at[i]);
-        cudaFree(m->pk_list[i]);
-        cudaFree(m->pk_count[i]);
-        cudaFree(m->pk_sym[i]);
-        if (m->pk_stream[i]) cudaStreamDestroy(m->pk_stream[i]);
-        if (m->pk_ev_go[i]) cudaEventDestroy(m->pk_ev_go[i]);
-        if (m->pk_ev_done[i]) cudaEventDestroy(m->pk_ev_done[i]);
-    }
-    for (int i = 0; i < N_PIPE; i++) {
-        cudaFree(m->stage_in[i]);
-        cudaFree(m->stage_res[i]);
-        cudaFree(m->stage_eq[i]);
-        cudaFree(m->stage_sym[i]);
-        if (m->pipe[i]) cudaStreamDestroy(m->pipe[i]);
-        if (m->ev_done[i]) cudaEventDestroy(m->ev_done[i]);
-    }
-    for (int q = 0; q < OV_RING; q++) {
-        cudaFree(m->ov_win[q]);
-        cudaFree(m->ov_max_index[q]);
-        cudaFree(m->ov_max_value[q]);
-        cudaFree(m->ov_state[q]);
-        cudaFree(m->ov_timing[q]);
-    }
-    for (int i = 0; i < N_PIPE; i++) {
-        if (m->ov_stream[i]) cudaStreamDestroy(m->ov_stream[i]);
-        for (int q = 0; q < 2; q++)
-            if (m->ov_data[i][q]) cudaStreamDestroy(m->ov_data[i][q]);
-        if (m->ov_ev_first[i]) cudaEventDestroy(m->ov_ev_first[i]);
-        for (int q = 0; q < 3; q++)
-            if (m->ov_join[i][q]) cudaEventDestroy(m->ov_join[i][q]);
-        for (int q = 0; q < OV_RING; q++) {
-            if (m->ov_ev_fe[i][q]) cudaEventDestroy(m->ov_ev_fe[i][q]);
-            if (m->ov_ev_train[i][q]) cudaEventDestroy(m->ov_ev_train[i][q]);
-            if (m->ov_ev_data[i][q]) cudaEventDestroy(m->ov_ev_data[i][q]);
-        }
-    }
-    if (m->ev_start) cudaEventDestroy(m->ev_start);
-    if (m->tab_stream) cudaStreamDestroy(m->tab_stream);
-    if (m->ev_tab1) cudaEventDestroy(m->ev_tab1);
-    if (m->ev_tab2) cudaEventDestroy(m->ev_tab2);
-    for (cudaEvent_t e : m->ev_tabc) cudaEventDestroy(e);
-    cudaGetLastError();
     delete m;
+    cudaGetLastError();
 }
 
-extern "C" int sc_reset(sc_modem *m) {
-    if (!m) return fail(SC_EINVAL, "sc_reset: null handle");
+// Wait for everything queued on the handle's own streams (a batch that failed part-way may have left the overlapped
+// chains' side streams unjoined: every successful batch joins them into the pipes).
+static int drain(sc_modem *m) {
     CU(cudaSetDevice(m->device));
     for (int i = 0; i < N_PIPE; i++) CU(cudaStreamSynchronize(m->pipe[i]));
     CU(cudaStreamSynchronize(m->tab_stream));
-    if (m->ov_ready)                    // a batch that failed part-way may have left the chains' side streams unjoined
+    if (m->ov_ready)
         for (int i = 0; i < N_PIPE; i++) {
             CU(cudaStreamSynchronize(m->ov_stream[i]));
             CU(cudaStreamSynchronize(m->ov_data[i][0]));
             CU(cudaStreamSynchronize(m->ov_data[i][1]));
         }
-    return modem_cold(m);
+    return SC_OK;
+}
+
+extern "C" int sc_reset(sc_modem *m) {
+    if (!m) return fail(SC_EINVAL, "sc_reset: null handle");
+    int rc = drain(m);
+    return rc != SC_OK ? rc : modem_cold(m);
 }
 
 // SC_OV_TRACE=1: time stamps (CUDA events) after every launch of the overlapped chains, printed per batch -- a
@@ -415,18 +402,16 @@ static OvTrace g_trace;
 // Make sure the mix table can hold slot 0 + n_frames frames and generate this batch's phasors
 // (calls call .. call+n_frames-1 into slots 1..n_frames) on stream st.
 static int prepare_tables(sc_modem *m, int n_frames, cudaStream_t st) {
-    if (m->mix_cap < n_frames + 1) {
-        float2 *nt = nullptr;
-        CU(cudaMalloc(&nt, (size_t) (n_frames + 1) * FRAME * sizeof(float2)));
+    if (m->mix_table.cap < (size_t) (n_frames + 1) * FRAME) {          // a larger table, keeping slot 0
+        DevBuf<float2> nt;
+        CU(nt.reserve((size_t) (n_frames + 1) * FRAME));
         if (m->mix_table) {
             CU(cudaMemcpyAsync(nt, m->mix_table, (size_t) FRAME * sizeof(float2), cudaMemcpyDeviceToDevice, st));
             CU(cudaStreamSynchronize(st));
-            CU(cudaFree(m->mix_table));
         } else {
             CU(cudaMemsetAsync(nt, 0, (size_t) FRAME * sizeof(float2), st));
         }
-        m->mix_table = nt;
-        m->mix_cap = n_frames + 1;
+        m->mix_table = std::move(nt);                                   // the old table goes with nt
     }
     // stored pre-multiplied by 1/16384: phasor*((float)in/16384) == (phasor/16384)*(float)in exactly.
     // Head on st (the calls wait for it); the rest on tab_stream in pieces, so that a call waits only for the piece
@@ -438,11 +423,8 @@ static int prepare_tables(sc_modem *m, int n_frames, cudaStream_t st) {
     g_trace.mark("tabhead", (uint32_t) head, 0, st);
     CU(cudaStreamWaitEvent(m->tab_stream, m->ev_tab1, 0));
     for (int f = head, c = 0; f < n_frames; f += TAB_CHUNK, c++) {
-        if ((int) m->ev_tabc.size() <= c) {
-            cudaEvent_t e;
-            CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            m->ev_tabc.push_back(e);
-        }
+        if ((int) m->ev_tabc.size() <= c) m->ev_tabc.emplace_back();
+        CU(m->ev_tabc[c].create());
         CU(launch_nco_table(m->rx_phase, m->rx_rect, NCO_RX, 0, std::min(TAB_CHUNK, n_frames - f), 1.0f / 16384.0f,
                             m->mix_table + (size_t) (f + 1) * FRAME, m->tab_stream));
         CU(cudaEventRecord(m->ev_tabc[c], m->tab_stream));
@@ -464,18 +446,14 @@ static int table_wait(sc_modem *m, cudaStream_t st, int slot, int &waited) {
     return SC_OK;
 }
 
-static cudaError_t prof_mark(std::vector<cudaEvent_t> &v, cudaStream_t st) {
-    cudaEvent_t e;
-    cudaError_t rc = cudaEventCreate(&e);
+static cudaError_t prof_mark(std::vector<Event> &v, cudaStream_t st) {
+    Event e;
+    cudaError_t rc = e.create(cudaEventDefault);
     if (rc != cudaSuccess) return rc;
-    v.push_back(e);
-    return cudaEventRecord(e, st);
+    v.push_back(std::move(e));
+    return cudaEventRecord(v.back(), st);
 }
 
-// One slab of streams [s0, s0+ns): the call loop.  `in` points at stream s0's first sample of the
-// first frame of this block, `results`/`eq_dbg` at stream s0's record of the block's first call.
-// call0 = index of the block's first call; kw = its keystream words; mix0 = table slot of frame
-// call0-1 (the frame filtered by call call0).
 struct PacketSink {
     sc_packet_result *packets = nullptr;    // device
     int64_t capacity = 0;
@@ -486,18 +464,18 @@ static const int PK_CAP = 65536;            // listed packets per pass; slabs ar
 
 // scratch of the packet pass, once per handle
 static int packet_scratch(sc_modem *m) {
-    if (m->pk_slab_cap) return SC_OK;
+    if (m->pk_ready) return SC_OK;
     for (int i = 0; i < N_PIPE; i++) {
-        CU(cudaMalloc(&m->pk_t_before[i], (size_t) PK_CAP * sizeof(int)));
-        CU(cudaMalloc(&m->pk_t_at[i], (size_t) PK_CAP * sizeof(int)));
-        CU(cudaMalloc(&m->pk_list[i], (size_t) PK_CAP * sizeof(int2)));
-        CU(cudaMalloc(&m->pk_count[i], sizeof(int)));
-        CU(cudaMalloc(&m->pk_sym[i], (size_t) (PK_CAP / 32) * PK_SYMS * 32 * sizeof(float2)));
-        CU(cudaStreamCreateWithFlags(&m->pk_stream[i], cudaStreamNonBlocking));
-        CU(cudaEventCreateWithFlags(&m->pk_ev_go[i], cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&m->pk_ev_done[i], cudaEventDisableTiming));
+        CU(m->pk_t_before[i].reserve(PK_CAP));
+        CU(m->pk_t_at[i].reserve(PK_CAP));
+        CU(m->pk_list[i].reserve(PK_CAP));
+        CU(m->pk_count[i].reserve(1));
+        CU(m->pk_sym[i].reserve((size_t) (PK_CAP / 32) * PK_SYMS * 32));
+        CU(m->pk_stream[i].create());
+        CU(m->pk_ev_go[i].create());
+        CU(m->pk_ev_done[i].create());
     }
-    m->pk_slab_cap = PK_CAP;
+    m->pk_ready = true;
     return SC_OK;
 }
 
@@ -506,24 +484,64 @@ static int overlap_scratch(sc_modem *m) {
     if (m->ov_ready) return SC_OK;
     const int64_t np = m->n_pad;
     for (int q = 0; q < OV_RING; q++) {
-        CU(cudaMalloc(&m->ov_win[q], (size_t) (np / 32) * WIN_ROWS_OV * 32 * sizeof(float2)));
-        CU(cudaMalloc(&m->ov_max_index[q], np * sizeof(int)));
-        CU(cudaMalloc(&m->ov_max_value[q], np * sizeof(float)));
-        CU(cudaMalloc(&m->ov_state[q], (size_t) np * TRK_STATE_WORDS * sizeof(float)));
-        CU(cudaMalloc(&m->ov_timing[q], np * sizeof(int)));
+        CU(m->ov_win[q].reserve((size_t) (np / 32) * WIN_ROWS_OV * 32));
+        CU(m->ov_max_index[q].reserve(np));
+        CU(m->ov_max_value[q].reserve(np));
+        CU(m->ov_state[q].reserve((size_t) np * TRK_STATE_WORDS));
+        CU(m->ov_timing[q].reserve(np));
     }
     for (int i = 0; i < N_PIPE; i++) {
-        CU(cudaStreamCreateWithFlags(&m->ov_stream[i], cudaStreamNonBlocking));
-        for (int q = 0; q < 2; q++) CU(cudaStreamCreateWithFlags(&m->ov_data[i][q], cudaStreamNonBlocking));
-        CU(cudaEventCreateWithFlags(&m->ov_ev_first[i], cudaEventDisableTiming));
-        for (int q = 0; q < 3; q++) CU(cudaEventCreateWithFlags(&m->ov_join[i][q], cudaEventDisableTiming));
+        CU(m->ov_stream[i].create());
+        for (int q = 0; q < 2; q++) CU(m->ov_data[i][q].create());
+        CU(m->ov_ev_first[i].create());
+        for (int q = 0; q < 3; q++) CU(m->ov_join[i][q].create());
         for (int q = 0; q < OV_RING; q++) {
-            CU(cudaEventCreateWithFlags(&m->ov_ev_fe[i][q], cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&m->ov_ev_train[i][q], cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&m->ov_ev_data[i][q], cudaEventDisableTiming));
+            CU(m->ov_ev_fe[i][q].create());
+            CU(m->ov_ev_train[i][q].create());
+            CU(m->ov_ev_data[i][q].create());
         }
     }
     m->ov_ready = true;
+    return SC_OK;
+}
+
+// One slab of streams [s0, s0+ns) over one block of frames, queued on st.  `in` points at stream s0's first sample of
+// the block's first frame, `results`/`eq_dbg`/`sym` at stream s0's record of the block's first call.  The block begins
+// slot0 frames into the batch: its first call is m->call + slot0, with keystream word m->kw[slot0], and filters the
+// frame whose phasors are in table slot slot0.
+struct Slab {
+    cudaStream_t st;
+    int pipe;
+    int64_t s0;
+    int ns;
+    const int16_t *in;
+    int64_t stride;
+    int n_frames;
+    int slot0;
+    sc_frame_result *results;
+    int64_t result_stride;
+    float *eq_dbg, *sym;
+    const PacketSink *pk;
+};
+
+// the frame fe(n) filters, for call n = call0 + j: frame j-1 of the block, or the last one of the previous block
+static const int16_t *fe_frame(const sc_modem *m, const Slab &s, int j, int64_t &fstride) {
+    fstride = j >= 1 ? s.stride : FRAME;
+    return j >= 1 ? s.in + (size_t) (j - 1) * FRAME : m->hist + (size_t) s.s0 * FRAME;
+}
+
+// The block's last frame becomes the history of the next block; in packet mode the one before it too (from this block
+// if it has two, else the frame the previous block saved).
+static int store_history(sc_modem *m, const Slab &s) {
+    const size_t pitch = FRAME * sizeof(int16_t), spitch = (size_t) s.stride * sizeof(int16_t);
+    int16_t *hist = m->hist + (size_t) s.s0 * FRAME;
+    if (m->packet && s.n_frames >= 2)
+        CU(cudaMemcpy2DAsync(m->pk_hist2 + (size_t) s.s0 * FRAME, pitch, s.in + (size_t) (s.n_frames - 2) * FRAME, spitch,
+                             pitch, (size_t) s.ns, cudaMemcpyDeviceToDevice, s.st));
+    else if (m->packet)
+        CU(cudaMemcpyAsync(m->pk_hist2 + (size_t) s.s0 * FRAME, hist, (size_t) s.ns * pitch, cudaMemcpyDeviceToDevice, s.st));
+    CU(cudaMemcpy2DAsync(hist, pitch, s.in + (size_t) (s.n_frames - 1) * FRAME, spitch, pitch, (size_t) s.ns,
+                         cudaMemcpyDeviceToDevice, s.st));
     return SC_OK;
 }
 
@@ -541,14 +559,17 @@ static int overlap_scratch(sc_modem *m) {
 // fe(k+3), which therefore waits for data(k).
 // The batch's first call runs the uncut tracker on the window the previous batch left (m->win, the serial layout) and
 // the last call's front-end writes that layout again, so the state between batches does not depend on the mode.
-static int run_slab_overlapped(sc_modem *m, cudaStream_t st, int pipe, int64_t s0, int ns, const int16_t *in,
-                               int64_t stride, int n_frames, uint32_t call0, const uint64_t *kw, const float2 *mix0,
-                               int slot0, sc_frame_result *results, int64_t result_stride, float *sym, bool save_hist,
-                               bool coop) {
+static int run_slab_overlapped(sc_modem *m, const Slab &s, bool coop) {
     int rc = overlap_scratch(m);
     if (rc != SC_OK) return rc;
+    const cudaStream_t st = s.st;
+    const int pipe = s.pipe, ns = s.ns, n_frames = s.n_frames, slot0 = s.slot0;
+    const int64_t s0 = s.s0;
+    const uint32_t call0 = m->call + (uint32_t) slot0;
+    const uint64_t *kw = m->kw.data() + slot0;
+    const float2 *mix0 = m->mix_table + (size_t) slot0 * FRAME;
     cudaStream_t C[2];
-    cudaStream_t *Dn = m->ov_data[pipe];
+    const Stream *Dn = m->ov_data[pipe];
     C[call0 & 1] = st;
     C[(call0 & 1) ^ 1] = m->ov_stream[pipe];
     CU(cudaEventRecord(m->ov_join[pipe][0], st));                   // the other streams start where st stands
@@ -574,26 +595,20 @@ static int run_slab_overlapped(sc_modem *m, cudaStream_t st, int pipe, int64_t s
         }
         return ts;
     };
-    auto frame_of = [&](uint32_t n, const int16_t *&frame, int64_t &fstride) {   // fe(n) filters frame n-1
-        const int j = (int) (n - call0);
-        frame = j >= 1 ? in + (size_t) (j - 1) * FRAME : m->hist + (size_t) s0 * FRAME;
-        fstride = j >= 1 ? stride : FRAME;
-    };
 
     // ---- the first call, and the window the second one reads
     {
         const int p = (int) (call0 & 1), q = p ^ 1;
         NvtxRange range("sc:track_kernel");
         CU(launch_track(false, win, m->max_index + s0, m->max_value + s0, m->timing[p] + s0,
-                        m->ov_timing[(call0 + 1) % OV_RING] + s0, results, result_stride, nullptr, nullptr, call0, kw[0], ns,
-                        C[p], coop, sym));
+                        m->ov_timing[(call0 + 1) % OV_RING] + s0, s.results, s.result_stride, nullptr, nullptr, call0, kw[0],
+                        ns, C[p], coop, s.sym));
         trace.mark("track", call0, p, C[p]);
         CU(cudaEventRecord(m->ov_ev_first[pipe], C[p]));
         const uint32_t k = call0 + 1;                               // consumer of fe(call0)
         if (call0 >= 1) {
-            const int16_t *frame;
             int64_t fstride;
-            frame_of(call0, frame, fstride);
+            const int16_t *frame = fe_frame(m, s, 0, fstride);
             if ((rc = table_wait(m, C[q], slot0, tab_waited[q])) != SC_OK) return rc;
             NvtxRange range2("sc:frontend_kernel");
             CU(launch_frontend(m->wide, frame, fstride, mix0, m->timing[p] + s0, nullptr, m->ov_win[k % OV_RING] + tile_ov,
@@ -617,9 +632,8 @@ static int run_slab_overlapped(sc_modem *m, cudaStream_t st, int pipe, int64_t s
         if (n < last) {
             // fe(n) on the other chain, behind train(n-1) (or the first call): T_n from slot n-1, or as the first call stored it
             const uint32_t k = n + 1;
-            const int16_t *frame;
             int64_t fstride;
-            frame_of(n, frame, fstride);
+            const int16_t *frame = fe_frame(m, s, j, fstride);
             CU(cudaStreamWaitEvent(C[q], m->ov_ev_fe[pipe][(n - 1) % OV_RING], 0));       // T_{n-1}
             if (n >= call0 + 4) CU(cudaStreamWaitEvent(C[q], m->ov_ev_data[pipe][(n - 3) % OV_RING], 0));   // slot k is free
             if ((rc = table_wait(m, C[q], slot0 + j, tab_waited[q])) != SC_OK) return rc;
@@ -644,9 +658,9 @@ static int run_slab_overlapped(sc_modem *m, cudaStream_t st, int pipe, int64_t s
             const TimingSrc ts = n < last ? TimingSrc() : timing_src(n, nullptr);
             NvtxRange range("sc:track_data");
             CU(launch_track_data(m->ov_win[r] + tile_ov, state_of(n), m->n_pad, m->ov_max_index[r] + s0, m->ov_max_value[r] + s0,
-                                 m->ov_timing[r] + s0, n == last ? m->timing[(n + 1) & 1] + s0 : nullptr, results + j,
-                                 result_stride, n, kw[j], ns, D, coop, &ts, n == last ? m->timing[n & 1] + s0 : nullptr,
-                                 sym ? sym + (size_t) j * SYM_FLOATS : nullptr));
+                                 m->ov_timing[r] + s0, n == last ? m->timing[(n + 1) & 1] + s0 : nullptr, s.results + j,
+                                 s.result_stride, n, kw[j], ns, D, coop, &ts, n == last ? m->timing[n & 1] + s0 : nullptr,
+                                 s.sym ? s.sym + (size_t) j * SYM_FLOATS : nullptr));
             trace.mark("data", n, 2 + p, D);
             CU(cudaEventRecord(m->ov_ev_data[pipe][r], D));
         }
@@ -654,9 +668,8 @@ static int run_slab_overlapped(sc_modem *m, cudaStream_t st, int pipe, int64_t s
     {
         // the last call's front-end in the serial layout: window, max_index and both rx_timing arrays for the next batch
         cudaStream_t D = Dn[last & 1];
-        const int16_t *frame;
         int64_t fstride;
-        frame_of(last, frame, fstride);
+        const int16_t *frame = fe_frame(m, s, n_frames - 1, fstride);
         if ((rc = table_wait(m, D, slot0 + n_frames - 1, tab_waited_d)) != SC_OK) return rc;
         NvtxRange range("sc:frontend_kernel");
         CU(launch_frontend(m->wide, frame, fstride, mix0 + (size_t) (n_frames - 1) * FRAME, m->timing[last & 1] + s0,
@@ -668,16 +681,20 @@ static int run_slab_overlapped(sc_modem *m, cudaStream_t st, int pipe, int64_t s
     CU(cudaEventRecord(m->ov_join[pipe][2], Dn[1]));
     for (int q = 0; q < 3; q++) CU(cudaStreamWaitEvent(st, m->ov_join[pipe][q], 0));
     trace.dump();
-    if (save_hist)
-        CU(cudaMemcpy2DAsync(m->hist + (size_t) s0 * FRAME, FRAME * sizeof(int16_t), in + (size_t) (n_frames - 1) * FRAME,
-                             (size_t) stride * sizeof(int16_t), FRAME * sizeof(int16_t), (size_t) ns, cudaMemcpyDeviceToDevice, st));
     return SC_OK;
 }
 
-static int run_slab(sc_modem *m, cudaStream_t st, int64_t s0, int ns, const int16_t *in, int64_t stride,
-                    int n_frames, uint32_t call0, const uint64_t *kw, const float2 *mix0, int slot0,
-                    sc_frame_result *results, int64_t result_stride, float *eq_dbg, float *sym, bool save_hist,
-                    const PacketSink *pk = nullptr, int pipe = 0) {
+// The call loop of one slab; afterwards the block's last frame (and in packet mode the one before it) is saved for the
+// block that follows.
+static int run_slab(sc_modem *m, const Slab &s) {
+    const cudaStream_t st = s.st;
+    const int pipe = s.pipe, ns = s.ns, n_frames = s.n_frames, slot0 = s.slot0;
+    const int64_t s0 = s.s0;
+    const PacketSink *pk = s.pk;
+    float *eq_dbg = s.eq_dbg;
+    const uint32_t call0 = m->call + (uint32_t) slot0;
+    const uint64_t *kw = m->kw.data() + slot0;
+    const float2 *mix0 = m->mix_table + (size_t) slot0 * FRAME;
     float2 *win = m->win + (size_t) (s0 / 32) * WIN_ROWS * 32;
     int tab_waited = -1;
     PacketSrc psrc;
@@ -687,10 +704,10 @@ static int run_slab(sc_modem *m, cudaStream_t st, int64_t s0, int ns, const int1
         // rx_timing at entry of calls call0-1 and call0 (the ping-pong arrays are overwritten as the calls run)
         CU(cudaMemcpyAsync(m->pk_t_before[pipe], m->timing[(call0 + 1) & 1] + s0, (size_t) ns * sizeof(int), cudaMemcpyDeviceToDevice, st));
         CU(cudaMemcpyAsync(m->pk_t_at[pipe], m->timing[call0 & 1] + s0, (size_t) ns * sizeof(int), cudaMemcpyDeviceToDevice, st));
-        psrc.results = results;
-        psrc.result_stride = result_stride;
-        psrc.in = in;
-        psrc.stride = stride;
+        psrc.results = s.results;
+        psrc.result_stride = s.result_stride;
+        psrc.in = s.in;
+        psrc.stride = s.stride;
         psrc.hist1 = m->hist + (size_t) s0 * FRAME;
         psrc.hist2 = m->pk_hist2 + (size_t) s0 * FRAME;
         psrc.mix0 = mix0;
@@ -704,9 +721,10 @@ static int run_slab(sc_modem *m, cudaStream_t st, int64_t s0, int ns, const int1
     }
     const bool tracker_coop = m->tracker == SC_TRACKER_COOP || (m->tracker == SC_TRACKER_AUTO && ns <= SC_TRACKER_COOP_MAX);
     const bool plain = !pk && !m->packet && !m->profile && !m->fe_search_mma && !eq_dbg && !m->state_dbg;
-    if (plain && n_frames >= 2 && (m->overlap == SC_OVERLAP_ON || (m->overlap == SC_OVERLAP_AUTO && m->n <= SC_OVERLAP_MAX)))
-        return run_slab_overlapped(m, st, pipe, s0, ns, in, stride, n_frames, call0, kw, mix0, slot0, results, result_stride,
-                                   sym, save_hist, tracker_coop);
+    if (plain && n_frames >= 2 && (m->overlap == SC_OVERLAP_ON || (m->overlap == SC_OVERLAP_AUTO && m->n <= SC_OVERLAP_MAX))) {
+        int rc = run_slab_overlapped(m, s, tracker_coop);
+        return rc != SC_OK ? rc : store_history(m, s);
+    }
     for (int j = 0; j < n_frames; j++) {
         const uint32_t n = call0 + (uint32_t) j;
         int *tc = m->timing[n & 1] + s0, *tn = m->timing[(n + 1) & 1] + s0;
@@ -714,21 +732,14 @@ static int run_slab(sc_modem *m, cudaStream_t st, int64_t s0, int ns, const int1
         {
             NvtxRange range("sc:track_kernel");
             CU(launch_track(m->debug_eq && eq_dbg != nullptr, win, m->max_index + s0, m->max_value + s0, tc, tn,
-                            results + j, result_stride, eq_dbg ? eq_dbg + (size_t) j * 10 : nullptr,
+                            s.results + j, s.result_stride, eq_dbg ? eq_dbg + (size_t) j * 10 : nullptr,
                             m->state_dbg ? m->state_dbg + (size_t) s0 * TRACK_STATE_FLOATS : nullptr, n, kw[j], ns, st, tracker_coop,
-                            sym ? sym + (size_t) j * SYM_FLOATS : nullptr));
+                            s.sym ? s.sym + (size_t) j * SYM_FLOATS : nullptr));
         }
         if (m->profile) CU(prof_mark(m->ev_tk, st));
         if (n >= 1) {
-            const int16_t *frame;
             int64_t fstride;
-            if (j >= 1) {
-                frame = in + (size_t) (j - 1) * FRAME;
-                fstride = stride;
-            } else {
-                frame = m->hist + (size_t) s0 * FRAME;
-                fstride = FRAME;
-            }
+            const int16_t *frame = fe_frame(m, s, j, fstride);
             int rcw = table_wait(m, st, slot0 + j, tab_waited);
             if (rcw != SC_OK) return rcw;
             if (m->profile) CU(prof_mark(m->ev_fe, st));
@@ -761,22 +772,7 @@ static int run_slab(sc_modem *m, cudaStream_t st, int64_t s0, int ns, const int1
         CU(cudaEventRecord(m->pk_ev_done[pipe], m->pk_stream[pipe]));
         CU(cudaStreamWaitEvent(st, m->pk_ev_done[pipe], 0));
     }
-    if (m->packet && save_hist && n_frames > 0) {
-        // the frame before the last one: from this block if it has two, else the frame saved by the previous block
-        if (n_frames >= 2)
-            CU(cudaMemcpy2DAsync(m->pk_hist2 + (size_t) s0 * FRAME, FRAME * sizeof(int16_t),
-                                 in + (size_t) (n_frames - 2) * FRAME, (size_t) stride * sizeof(int16_t),
-                                 FRAME * sizeof(int16_t), (size_t) ns, cudaMemcpyDeviceToDevice, st));
-        else
-            CU(cudaMemcpyAsync(m->pk_hist2 + (size_t) s0 * FRAME, m->hist + (size_t) s0 * FRAME,
-                               (size_t) ns * FRAME * sizeof(int16_t), cudaMemcpyDeviceToDevice, st));
-    }
-    if (save_hist && n_frames > 0) {
-        CU(cudaMemcpy2DAsync(m->hist + (size_t) s0 * FRAME, FRAME * sizeof(int16_t),
-                             in + (size_t) (n_frames - 1) * FRAME, (size_t) stride * sizeof(int16_t),
-                             FRAME * sizeof(int16_t), (size_t) ns, cudaMemcpyDeviceToDevice, st));
-    }
-    return SC_OK;
+    return store_history(m, s);
 }
 
 static int64_t pick_slab(int64_t n, int64_t lo, int64_t parts) {
@@ -786,104 +782,74 @@ static int64_t pick_slab(int64_t n, int64_t lo, int64_t parts) {
     return s;
 }
 
-// Common entry checks of the two batch entry points; the keystream words of the batch are drawn from a
-// COPY of the descrambler register, which is committed together with the call index only when the whole
-// batch has been queued (a failing call must not leave RXMemory ahead of m->call).
-static int rx_begin(sc_modem *m, const char *who, const int16_t *in, int64_t stream_stride, int n_frames,
-                    sc_frame_result *results, int64_t result_stride, float *eq_dbg, std::vector<uint64_t> &kw,
-                    uint16_t &lfsr) {
-    if (!m || !in || !results || n_frames < 0) return fail(SC_EINVAL, "%s: bad arguments", who);
-    if (m->poisoned) return fail(SC_ESTATE, "%s: an earlier batch failed part-way; call sc_reset() first", who);
-    if (n_frames == 0) return SC_OK;
-    if (stream_stride < (int64_t) n_frames * FRAME || result_stride < n_frames)
-        return fail(SC_EINVAL, "%s: stride smaller than the batch", who);
-    if (eq_dbg && !m->debug_eq) return fail(SC_EINVAL, "%s: eq_dbg needs SC_FLAG_DEBUG_EQ", who);
-    if (m->fe_search_mma) {                 // per batch, not per handle: sc_release_caches() may have freed the table
-        int rc = m->fe_search_umma ? search_umma_master(m->device, &m->search_umma_master)
-                                   : search_table(m->device, &m->search_a_table);
-        if (rc != SC_OK) return rc;
-    }
-    lfsr = m->lfsr_rx;
-    kw.resize(n_frames);
-    for (int j = 0; j < n_frames; j++) kw[j] = keystream_next_word(lfsr);
-    return SC_OK;
-}
+// One batch of any of the eight RX entry points (include/singlecarrier_b200.h): device or host buffers, the optional
+// equalizer outputs (eq_dbg of debug banks, sym of the soft forms) and, for the packet entry points, the records.
+struct RxBatch {
+    const char *who;
+    const int16_t *in;
+    int64_t stream_stride;
+    int n_frames;
+    sc_frame_result *results;
+    int64_t result_stride;
+    float *eq_dbg = nullptr, *sym = nullptr;
+    bool host = false;
+    cudaStream_t stream = nullptr;          // the caller's stream (device buffers)
+    bool packet_mode = false;
+    sc_packet_result *packets = nullptr;
+    int64_t capacity = 0;
+    uint64_t *n_packets = nullptr;
+    float *packet_symbols = nullptr;
+};
 
-static int rx_end(sc_modem *m, int rc, int n_frames, uint16_t lfsr) {
-    if (rc != SC_OK) {
-        if (m->in_flight) m->poisoned = true;      // something was launched: per-stream state is inconsistent
-        m->in_flight = false;
-        return rc;
-    }
-    m->in_flight = false;
-    m->lfsr_rx = lfsr;
-    m->call += (uint32_t) n_frames;
-    return SC_OK;
-}
-
-static int rx_frames_dev_body(sc_modem *m, const int16_t *in, int64_t stream_stride, int n_frames,
-                              sc_frame_result *results, int64_t result_stride, float *eq_dbg, float *sym,
-                              cudaStream_t user, const uint64_t *kw, const PacketSink *pk = nullptr) {
-    CU(cudaSetDevice(m->device));
-    // order after the caller's stream, build the tables once, fan out over the pipe streams
-    CU(cudaEventRecord(m->ev_start, user));
-    CU(cudaStreamWaitEvent(m->pipe[0], m->ev_start, 0));
+// Generate the batch's phasor tables on pipe[0] and order the other pipes after them.  The batch is in flight from
+// here: a failure from now on may leave some streams advanced and others not.
+static int start_tables(sc_modem *m, int n_frames) {
     m->in_flight = true;
     int rc = prepare_tables(m, n_frames, m->pipe[0]);
     if (rc != SC_OK) return rc;
     CU(cudaEventRecord(m->ev_start, m->pipe[0]));
     for (int i = 1; i < N_PIPE; i++) CU(cudaStreamWaitEvent(m->pipe[i], m->ev_start, 0));
+    return SC_OK;
+}
+
+// the last frame's phasors become slot 0 of the next batch, and in packet mode the one before it the table of frame call-2
+static int rotate_tables(sc_modem *m, int n_frames, cudaStream_t st) {
+    if (m->packet)
+        CU(cudaMemcpyAsync(m->pk_mix_hist2, m->mix_table + (size_t) (n_frames - 1) * FRAME, FRAME * sizeof(float2),
+                           cudaMemcpyDeviceToDevice, st));
+    CU(cudaMemcpyAsync(m->mix_table, m->mix_table + (size_t) n_frames * FRAME, FRAME * sizeof(float2),
+                       cudaMemcpyDeviceToDevice, st));
+    return SC_OK;
+}
+
+static int rx_dev_body(sc_modem *m, const RxBatch &b, const PacketSink *pk) {
+    CU(cudaSetDevice(m->device));
+    // order after the caller's stream, build the tables once, fan out over the pipe streams
+    CU(cudaEventRecord(m->ev_start, b.stream));
+    CU(cudaStreamWaitEvent(m->pipe[0], m->ev_start, 0));
+    int rc = start_tables(m, b.n_frames);
+    if (rc != SC_OK) return rc;
 
     // default: two slabs, each on its own stream, so one slab's tail waves overlap the other's kernels
     int64_t slab = pick_slab(m->n, m->slab_parts > 0 ? 128 : 8192, m->slab_parts > 0 ? m->slab_parts : 2);
     if (pk) slab = std::min<int64_t>(slab, PK_CAP);
     int k = 0;
     for (int64_t s0 = 0; s0 < m->n; s0 += slab, k++) {
-        const int ns = (int) std::min<int64_t>(slab, m->n - s0);
-        rc = run_slab(m, m->pipe[k % N_PIPE], s0, ns, in + (size_t) s0 * stream_stride, stream_stride, n_frames,
-                      m->call, kw, m->mix_table, 0, results + (size_t) s0 * result_stride, result_stride,
-                      eq_dbg ? eq_dbg + (size_t) s0 * result_stride * 10 : nullptr,
-                      sym ? sym + (size_t) s0 * result_stride * SYM_FLOATS : nullptr, true, pk, k % N_PIPE);
-        if (rc != SC_OK) return rc;
+        const Slab s = {m->pipe[k % N_PIPE], k % N_PIPE, s0, (int) std::min<int64_t>(slab, m->n - s0),
+                        b.in + (size_t) s0 * b.stream_stride, b.stream_stride, b.n_frames, 0,
+                        b.results + (size_t) s0 * b.result_stride, b.result_stride,
+                        b.eq_dbg ? b.eq_dbg + (size_t) s0 * b.result_stride * 10 : nullptr,
+                        b.sym ? b.sym + (size_t) s0 * b.result_stride * SYM_FLOATS : nullptr, pk};
+        if ((rc = run_slab(m, s)) != SC_OK) return rc;
     }
-    // the last frame's phasors become slot 0 of the next batch
     for (int i = 0; i < N_PIPE; i++) {
         CU(cudaEventRecord(m->ev_done[i], m->pipe[i]));
-        CU(cudaStreamWaitEvent(user, m->ev_done[i], 0));
+        CU(cudaStreamWaitEvent(b.stream, m->ev_done[i], 0));
     }
-    CU(cudaStreamWaitEvent(user, m->ev_tab2, 0));
-    if (m->packet)                                      // ... and the one before it the table of frame call-2
-        CU(cudaMemcpyAsync(m->pk_mix_hist2, m->mix_table + (size_t) (n_frames - 1) * FRAME, FRAME * sizeof(float2),
-                           cudaMemcpyDeviceToDevice, user));
-    CU(cudaMemcpyAsync(m->mix_table, m->mix_table + (size_t) n_frames * FRAME, FRAME * sizeof(float2),
-                       cudaMemcpyDeviceToDevice, user));
-    CU(cudaEventRecord(m->ev_start, user));
+    CU(cudaStreamWaitEvent(b.stream, m->ev_tab2, 0));
+    if ((rc = rotate_tables(m, b.n_frames, b.stream)) != SC_OK) return rc;
+    CU(cudaEventRecord(m->ev_start, b.stream));
     for (int i = 0; i < N_PIPE; i++) CU(cudaStreamWaitEvent(m->pipe[i], m->ev_start, 0));
-    return SC_OK;
-}
-
-extern "C" int sc_rx_frames_dev(sc_modem *m, const int16_t *in, int64_t stream_stride, int n_frames,
-                                sc_frame_result *results, int64_t result_stride, float *eq_dbg, void *stream) {
-    std::vector<uint64_t> kw;
-    uint16_t lfsr = 0;
-    int rc = rx_begin(m, "sc_rx_frames_dev", in, stream_stride, n_frames, results, result_stride, eq_dbg, kw, lfsr);
-    if (rc != SC_OK || n_frames == 0) return rc;
-    NvtxRange range("sc_rx_frames_dev");
-    rc = rx_frames_dev_body(m, in, stream_stride, n_frames, results, result_stride, eq_dbg, nullptr, (cudaStream_t) stream,
-                            kw.data());
-    return rx_end(m, rc, n_frames, lfsr);
-}
-
-template <typename T>
-static int grow(T **p, size_t *cap, size_t want, int count) {
-    if (*cap >= want) return SC_OK;
-    for (int i = 0; i < count; i++) {
-        if (p[i]) CU(cudaFree(p[i]));
-        p[i] = nullptr;
-        *cap = 0;
-        CU(cudaMalloc(&p[i], want));
-    }
-    *cap = want;
     return SC_OK;
 }
 
@@ -949,18 +915,17 @@ extern "C" int sc_transfer_bytes(const sc_modem *m, uint64_t out[2]) {
 
 static const size_t STAGE_BYTES = (size_t) 768 << 20;     // staging per pipe stream
 
-static int rx_frames_host_body(sc_modem *m, const int16_t *in, int64_t stream_stride, int n_frames,
-                               sc_frame_result *results, int64_t result_stride, float *eq_dbg, float *sym,
-                               const uint64_t *kw, const PacketSink *pk = nullptr) {
+static int rx_host_body(sc_modem *m, const RxBatch &b, const PacketSink *pk) {
     CU(cudaSetDevice(m->device));
     // slabs of streams x blocks of frames; slab k always runs on pipe k % N_PIPE, so its blocks
     // stay in order and the staging buffer of that pipe is reused safely (stream order)
+    const int n_frames = b.n_frames;
     const size_t frame_bytes = FRAME * sizeof(int16_t);
     int64_t slab;
     int fblk;
     // packet mode reads whole frames (the 248 data symbols reach past the columns the ordinary chain needs)
     const int h2d_mode = m->packet ? (int) SC_H2D_FULL : m->h2d_mode;
-    const bool contiguous = h2d_mode == SC_H2D_FULL && stream_stride == (int64_t) n_frames * FRAME &&
+    const bool contiguous = h2d_mode == SC_H2D_FULL && b.stream_stride == (int64_t) n_frames * FRAME &&
                             (size_t) n_frames * frame_bytes * 128 <= STAGE_BYTES;
     if (contiguous && m->slab_parts <= 0) {
         // all frames of a slab in one plain copy: as many streams as the staging buffer holds
@@ -973,16 +938,15 @@ static int rx_frames_host_body(sc_modem *m, const int16_t *in, int64_t stream_st
         if (pk) slab = std::min<int64_t>(slab, PK_CAP);
         fblk = (int) std::max<int64_t>(1, std::min<int64_t>(n_frames, (int64_t) STAGE_BYTES / (slab * (int64_t) frame_bytes)));
     }
-    int rc;
-    if ((rc = grow(m->stage_in, &m->stage_in_cap, (size_t) slab * fblk * frame_bytes, N_PIPE)) != SC_OK) return rc;
-    if ((rc = grow(m->stage_res, &m->stage_res_cap, (size_t) slab * fblk * sizeof(sc_frame_result), N_PIPE)) != SC_OK) return rc;
-    if (eq_dbg && (rc = grow(m->stage_eq, &m->stage_eq_cap, (size_t) slab * fblk * 10 * sizeof(float), N_PIPE)) != SC_OK) return rc;
-    if (sym && (rc = grow(m->stage_sym, &m->stage_sym_cap, (size_t) slab * fblk * SYM_BYTES, N_PIPE)) != SC_OK) return rc;
-
-    m->in_flight = true;
-    if ((rc = prepare_tables(m, n_frames, m->pipe[0])) != SC_OK) return rc;
-    CU(cudaEventRecord(m->ev_start, m->pipe[0]));
-    for (int i = 1; i < N_PIPE; i++) CU(cudaStreamWaitEvent(m->pipe[i], m->ev_start, 0));
+    const size_t records = (size_t) slab * fblk;
+    for (int p = 0; p < N_PIPE; p++) {
+        CU(m->stage_in[p].reserve(records * FRAME));
+        CU(m->stage_res[p].reserve(records));
+        if (b.eq_dbg) CU(m->stage_eq[p].reserve(records * 10));
+        if (b.sym) CU(m->stage_sym[p].reserve(records * SYM_FLOATS));
+    }
+    int rc = start_tables(m, n_frames);
+    if (rc != SC_OK) return rc;
 
     for (int f0 = 0; f0 < n_frames; f0 += fblk) {
         const int nf = std::min(fblk, n_frames - f0);
@@ -991,48 +955,112 @@ static int rx_frames_host_body(sc_modem *m, const int16_t *in, int64_t stream_st
             const int p = k % N_PIPE;
             cudaStream_t st = m->pipe[p];
             const int ns = (int) std::min<int64_t>(slab, m->n - s0);
-            const int64_t dstride = (int64_t) nf * FRAME;
-            if ((rc = h2d_block(m, h2d_mode, m->stage_in[p], in, stream_stride, s0, ns, f0, nf, st)) != SC_OK) return rc;
-            rc = run_slab(m, st, s0, ns, m->stage_in[p], dstride, nf, m->call + (uint32_t) f0, kw + f0,
-                          m->mix_table + (size_t) f0 * FRAME, f0, m->stage_res[p], nf, eq_dbg ? m->stage_eq[p] : nullptr,
-                          sym ? m->stage_sym[p] : nullptr, true, pk, p);
-            if (rc != SC_OK) return rc;
+            if ((rc = h2d_block(m, h2d_mode, m->stage_in[p], b.in, b.stream_stride, s0, ns, f0, nf, st)) != SC_OK) return rc;
+            const Slab s = {st, p, s0, ns, m->stage_in[p], (int64_t) nf * FRAME, nf, f0, m->stage_res[p], nf,
+                            b.eq_dbg ? m->stage_eq[p].p : nullptr, b.sym ? m->stage_sym[p].p : nullptr, pk};
+            if ((rc = run_slab(m, s)) != SC_OK) return rc;
             NvtxRange range("sc:d2h");
-            m->d2h_bytes += (size_t) nf * sizeof(sc_frame_result) * (size_t) ns + (eq_dbg ? (size_t) nf * 10 * sizeof(float) * (size_t) ns : 0) +
-                            (sym ? (size_t) nf * SYM_BYTES * (size_t) ns : 0);
-            CU(cudaMemcpy2DAsync(results + (size_t) s0 * result_stride + f0, (size_t) result_stride * sizeof(sc_frame_result),
+            m->d2h_bytes += (size_t) nf * sizeof(sc_frame_result) * (size_t) ns + (b.eq_dbg ? (size_t) nf * 10 * sizeof(float) * (size_t) ns : 0) +
+                            (b.sym ? (size_t) nf * SYM_BYTES * (size_t) ns : 0);
+            CU(cudaMemcpy2DAsync(b.results + (size_t) s0 * b.result_stride + f0, (size_t) b.result_stride * sizeof(sc_frame_result),
                                  m->stage_res[p], (size_t) nf * sizeof(sc_frame_result),
                                  (size_t) nf * sizeof(sc_frame_result), (size_t) ns, cudaMemcpyDeviceToHost, st));
-            if (eq_dbg)
-                CU(cudaMemcpy2DAsync(eq_dbg + ((size_t) s0 * result_stride + f0) * 10, (size_t) result_stride * 10 * sizeof(float),
+            if (b.eq_dbg)
+                CU(cudaMemcpy2DAsync(b.eq_dbg + ((size_t) s0 * b.result_stride + f0) * 10, (size_t) b.result_stride * 10 * sizeof(float),
                                      m->stage_eq[p], (size_t) nf * 10 * sizeof(float), (size_t) nf * 10 * sizeof(float),
                                      (size_t) ns, cudaMemcpyDeviceToHost, st));
-            if (sym)
-                CU(cudaMemcpy2DAsync(sym + ((size_t) s0 * result_stride + f0) * SYM_FLOATS, (size_t) result_stride * SYM_BYTES,
+            if (b.sym)
+                CU(cudaMemcpy2DAsync(b.sym + ((size_t) s0 * b.result_stride + f0) * SYM_FLOATS, (size_t) b.result_stride * SYM_BYTES,
                                      m->stage_sym[p], (size_t) nf * SYM_BYTES, (size_t) nf * SYM_BYTES, (size_t) ns,
                                      cudaMemcpyDeviceToHost, st));
         }
     }
     for (int i = 0; i < N_PIPE; i++) CU(cudaStreamSynchronize(m->pipe[i]));
     CU(cudaStreamSynchronize(m->tab_stream));
-    if (m->packet)
-        CU(cudaMemcpyAsync(m->pk_mix_hist2, m->mix_table + (size_t) (n_frames - 1) * FRAME, FRAME * sizeof(float2),
-                           cudaMemcpyDeviceToDevice, m->pipe[0]));
-    CU(cudaMemcpyAsync(m->mix_table, m->mix_table + (size_t) n_frames * FRAME, FRAME * sizeof(float2),
-                       cudaMemcpyDeviceToDevice, m->pipe[0]));
+    if ((rc = rotate_tables(m, n_frames, m->pipe[0])) != SC_OK) return rc;
     CU(cudaStreamSynchronize(m->pipe[0]));
     return SC_OK;
 }
 
+// Checks, the batch's keystream words and the packet sink, then the device or host body.  The words are drawn from a
+// COPY of the descrambler register, which is committed together with the call index only when the whole batch has
+// been queued (a failing call must not leave RXMemory ahead of m->call).
+static int rx_batch(sc_modem *m, const RxBatch &b) {
+    const char *who = b.who;
+    if (b.packet_mode) {
+        if (!m || !b.packets || b.capacity < 0 || !b.n_packets) return fail(SC_EINVAL, "%s: bad arguments", who);
+        if (!m->packet) return fail(SC_EINVAL, "%s: the bank was not created with SC_FLAG_PACKET", who);
+        int rc = packet_scratch(m);
+        if (rc != SC_OK) return rc;
+        if (b.host) *b.n_packets = 0;
+    }
+    if (!m || !b.in || !b.results || b.n_frames < 0) return fail(SC_EINVAL, "%s: bad arguments", who);
+    if (m->poisoned) return fail(SC_ESTATE, "%s: an earlier batch failed part-way; call sc_reset() first", who);
+    if (b.n_frames == 0) return SC_OK;
+    if (b.stream_stride < (int64_t) b.n_frames * FRAME || b.result_stride < b.n_frames)
+        return fail(SC_EINVAL, "%s: stride smaller than the batch", who);
+    if (b.eq_dbg && !m->debug_eq) return fail(SC_EINVAL, "%s: eq_dbg needs SC_FLAG_DEBUG_EQ", who);
+    if (m->fe_search_mma) {                 // per batch, not per handle: sc_release_caches() may have freed the table
+        int rc = m->fe_search_umma ? search_umma_master(m->device, &m->search_umma_master)
+                                   : search_table(m->device, &m->search_a_table);
+        if (rc != SC_OK) return rc;
+    }
+    uint16_t lfsr = m->lfsr_rx;
+    m->kw.resize(b.n_frames);
+    for (int j = 0; j < b.n_frames; j++) m->kw[j] = keystream_next_word(lfsr);
+    NvtxRange range(who);
+
+    PacketSink sink;
+    if (b.packet_mode && b.host) {          // the records are staged on the device and read back below
+        CU(cudaSetDevice(m->device));
+        CU(m->pk_stage.reserve((size_t) b.capacity));
+        if (b.packet_symbols) CU(m->pk_sym_stage.reserve((size_t) b.capacity * PK_DATA));
+        CU(cudaMemset(m->pk_n_host_dev, 0, sizeof(unsigned long long)));
+        sink = {m->pk_stage, b.capacity, m->pk_n_host_dev, b.packet_symbols ? m->pk_sym_stage.p : nullptr};
+    } else if (b.packet_mode) {
+        sink = {b.packets, b.capacity, (unsigned long long *) b.n_packets, reinterpret_cast<float2 *>(b.packet_symbols)};
+    }
+    const PacketSink *pk = b.packet_mode ? &sink : nullptr;
+    int rc = b.host ? rx_host_body(m, b, pk) : rx_dev_body(m, b, pk);
+    if (rc == SC_OK && b.packet_mode && b.host) {
+        unsigned long long n = 0;
+        cudaError_t e = cudaMemcpy(&n, m->pk_n_host_dev, sizeof n, cudaMemcpyDeviceToHost);
+        const size_t kept = (size_t) std::min<unsigned long long>(n, (unsigned long long) b.capacity);
+        if (e == cudaSuccess && n > 0)
+            e = cudaMemcpy(b.packets, m->pk_stage, kept * sizeof(sc_packet_result), cudaMemcpyDeviceToHost);
+        if (e == cudaSuccess && n > 0 && b.packet_symbols)
+            e = cudaMemcpy(b.packet_symbols, m->pk_sym_stage, kept * PK_DATA * sizeof(float2), cudaMemcpyDeviceToHost);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            rc = fail(SC_ECUDA, "%s: %s", who, cudaGetErrorString(e));
+        }
+        *b.n_packets = n;
+    }
+    if (rc != SC_OK) {
+        if (m->in_flight) m->poisoned = true;      // something was launched: per-stream state is inconsistent
+        m->in_flight = false;
+        return rc;
+    }
+    m->in_flight = false;
+    m->lfsr_rx = lfsr;
+    m->call += (uint32_t) b.n_frames;
+    return SC_OK;
+}
+
+extern "C" int sc_rx_frames_dev(sc_modem *m, const int16_t *in, int64_t stream_stride, int n_frames,
+                                sc_frame_result *results, int64_t result_stride, float *eq_dbg, void *stream) {
+    RxBatch b = {"sc_rx_frames_dev", in, stream_stride, n_frames, results, result_stride};
+    b.eq_dbg = eq_dbg;
+    b.stream = (cudaStream_t) stream;
+    return rx_batch(m, b);
+}
+
 extern "C" int sc_rx_frames_host(sc_modem *m, const int16_t *in, int64_t stream_stride, int n_frames,
                                  sc_frame_result *results, int64_t result_stride, float *eq_dbg) {
-    std::vector<uint64_t> kw;
-    uint16_t lfsr = 0;
-    int rc = rx_begin(m, "sc_rx_frames_host", in, stream_stride, n_frames, results, result_stride, eq_dbg, kw, lfsr);
-    if (rc != SC_OK || n_frames == 0) return rc;
-    NvtxRange range("sc_rx_frames_host");
-    rc = rx_frames_host_body(m, in, stream_stride, n_frames, results, result_stride, eq_dbg, nullptr, kw.data());
-    return rx_end(m, rc, n_frames, lfsr);
+    RxBatch b = {"sc_rx_frames_host", in, stream_stride, n_frames, results, result_stride};
+    b.eq_dbg = eq_dbg;
+    b.host = true;
+    return rx_batch(m, b);
 }
 
 // The same calls with the equalizer outputs of the data steps (include/singlecarrier_b200.h).  Nothing else changes:
@@ -1041,114 +1069,51 @@ extern "C" int sc_rx_frames_soft_dev(sc_modem *m, const int16_t *in, int64_t str
                                      sc_frame_result *results, int64_t result_stride, float *symbols, void *stream) {
     if (!symbols) return fail(SC_EINVAL, "sc_rx_frames_soft_dev: symbols is NULL");
     if (((uintptr_t) symbols & 7) != 0) return fail(SC_EINVAL, "sc_rx_frames_soft_dev: symbols not 8-byte aligned");
-    std::vector<uint64_t> kw;
-    uint16_t lfsr = 0;
-    int rc = rx_begin(m, "sc_rx_frames_soft_dev", in, stream_stride, n_frames, results, result_stride, nullptr, kw, lfsr);
-    if (rc != SC_OK || n_frames == 0) return rc;
-    NvtxRange range("sc_rx_frames_soft_dev");
-    rc = rx_frames_dev_body(m, in, stream_stride, n_frames, results, result_stride, nullptr, symbols, (cudaStream_t) stream,
-                            kw.data());
-    return rx_end(m, rc, n_frames, lfsr);
+    RxBatch b = {"sc_rx_frames_soft_dev", in, stream_stride, n_frames, results, result_stride};
+    b.sym = symbols;
+    b.stream = (cudaStream_t) stream;
+    return rx_batch(m, b);
 }
 
 extern "C" int sc_rx_frames_soft_host(sc_modem *m, const int16_t *in, int64_t stream_stride, int n_frames,
                                       sc_frame_result *results, int64_t result_stride, float *symbols) {
     if (!symbols) return fail(SC_EINVAL, "sc_rx_frames_soft_host: symbols is NULL");
-    std::vector<uint64_t> kw;
-    uint16_t lfsr = 0;
-    int rc = rx_begin(m, "sc_rx_frames_soft_host", in, stream_stride, n_frames, results, result_stride, nullptr, kw, lfsr);
-    if (rc != SC_OK || n_frames == 0) return rc;
-    NvtxRange range("sc_rx_frames_soft_host");
-    rc = rx_frames_host_body(m, in, stream_stride, n_frames, results, result_stride, nullptr, symbols, kw.data());
-    return rx_end(m, rc, n_frames, lfsr);
-}
-
-static int packets_begin(sc_modem *m, const char *who, sc_packet_result *packets, int64_t capacity, uint64_t *n_packets) {
-    if (!m || !packets || capacity < 0 || !n_packets) return fail(SC_EINVAL, "%s: bad arguments", who);
-    if (!m->packet) return fail(SC_EINVAL, "%s: the bank was not created with SC_FLAG_PACKET", who);
-    return packet_scratch(m);
+    RxBatch b = {"sc_rx_frames_soft_host", in, stream_stride, n_frames, results, result_stride};
+    b.sym = symbols;
+    b.host = true;
+    return rx_batch(m, b);
 }
 
 // The packet entry points and their soft forms.  symbols (per call) and packet_symbols are nullptr for the plain ones.
-static int rx_packets_dev(sc_modem *m, const char *who, const int16_t *in, int64_t stream_stride, int n_frames,
-                          sc_frame_result *results, int64_t result_stride, float *symbols, sc_packet_result *packets,
-                          int64_t capacity, uint64_t *n_packets, float *packet_symbols, void *stream) {
-    int rc = packets_begin(m, who, packets, capacity, n_packets);
-    if (rc != SC_OK) return rc;
-    std::vector<uint64_t> kw;
-    uint16_t lfsr = 0;
-    rc = rx_begin(m, who, in, stream_stride, n_frames, results, result_stride, nullptr, kw, lfsr);
-    if (rc != SC_OK || n_frames == 0) return rc;
-    NvtxRange range(who);
-    PacketSink sink;
-    sink.packets = packets;
-    sink.capacity = capacity;
-    sink.n_packets = (unsigned long long *) n_packets;
-    sink.symbols = reinterpret_cast<float2 *>(packet_symbols);
-    rc = rx_frames_dev_body(m, in, stream_stride, n_frames, results, result_stride, nullptr, symbols, (cudaStream_t) stream,
-                            kw.data(), &sink);
-    return rx_end(m, rc, n_frames, lfsr);
-}
-
-static int rx_packets_host(sc_modem *m, const char *who, const int16_t *in, int64_t stream_stride, int n_frames,
-                           sc_frame_result *results, int64_t result_stride, float *symbols, sc_packet_result *packets,
-                           int64_t capacity, uint64_t *n_packets, float *packet_symbols) {
-    int rc = packets_begin(m, who, packets, capacity, n_packets);
-    if (rc != SC_OK) return rc;
-    *n_packets = 0;
-    std::vector<uint64_t> kw;
-    uint16_t lfsr = 0;
-    rc = rx_begin(m, who, in, stream_stride, n_frames, results, result_stride, nullptr, kw, lfsr);
-    if (rc != SC_OK || n_frames == 0) return rc;
-    NvtxRange range(who);
-    CU(cudaSetDevice(m->device));
-    if (m->pk_stage_cap < (size_t) capacity) {
-        if (m->pk_stage) CU(cudaFree(m->pk_stage));
-        m->pk_stage = nullptr;
-        m->pk_stage_cap = 0;
-        CU(cudaMalloc(&m->pk_stage, std::max<size_t>((size_t) capacity, 1) * sizeof(sc_packet_result)));
-        m->pk_stage_cap = (size_t) capacity;
-    }
-    if (packet_symbols && m->pk_sym_stage_cap < (size_t) capacity) {
-        if (m->pk_sym_stage) CU(cudaFree(m->pk_sym_stage));
-        m->pk_sym_stage = nullptr;
-        m->pk_sym_stage_cap = 0;
-        CU(cudaMalloc(&m->pk_sym_stage, std::max<size_t>((size_t) capacity, 1) * PK_DATA * sizeof(float2)));
-        m->pk_sym_stage_cap = (size_t) capacity;
-    }
-    CU(cudaMemset(m->pk_n_host_dev, 0, sizeof(unsigned long long)));
-    PacketSink sink;
-    sink.packets = m->pk_stage;
-    sink.capacity = capacity;
-    sink.n_packets = m->pk_n_host_dev;
-    sink.symbols = packet_symbols ? m->pk_sym_stage : nullptr;
-    rc = rx_frames_host_body(m, in, stream_stride, n_frames, results, result_stride, nullptr, symbols, kw.data(), &sink);
-    if (rc == SC_OK) {
-        unsigned long long n = 0;
-        cudaError_t e = cudaMemcpy(&n, m->pk_n_host_dev, sizeof n, cudaMemcpyDeviceToHost);
-        const size_t kept = (size_t) std::min<unsigned long long>(n, (unsigned long long) capacity);
-        if (e == cudaSuccess && n > 0)
-            e = cudaMemcpy(packets, m->pk_stage, kept * sizeof(sc_packet_result), cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess && n > 0 && packet_symbols)
-            e = cudaMemcpy(packet_symbols, m->pk_sym_stage, kept * PK_DATA * sizeof(float2), cudaMemcpyDeviceToHost);
-        if (e != cudaSuccess) rc = fail(SC_ECUDA, "%s: %s", who, cudaGetErrorString(e));
-        *n_packets = n;
-    }
-    return rx_end(m, rc, n_frames, lfsr);
+static RxBatch packet_batch(const char *who, const int16_t *in, int64_t stream_stride, int n_frames,
+                            sc_frame_result *results, int64_t result_stride, float *symbols, sc_packet_result *packets,
+                            int64_t capacity, uint64_t *n_packets, float *packet_symbols) {
+    RxBatch b = {who, in, stream_stride, n_frames, results, result_stride};
+    b.sym = symbols;
+    b.packet_mode = true;
+    b.packets = packets;
+    b.capacity = capacity;
+    b.n_packets = n_packets;
+    b.packet_symbols = packet_symbols;
+    return b;
 }
 
 extern "C" int sc_rx_packets_dev(sc_modem *m, const int16_t *in, int64_t stream_stride, int n_frames,
                                  sc_frame_result *results, int64_t result_stride, sc_packet_result *packets,
                                  int64_t capacity, uint64_t *n_packets, void *stream) {
-    return rx_packets_dev(m, "sc_rx_packets_dev", in, stream_stride, n_frames, results, result_stride, nullptr, packets,
-                          capacity, n_packets, nullptr, stream);
+    RxBatch b = packet_batch("sc_rx_packets_dev", in, stream_stride, n_frames, results, result_stride, nullptr, packets,
+                             capacity, n_packets, nullptr);
+    b.stream = (cudaStream_t) stream;
+    return rx_batch(m, b);
 }
 
 extern "C" int sc_rx_packets_host(sc_modem *m, const int16_t *in, int64_t stream_stride, int n_frames,
                                   sc_frame_result *results, int64_t result_stride, sc_packet_result *packets,
                                   int64_t capacity, uint64_t *n_packets) {
-    return rx_packets_host(m, "sc_rx_packets_host", in, stream_stride, n_frames, results, result_stride, nullptr, packets,
-                           capacity, n_packets, nullptr);
+    RxBatch b = packet_batch("sc_rx_packets_host", in, stream_stride, n_frames, results, result_stride, nullptr, packets,
+                             capacity, n_packets, nullptr);
+    b.host = true;
+    return rx_batch(m, b);
 }
 
 // Packet mode with the equalizer outputs (include/singlecarrier_b200.h): the 248 of every packet record, and, when
@@ -1161,8 +1126,10 @@ extern "C" int sc_rx_packets_soft_dev(sc_modem *m, const int16_t *in, int64_t st
     if (((uintptr_t) packet_symbols & 7) != 0)
         return fail(SC_EINVAL, "sc_rx_packets_soft_dev: packet_symbols not 8-byte aligned");
     if (((uintptr_t) symbols & 7) != 0) return fail(SC_EINVAL, "sc_rx_packets_soft_dev: symbols not 8-byte aligned");
-    return rx_packets_dev(m, "sc_rx_packets_soft_dev", in, stream_stride, n_frames, results, result_stride, symbols,
-                          packets, capacity, n_packets, packet_symbols, stream);
+    RxBatch b = packet_batch("sc_rx_packets_soft_dev", in, stream_stride, n_frames, results, result_stride, symbols,
+                             packets, capacity, n_packets, packet_symbols);
+    b.stream = (cudaStream_t) stream;
+    return rx_batch(m, b);
 }
 
 extern "C" int sc_rx_packets_soft_host(sc_modem *m, const int16_t *in, int64_t stream_stride, int n_frames,
@@ -1170,8 +1137,10 @@ extern "C" int sc_rx_packets_soft_host(sc_modem *m, const int16_t *in, int64_t s
                                        sc_packet_result *packets, int64_t capacity, uint64_t *n_packets,
                                        float *packet_symbols) {
     if (!packet_symbols) return fail(SC_EINVAL, "sc_rx_packets_soft_host: packet_symbols is NULL");
-    return rx_packets_host(m, "sc_rx_packets_soft_host", in, stream_stride, n_frames, results, result_stride, symbols,
-                           packets, capacity, n_packets, packet_symbols);
+    RxBatch b = packet_batch("sc_rx_packets_soft_host", in, stream_stride, n_frames, results, result_stride, symbols,
+                             packets, capacity, n_packets, packet_symbols);
+    b.host = true;
+    return rx_batch(m, b);
 }
 
 extern "C" uint64_t sc_packet_keystream_word(int frame) {
@@ -1318,46 +1287,41 @@ extern "C" int sc_fir_batch_dev(int device, int64_t n_streams, int wide, float *
     return SC_OK;
 }
 
-// A fragments of the tensor-core proposer (sc_search_mma.cuh): one small immutable table per device
-static std::mutex g_search_mu;
-static std::map<int, void *> g_search_tables;
-static std::map<int, void *> g_search_fft_tables;     // the FFT proposer's spectrum of the preamble
-static std::map<int, void *> g_search_umma_masters;   // the fused tcgen05 proposer's A-operand master (sc_frontend_umma.cu)
+// Immutable per-device tables, shared by every call and stream, built on first use and freed by sc_release_caches():
+// the search proposers' operand tables and the FFT tables.  The map is never destroyed: freeing device memory while
+// the process exits would race the CUDA runtime's own teardown.
+enum TableKind { TAB_SEARCH_MMA, TAB_SEARCH_UMMA, TAB_SEARCH_FFT, TAB_FFT_TW, TAB_FFT_SUPER_TW, TAB_FFT_PERM };
+using TableKey = std::tuple<int, int, int, int, int>;     // (kind, device, n, inverse, real)
+static std::mutex g_tables_mu;
+static std::map<TableKey, DevBuf<char>> &g_tables = *new std::map<TableKey, DevBuf<char>>();
 
-static int search_umma_master(int device, const void **out) {
-    std::lock_guard<std::mutex> lock(g_search_mu);
-    auto it = g_search_umma_masters.find(device);
-    if (it != g_search_umma_masters.end()) {
-        *out = it->second;
-        return SC_OK;
+// The table `key` on its device, `count` elements of T written by make() on the host when it is built.
+template <typename T, typename Make>
+static int device_table(const TableKey &key, size_t count, Make make, const void **out) {
+    std::lock_guard<std::mutex> lock(g_tables_mu);
+    auto it = g_tables.find(key);
+    if (it == g_tables.end()) {
+        std::vector<T> h(count);
+        make(h.data());
+        DevBuf<char> d;                     // released, with its device current, if it is not completed
+        CU(cudaSetDevice(std::get<1>(key)));
+        CU(d.reserve(count * sizeof(T)));
+        CU(cudaMemcpy(d, h.data(), count * sizeof(T), cudaMemcpyHostToDevice));
+        it = g_tables.emplace(key, std::move(d)).first;
     }
-    std::vector<uint16_t> h((size_t) SU_A_WORDS4 * 8);
-    search_umma_make_master(h.data());
-    void *d = nullptr;
-    CU(cudaSetDevice(device));
-    CU(cudaMalloc(&d, h.size() * sizeof(uint16_t)));
-    CU(cudaMemcpy(d, h.data(), h.size() * sizeof(uint16_t), cudaMemcpyHostToDevice));
-    g_search_umma_masters[device] = d;
-    *out = d;
+    *out = it->second.p;
     return SC_OK;
 }
 
+// A fragments of the tensor-core proposer (sc_search_mma.cuh) and the fused tcgen05 proposer's A-operand master
+// (sc_frontend_umma.cu)
 static int search_table(int device, const void **out) {
-    std::lock_guard<std::mutex> lock(g_search_mu);
-    auto it = g_search_tables.find(device);
-    if (it != g_search_tables.end()) {
-        *out = it->second;
-        return SC_OK;
-    }
-    std::vector<uint32_t> h((size_t) 9 * 32 * 4);
-    search_mma_make_table(h.data());
-    void *d = nullptr;
-    CU(cudaSetDevice(device));
-    CU(cudaMalloc(&d, h.size() * sizeof(uint32_t)));
-    CU(cudaMemcpy(d, h.data(), h.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    g_search_tables[device] = d;
-    *out = d;
-    return SC_OK;
+    return device_table<uint32_t>(TableKey(TAB_SEARCH_MMA, device, 0, 0, 0), (size_t) 9 * 32 * 4, search_mma_make_table, out);
+}
+
+static int search_umma_master(int device, const void **out) {
+    return device_table<uint16_t>(TableKey(TAB_SEARCH_UMMA, device, 0, 0, 0), (size_t) SU_A_WORDS4 * 8,
+                                  search_umma_make_master, out);
 }
 
 static int search_args(int64_t n_streams, const float *symbols, int64_t symbol_stride, int32_t *max_index, float *max_value) {
@@ -1497,47 +1461,27 @@ void fft_make_super_twiddles(int ncfft, int inverse, float2 *tw) {
 }
 }  // namespace sc
 
-// Immutable per-(device, n, direction) tables, shared by every call and stream: twiddles, the real-FFT
-// super twiddles and the digit-reversal permutation of kf_work()'s leaves.  Working storage is NOT cached:
-// transforms too long for shared memory get stream-ordered scratch per call (two calls on two streams must
-// not share it).  sc_release_caches() frees the tables.
+// Per-(device, n, direction) FFT tables: twiddles, the real-FFT super twiddles and the digit-reversal permutation of
+// kf_work()'s leaves.  Working storage is NOT cached: transforms too long for shared memory get stream-ordered scratch
+// per call (two calls on two streams must not share it).
 struct FftDeviceTables {
-    float2 *tw = nullptr, *super_tw = nullptr;
-    int *perm = nullptr;
+    const void *tw = nullptr, *super_tw = nullptr, *perm = nullptr;
 };
-static std::mutex g_fft_mu;
-static std::map<std::tuple<int, int, int, int>, FftDeviceTables> g_fft_tables;   // (device, n, inverse, real)
 
-static int fft_tables(int device, int n, int inverse, bool real, FftDeviceTables *out) {
-    std::lock_guard<std::mutex> lock(g_fft_mu);
-    auto key = std::make_tuple(device, n, inverse ? 1 : 0, real ? 1 : 0);
-    auto it = g_fft_tables.find(key);
-    if (it != g_fft_tables.end()) {
-        *out = it->second;
-        return SC_OK;
-    }
-    FftDeviceTables t;
-    std::vector<float2> h(n);
-    fft_make_twiddles(n, inverse, h.data());
-    CU(cudaMalloc(&t.tw, (size_t) n * sizeof(float2)));
-    CU(cudaMemcpy(t.tw, h.data(), (size_t) n * sizeof(float2), cudaMemcpyHostToDevice));
-    if (real) {
-        std::vector<float2> hs(std::max(n / 2, 1));
-        fft_make_super_twiddles(n, inverse, hs.data());
-        CU(cudaMalloc(&t.super_tw, hs.size() * sizeof(float2)));
-        CU(cudaMemcpy(t.super_tw, hs.data(), hs.size() * sizeof(float2), cudaMemcpyHostToDevice));
-    }
-    {
-        FftPlan plan;
-        fft_make_plan(n, inverse, &plan);
-        std::vector<int> perm(n);
-        fft_make_permutation(plan, perm.data());
-        CU(cudaMalloc(&t.perm, (size_t) n * sizeof(int)));
-        CU(cudaMemcpy(t.perm, perm.data(), (size_t) n * sizeof(int), cudaMemcpyHostToDevice));
-    }
-    g_fft_tables[key] = t;
-    *out = t;
-    return SC_OK;
+static int fft_tables(int device, int n, int inverse, bool real, FftDeviceTables *t) {
+    inverse = inverse ? 1 : 0;
+    auto key = [&](int kind) { return TableKey(kind, device, n, inverse, real ? 1 : 0); };
+    int rc = device_table<float2>(key(TAB_FFT_TW), n, [&](float2 *h) { fft_make_twiddles(n, inverse, h); }, &t->tw);
+    if (rc == SC_OK && real)
+        rc = device_table<float2>(key(TAB_FFT_SUPER_TW), std::max(n / 2, 1),
+                                  [&](float2 *h) { fft_make_super_twiddles(n, inverse, h); }, &t->super_tw);
+    if (rc == SC_OK)
+        rc = device_table<int>(key(TAB_FFT_PERM), n, [&](int *h) {
+            FftPlan plan;
+            fft_make_plan(n, inverse, &plan);
+            fft_make_permutation(plan, h);
+        }, &t->perm);
+    return rc;
 }
 
 static int fft_run(int device, int64_t n_batches, int n_core, int inverse, int mode, const void *in, void *out,
@@ -1552,38 +1496,18 @@ static int fft_run(int device, int64_t n_batches, int n_core, int inverse, int m
     cudaStream_t st = (cudaStream_t) stream;
     AsyncBuf<float2> scratch(st);
     if (fft_needs_scratch(n_core)) CU(scratch.alloc((size_t) FFT_SCRATCH_CTAS * 2 * n_core));
-    CU(launch_fft(plan, t.tw, t.super_tw, t.perm, mode, in, out, scratch.p, n_batches, st));
+    CU(launch_fft(plan, (const float2 *) t.tw, (const float2 *) t.super_tw, (const int *) t.perm, mode, in, out, scratch.p,
+                  n_batches, st));
     return SC_OK;
 }
 
 extern "C" int sc_release_caches(void) {
-    std::lock_guard<std::mutex> lock(g_fft_mu);
+    std::lock_guard<std::mutex> lock(g_tables_mu);
     int dev0 = 0;
     cudaGetDevice(&dev0);
-    for (auto &kv : g_fft_tables) {
-        cudaSetDevice(std::get<0>(kv.first));
-        cudaFree(kv.second.tw);
-        cudaFree(kv.second.super_tw);
-        cudaFree(kv.second.perm);
-    }
-    g_fft_tables.clear();
-    {
-        std::lock_guard<std::mutex> lock2(g_search_mu);
-        for (auto &kv : g_search_tables) {
-            cudaSetDevice(kv.first);
-            cudaFree(kv.second);
-        }
-        g_search_tables.clear();
-        for (auto &kv : g_search_umma_masters) {
-            cudaSetDevice(kv.first);
-            cudaFree(kv.second);
-        }
-        g_search_umma_masters.clear();
-        for (auto &kv : g_search_fft_tables) {
-            cudaSetDevice(kv.first);
-            cudaFree(kv.second);
-        }
-        g_search_fft_tables.clear();
+    while (!g_tables.empty()) {
+        cudaSetDevice(std::get<1>(g_tables.begin()->first));
+        g_tables.erase(g_tables.begin());
     }
     cudaSetDevice(dev0);
     cudaGetLastError();
@@ -1618,20 +1542,11 @@ extern "C" int sc_preamble_search_fft_batch_dev(int device, int64_t n_streams, c
     if (n_streams == 0) return SC_OK;
     FftDeviceTables t;
     if ((rc = fft_tables(device, 256, 0, false, &t)) != SC_OK) return rc;
-    void *ptab = nullptr;
-    {
-        std::lock_guard<std::mutex> lock(g_search_mu);
-        auto it = g_search_fft_tables.find(device);
-        if (it != g_search_fft_tables.end()) ptab = it->second;
-        else {
-            std::vector<float> h((size_t) 8 * 32 * 2);
-            search_fft_make_table(h.data());
-            CU(cudaMalloc(&ptab, h.size() * sizeof(float)));
-            CU(cudaMemcpy(ptab, h.data(), h.size() * sizeof(float), cudaMemcpyHostToDevice));
-            g_search_fft_tables[device] = ptab;
-        }
-    }
-    CU(launch_search_fft_batch(n_streams, (const float2 *) symbols, symbol_stride, t.tw, ptab, max_index, max_value,
+    const void *ptab = nullptr;
+    if ((rc = device_table<float>(TableKey(TAB_SEARCH_FFT, device, 0, 0, 0), (size_t) 8 * 32 * 2, search_fft_make_table,
+                                  &ptab)) != SC_OK)
+        return rc;
+    CU(launch_search_fft_batch(n_streams, (const float2 *) symbols, symbol_stride, (const float2 *) t.tw, ptab, max_index, max_value,
                                (cudaStream_t) stream));
     return SC_OK;
 }
@@ -1711,26 +1626,13 @@ StateLayout state_layout(const sc_modem *m) {
 
 extern "C" int64_t sc_state_size(const sc_modem *m) { return m ? (int64_t) state_layout(m).total : 0; }
 
-static int state_quiesce(sc_modem *m) {
-    CU(cudaSetDevice(m->device));
-    for (int i = 0; i < N_PIPE; i++) CU(cudaStreamSynchronize(m->pipe[i]));
-    CU(cudaStreamSynchronize(m->tab_stream));
-    if (m->ov_ready)                    // joined into the pipes by every successful batch; a failed one may not have
-        for (int i = 0; i < N_PIPE; i++) {
-            CU(cudaStreamSynchronize(m->ov_stream[i]));
-            CU(cudaStreamSynchronize(m->ov_data[i][0]));
-            CU(cudaStreamSynchronize(m->ov_data[i][1]));
-        }
-    return SC_OK;
-}
-
 extern "C" int sc_state_export(sc_modem *m, void *buf, int64_t buf_bytes) {
     if (!m || !buf) return fail(SC_EINVAL, "sc_state_export: bad arguments");
     if (m->poisoned) return fail(SC_ESTATE, "sc_state_export: the bank is in a failed-batch state");
     if (m->packet) return fail(SC_EINVAL, "sc_state_export: not available for SC_FLAG_PACKET banks");
     const StateLayout L = state_layout(m);
     if (buf_bytes < (int64_t) L.total) return fail(SC_EINVAL, "sc_state_export: buffer smaller than sc_state_size()");
-    int rc = state_quiesce(m);
+    int rc = drain(m);
     if (rc != SC_OK) return rc;
     CU(cudaDeviceSynchronize());                           // the caller's stream may still be writing state
     char *b = (char *) buf;
@@ -1767,12 +1669,9 @@ extern "C" int sc_state_import(sc_modem *m, const void *buf, int64_t buf_bytes) 
     if (h.magic != STATE_MAGIC || h.version != STATE_VERSION) return fail(SC_EINVAL, "sc_state_import: not a state image");
     if (h.n != m->n || h.n_pad != m->n_pad || h.flags != m->flags || h.foffset != m->foffset)
         return fail(SC_EINVAL, "sc_state_import: the image was taken from a bank with other parameters");
-    int rc = state_quiesce(m);
+    int rc = drain(m);
     if (rc != SC_OK) return rc;
-    if (m->mix_cap < 1) {
-        CU(cudaMalloc(&m->mix_table, (size_t) 2 * FRAME * sizeof(float2)));
-        m->mix_cap = 1;
-    }
+    CU(m->mix_table.reserve(FRAME));
     CU(cudaMemcpy(m->rx_phase, &h.rx_phase, sizeof(float2), cudaMemcpyHostToDevice));
     CU(cudaMemcpy(m->timing[h.call & 1], b + L.off_timing, (size_t) m->n_pad * sizeof(int), cudaMemcpyHostToDevice));
     CU(cudaMemcpy(m->max_index, b + L.off_maxi, (size_t) m->n_pad * sizeof(int), cudaMemcpyHostToDevice));
@@ -1820,7 +1719,7 @@ extern "C" int sc_set_option(sc_modem *m, int option, int64_t value) {
     }
 }
 
-static int prof_sum(std::vector<cudaEvent_t> &v, double *ms, double *count) {
+static int prof_sum(std::vector<Event> &v, double *ms, double *count) {
     *ms = 0.0;
     *count = 0.0;
     for (size_t i = 0; i + 1 < v.size(); i += 2) {
@@ -1829,7 +1728,6 @@ static int prof_sum(std::vector<cudaEvent_t> &v, double *ms, double *count) {
         *ms += t;
         *count += 1.0;
     }
-    for (cudaEvent_t e : v) cudaEventDestroy(e);
     v.clear();
     return SC_OK;
 }
