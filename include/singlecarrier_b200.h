@@ -44,6 +44,9 @@ extern "C" {
 #define SC_FLAG_DEBUG_EQ  0x2u      /* keep eq_coeff[5] of every call (parity tests)         */
 #define SC_FLAG_PACKET    0x4u      /* packet mode (extension, see sc_rx_packets_*): TX scrambles,
                                        RX can decode all 8 x 31 data symbols of a packet     */
+#define SC_FLAG_PACKET_DD 0x8u      /* with SC_FLAG_PACKET only (else sc_create: SC_EINVAL):
+                                       packets decoded by a decision-directed equalizer and
+                                       carrier loop instead of the reference's Kalman one    */
 
 typedef struct sc_modem sc_modem;
 
@@ -194,6 +197,12 @@ int sc_rx_frames_soft_host(sc_modem *m, const int16_t *in, int64_t stream_stride
  * matched-filter output at 1880 (n-2) + 5 (max_index + j) + T.  Specification: oracle/sc_oracle_ext.c.
  * The transmit side (sc_tx_*_dev of a SC_FLAG_PACKET bank) seeds the TX register after every preamble and
  * scrambles every data dibit (qpsk.c:386,397 un-commented); `bits` / `bits_out` are the payload.
+ *
+ * The reference's equalizer diverges (its bits are near chance).  SC_FLAG_PACKET_DD decodes the same records, on the
+ * same symbol grid, with a 5-tap normalised LMS filter and a second-order carrier loop instead (DESIGN.md section 8):
+ * trained on the 128 preamble symbols, then decision-directed over the 248 data symbols.  Fields then: bits as below;
+ * matches is the call's; cost is the float32 sequential sum of |d - y|^2 over the 248 data steps (d the decision, y
+ * the derotated equalizer output, the value the soft forms return).  Every other result is unchanged.
  */
 typedef struct {
     uint64_t bits[8];       /* frame f: bit 2i = Q, bit 2i+1 = I of data symbol i, descrambled */
@@ -201,7 +210,7 @@ typedef struct {
     uint32_t call_index;    /* the valid call this packet belongs to */
     int16_t  max_index;
     int16_t  matches;       /* of the packet's own training pass (equals the call's) */
-    float    cost;          /* sum of the 248 data_eq() returns */
+    float    cost;          /* sum of the 248 data_eq() returns (SC_FLAG_PACKET_DD: of |d - y|^2) */
     uint32_t reserved0, reserved1;
     uint64_t reserved2;
 } sc_packet_result;         /* 96 bytes */
@@ -232,7 +241,8 @@ int sc_rx_packets_host(sc_modem *m, const int16_t *in, int64_t stream_stride, in
  * Bit mapping: in data frame f (0..7) of a packet, with sym = the record's block, bit 2i of the raw decision is
  * (Im(sym[31 f + i]) < 0) and bit 2i+1 is (Re(sym[31 f + i]) < 0), and packets[k].bits[f] = raw decision XOR
  * sc_packet_keystream_word(f).  packets[k].cost is the float32 sequential sum over the 248 steps of
- * (c - Re) * 0.1f, c = (Re < 0 ? -1 : 1), each operation rounded.
+ * (c - Re) * 0.1f, c = (Re < 0 ? -1 : 1), each operation rounded.  On a SC_FLAG_PACKET_DD bank sym is the derotated
+ * equalizer output y, the bit mapping is the same and cost is the sum of |d - y|^2 (d = the sliced +-1 +-1j).
  * sc_transfer_bytes counts what _host moves for the ordinary calls (results and per-call symbols) as for
  * sc_rx_frames_soft_host; like sc_rx_packets_host it does not count packet records or packet symbols.
  */

@@ -147,6 +147,7 @@ struct sc_modem {
     // packet mode (SC_FLAG_PACKET, extension): the frame before the saved one, its phasor table, the rx_timing
     // snapshots and per-pipe scratch for the packet pass
     bool packet = false;
+    bool packet_dd = false;                 // SC_FLAG_PACKET_DD: packets decoded by the decision-directed equalizer
     DevBuf<int16_t> pk_hist2;               // frame call-2, [n][1880]
     DevBuf<float2> pk_mix_hist2;            // phasor table of frame call-2
     DevBuf<int> pk_t_before[N_PIPE], pk_t_at[N_PIPE];         // [slab] rx_timing at entry of calls call0-1 / call0
@@ -265,6 +266,8 @@ static int search_umma_master(int device, const void **out);
 extern "C" int sc_create(sc_modem **out, int device, int64_t n_streams, uint32_t flags, float foffset_hz) {
     if (!out || n_streams <= 0 || n_streams > (int64_t) 1 << 30) return fail(SC_EINVAL, "sc_create: bad arguments");
     *out = nullptr;
+    if ((flags & SC_FLAG_PACKET_DD) && !(flags & SC_FLAG_PACKET))
+        return fail(SC_EINVAL, "sc_create: SC_FLAG_PACKET_DD needs SC_FLAG_PACKET");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
         cudaGetLastError();
@@ -280,6 +283,7 @@ extern "C" int sc_create(sc_modem **out, int device, int64_t n_streams, uint32_t
     m->wide = (flags & SC_FLAG_WIDE) != 0;
     m->debug_eq = (flags & SC_FLAG_DEBUG_EQ) != 0;
     m->packet = (flags & SC_FLAG_PACKET) != 0;
+    m->packet_dd = (flags & SC_FLAG_PACKET_DD) != 0;
     {
         uint16_t r = 0x4A80;                                             // scramble_init per packet
         for (int f = 0; f < 8; f++) m->pk_key.k[f] = keystream_next_word(r);
@@ -764,7 +768,8 @@ static int run_slab(sc_modem *m, const Slab &s) {
             CU(cudaEventRecord(m->pk_ev_go[pipe], st));
             CU(cudaStreamWaitEvent(m->pk_stream[pipe], m->pk_ev_go[pipe], 0));
             CU(launch_packet_pass(psrc, ns, pk_done, j + 1, PK_CAP, m->pk_list[pipe], m->pk_count[pipe], m->pk_sym[pipe],
-                                  m->pk_key, pk->packets, pk->capacity, pk->n_packets, pk->symbols, m->pk_stream[pipe]));
+                                  m->pk_key, pk->packets, pk->capacity, pk->n_packets, pk->symbols, m->packet_dd,
+                                  m->pk_stream[pipe]));
             pk_done = j + 1;
         }
     }

@@ -126,9 +126,10 @@ struct PacketSrc {              // one block of calls [call0, call0 + nf) of a s
 };
 cudaError_t launch_packet_pass(const PacketSrc &src, int n_streams, int j_lo, int j_hi, int cap, int2 *list, int *count,
                                float2 *sym, const PacketKey &key, sc_packet_result *packets, long packet_capacity,
-                               unsigned long long *n_packets, float2 *packet_sym, cudaStream_t st);
+                               unsigned long long *n_packets, float2 *packet_sym, bool dd, cudaStream_t st);
 // packet_sym: nullptr, or the equalizer outputs of the 248 data steps of every packet, PK_DATA float2 per record slot
-// (record packets[k] <-> packet_sym[k * PK_DATA ..]); slots beyond packet_capacity are not written
+// (record packets[k] <-> packet_sym[k * PK_DATA ..]); slots beyond packet_capacity are not written.
+// dd: decode with the decision-directed equalizer (SC_FLAG_PACKET_DD) instead of the reference's
 
 // sc_tx_kernels.cu
 struct TxArgs {

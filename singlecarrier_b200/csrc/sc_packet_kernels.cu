@@ -14,6 +14,7 @@
 //   packet_list_kernel    (one thread per stream x call)  valid calls of the block -> compact list
 //   packet_fir_kernel     (one warp per listed packet)    int16 -> mix -> 49-tap RRC at the 380 symbol instants
 //   packet_track_kernel   (one thread per listed packet)  the sequential loop, 128 + 248 steps
+//   packet_track_dd_kernel                                 the same with the decision-directed equalizer (SC_FLAG_PACKET_DD)
 #include "sc_common.cuh"
 #include "sc_tables.cuh"
 #include "sc_tracker.cuh"
@@ -173,9 +174,123 @@ packet_track_kernel(PacketSrc src, const int2 *__restrict__ list, const int *__r
     if ((long) pos < packet_capacity) packets[pos] = r;
 }
 
+// ---- SC_FLAG_PACKET_DD: the decision-directed equalizer over one packet ---------------------------------------------
+// The same grid, list and record-slot protocol as packet_track_kernel; the loop is a 5-tap normalised LMS filter and a
+// second-order carrier loop (DESIGN.md section 8; specification tests/packet_dd_ref.c, scd_dd_packet), written out
+// operation for operation.  matches is the call's; cost is the sum of |d - y|^2 over the 248 data steps.
+constexpr float DD_MU = 0.03f, DD_ALPHA = 0.05f, DD_BETA = 0.002f, DD_EPS = 1e-6f, DD_TRAIN_AMP = 0.5f,
+                DD_PEPS = 1e-6f;
+
+struct DdLoop {
+    c32 w[EQ];
+    c32 p;
+    float nu;
+
+    __device__ __forceinline__ void reset() {
+#pragma unroll
+        for (int k = 0; k < EQ; k++) w[k] = mk(0.0f, 0.0f);
+        p = mk(1.0f, 0.0f);
+        nu = 0.0f;
+    }
+    // the derotated output y of the window x
+    __device__ __forceinline__ c32 output(const c32 (&x)[EQ]) const {
+        c32 z = mk(0.0f, 0.0f);
+#pragma unroll
+        for (int k = 0; k < EQ; k++) z = cadd(z, cmulc(x[k], w[k]));
+        return cmulc(z, p);
+    }
+    // one step towards the decision d; returns e = d - y
+    __device__ __forceinline__ c32 step(const c32 (&x)[EQ], c32 y, c32 d) {
+        const c32 e = mk(__fsub_rn(d.r, y.r), __fsub_rn(d.i, y.i));
+        const c32 q = cmulc(y, d);
+        const float qm = __fsqrt_rn(__fadd_rn(__fmul_rn(q.r, q.r), __fmul_rn(q.i, q.i)));
+        const float pe = __fdiv_rn(q.i, __fadd_rn(qm, DD_PEPS));
+        float n = DD_EPS;
+#pragma unroll
+        for (int k = 0; k < EQ; k++) n = __fadd_rn(n, __fadd_rn(__fmul_rn(x[k].r, x[k].r), __fmul_rn(x[k].i, x[k].i)));
+        const float g = __fdiv_rn(DD_MU, n);
+        const c32 ep = cmul(e, p);
+        const c32 u = mk(__fmul_rn(ep.r, g), -__fmul_rn(ep.i, g));
+#pragma unroll
+        for (int k = 0; k < EQ; k++) w[k] = cadd(w[k], cmul(x[k], u));
+        nu = __fadd_rn(nu, __fmul_rn(DD_BETA, pe));
+        const float phi = __fadd_rn(__fmul_rn(DD_ALPHA, pe), nu);
+        p = mk(__fsub_rn(p.r, __fmul_rn(p.i, phi)), __fadd_rn(p.i, __fmul_rn(p.r, phi)));
+        const float m = __fsqrt_rn(__fadd_rn(__fmul_rn(p.r, p.r), __fmul_rn(p.i, p.i)));
+        p = mk(__fdiv_rn(p.r, m), __fdiv_rn(p.i, m));
+        return e;
+    }
+};
+
+template <bool SOFT>
+__global__ void __launch_bounds__(128)
+packet_track_dd_kernel(PacketSrc src, const int2 *__restrict__ list, const int *__restrict__ count, int cap,
+                       const float2 *__restrict__ sym, PacketKey key, sc_packet_result *__restrict__ packets,
+                       long packet_capacity, unsigned long long *__restrict__ n_packets, float2 *__restrict__ psym) {
+    const int n_list = min(*count, cap);
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n_list) return;
+    const int2 ent = list[e];
+    const float2 *X = sym + ((long) (e >> 5) * PK_SYMS) * 32 + (e & 31);
+
+    DdLoop dd;
+    dd.reset();
+    c32 x[EQ];
+#pragma unroll
+    for (int i = 0; i < EQ - 1; i++) x[i] = from2(X[i * 32]);
+    c32 nxt = from2(X[(EQ - 1) * 32]);
+#pragma unroll 1
+    for (int i = 0; i < PRE; i++) {
+        x[EQ - 1] = nxt;
+        nxt = from2(X[(i + EQ) * 32]);
+        const float a = ((c_pk_pre_neg[i >> 5] >> (i & 31)) & 1u) ? -DD_TRAIN_AMP : DD_TRAIN_AMP;
+        dd.step(x, dd.output(x), mk(a, a));
+#pragma unroll
+        for (int k = 0; k < EQ - 1; k++) x[k] = x[k + 1];
+    }
+    sc_packet_result r;
+    float cost = 0.0f;
+    unsigned long long word = 0ull;
+    unsigned long long pos = 0ull;
+    float2 *out = nullptr;
+    if (SOFT) {
+        pos = atomicAdd(n_packets, 1ull);
+        if ((long) pos < packet_capacity) out = psym + (long) pos * PK_DATA;
+    }
+#pragma unroll 1
+    for (int i = 0; i < PK_DATA; i++) {
+        x[EQ - 1] = nxt;
+        nxt = from2(X[min(PRE + i + EQ, PK_SYMS - 1) * 32]);
+        const c32 y = dd.output(x);
+        const int bI = y.r < 0.0f, bQ = y.i < 0.0f;
+        const c32 er = dd.step(x, y, mk(bI ? -1.0f : 1.0f, bQ ? -1.0f : 1.0f));
+        cost = __fadd_rn(cost, __fadd_rn(__fmul_rn(er.r, er.r), __fmul_rn(er.i, er.i)));
+        if (SOFT && out) out[i] = to2(y);
+        const int f = i / NDATA, k = i - f * NDATA;
+        word |= ((unsigned long long) (unsigned) (bQ | (bI << 1))) << (2 * k);
+        if (k == NDATA - 1) {
+            r.bits[f] = word ^ key.k[f];
+            word = 0ull;
+        }
+#pragma unroll
+        for (int kk = 0; kk < EQ - 1; kk++) x[kk] = x[kk + 1];
+    }
+    const sc_frame_result *rec = src.results + (long) ent.x * src.result_stride + ent.y;
+    r.stream = src.stream0 + ent.x;
+    r.call_index = src.call0 + (uint32_t) ent.y;
+    r.max_index = rec->max_index;
+    r.matches = rec->matches;
+    r.cost = cost;
+    r.reserved0 = 0;
+    r.reserved1 = 0;
+    r.reserved2 = 0;
+    if (!SOFT) pos = atomicAdd(n_packets, 1ull);
+    if ((long) pos < packet_capacity) packets[pos] = r;
+}
+
 cudaError_t launch_packet_pass(const PacketSrc &src, int n_streams, int j_lo, int j_hi, int cap, int2 *list, int *count,
                                float2 *sym, const PacketKey &key, sc_packet_result *packets, long packet_capacity,
-                               unsigned long long *n_packets, float2 *packet_sym, cudaStream_t st) {
+                               unsigned long long *n_packets, float2 *packet_sym, bool dd, cudaStream_t st) {
     cudaError_t e = cudaMemsetAsync(count, 0, sizeof(int), st);
     if (e != cudaSuccess) return e;
     const long total = (long) n_streams * (j_hi - j_lo);
@@ -188,7 +303,13 @@ cudaError_t launch_packet_pass(const PacketSrc &src, int n_streams, int j_lo, in
     const int g2 = (int) std::min<long>((worst + PK_FIR_WARPS - 1) / PK_FIR_WARPS, 148L * 16);
     packet_fir_kernel<<<g2, PK_FIR_WARPS * 32, 0, st>>>(src, list, count, cap, sym);
     const int g3 = (int) ((worst + 127) / 128);
-    if (packet_sym)
+    if (dd && packet_sym)
+        packet_track_dd_kernel<true><<<g3, 128, 0, st>>>(src, list, count, cap, sym, key, packets, packet_capacity,
+                                                         n_packets, packet_sym);
+    else if (dd)
+        packet_track_dd_kernel<false><<<g3, 128, 0, st>>>(src, list, count, cap, sym, key, packets, packet_capacity,
+                                                          n_packets, nullptr);
+    else if (packet_sym)
         packet_track_kernel<true><<<g3, 128, 0, st>>>(src, list, count, cap, sym, key, packets, packet_capacity, n_packets,
                                                       packet_sym);
     else

@@ -12,7 +12,7 @@ from typing import Optional
 
 import numpy as np
 
-from ._lib import SC_FLAG_DEBUG_EQ, SC_FLAG_PACKET, SC_FLAG_WIDE, Channel, check, lib
+from ._lib import SC_FLAG_DEBUG_EQ, SC_FLAG_PACKET, SC_FLAG_PACKET_DD, SC_FLAG_WIDE, Channel, check, lib
 
 FRAME_SIZE = 1880
 SYMBOLS_PER_FRAME = 376
@@ -194,10 +194,14 @@ class ModemBank:
     """A bank of ``n_streams`` synchronized modems on one GPU (sc_modem handle)."""
 
     def __init__(self, n_streams: int, device: int = 0, wide: bool = False, foffset_hz: float = 0.0,
-                 debug_eq: bool = False, packet: bool = False):
+                 debug_eq: bool = False, packet: bool = False, dd: bool = False):
+        """packet: packet mode (SC_FLAG_PACKET); dd: its packets decoded by the decision-directed equalizer
+        (SC_FLAG_PACKET_DD, needs packet=True)."""
         self._h = C.c_void_p()
-        flags = (SC_FLAG_WIDE if wide else 0) | (SC_FLAG_DEBUG_EQ if debug_eq else 0) | (SC_FLAG_PACKET if packet else 0)
+        flags = (SC_FLAG_WIDE if wide else 0) | (SC_FLAG_DEBUG_EQ if debug_eq else 0) | (SC_FLAG_PACKET if packet else 0) \
+            | (SC_FLAG_PACKET_DD if dd else 0)
         self.packet = packet
+        self.dd = dd
         check(lib.sc_create(C.byref(self._h), device, n_streams, flags, foffset_hz))
         self.n_streams = n_streams
         self.device = device

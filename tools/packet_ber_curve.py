@@ -12,7 +12,8 @@ Timing, CUDA events after warm-up, medians over the repetitions:
   counter_hbm  one launch per repetition after a 512 MB buffer has been overwritten (its inputs come from HBM)
 The counter is timed with the 13 groups (each block sums in shared memory), with the same 13 groups among 129
 (above 128 groups the atomics go to global memory directly) and with one group.
-usage: python tools/packet_ber_curve.py [--out FILE] [--reps R] [--warmup W] [--launches L] [--streams N]"""
+--dd decodes the packets with the decision-directed equalizer (SC_FLAG_PACKET_DD) instead of the reference's.
+usage: python tools/packet_ber_curve.py [--out FILE] [--reps R] [--warmup W] [--launches L] [--streams N] [--dd]"""
 import argparse
 import json
 import os
@@ -74,11 +75,12 @@ def main():
     ap.add_argument("--launches", type=int, default=200)
     ap.add_argument("--streams", type=int, default=65536)
     ap.add_argument("--seed", type=int, default=0xBE4C)
+    ap.add_argument("--dd", action="store_true", help="decode with the decision-directed equalizer (SC_FLAG_PACKET_DD)")
     a = ap.parse_args()
     assert torch.cuda.is_available(), "packet_ber_curve needs a CUDA device"
-    out = {"gpu": gpu_info(), "reps": a.reps, "warmup": a.warmup, "launches": a.launches}
+    out = {"gpu": gpu_info(), "reps": a.reps, "warmup": a.warmup, "launches": a.launches, "dd": a.dd}
     ns, dev = a.streams, torch.device("cuda", 0)
-    bank = sc.ModemBank(ns, packet=True)
+    bank = sc.ModemBank(ns, packet=True, dd=a.dd)
     wl = harness.synthesize(bank, NF * FRAME, seed=a.seed, config=3)
     cap = ns * 8
     res = torch.empty((ns, NF * 32), dtype=torch.uint8, device=dev)
