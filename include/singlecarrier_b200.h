@@ -47,6 +47,9 @@ extern "C" {
 #define SC_FLAG_PACKET_DD 0x8u      /* with SC_FLAG_PACKET only (else sc_create: SC_EINVAL):
                                        packets decoded by a decision-directed equalizer and
                                        carrier loop instead of the reference's Kalman one    */
+#define SC_FLAG_PACKET_ACQ 0x10u    /* with SC_FLAG_PACKET | SC_FLAG_PACKET_DD only (else
+                                       sc_create: SC_EINVAL): packets found by acquisition on
+                                       the samples, not by the reference's per-call detection */
 
 typedef struct sc_modem sc_modem;
 
@@ -203,6 +206,14 @@ int sc_rx_frames_soft_host(sc_modem *m, const int16_t *in, int64_t stream_stride
  * trained on the 128 preamble symbols, then decision-directed over the 248 data symbols.  Fields then: bits as below;
  * matches is the call's; cost is the float32 sequential sum of |d - y|^2 over the 248 data steps (d the decision, y
  * the derotated equalizer output, the value the soft forms return).  Every other result is unchanged.
+ *
+ * SC_FLAG_PACKET_ACQ (with SC_FLAG_PACKET | SC_FLAG_PACKET_DD) replaces the per-call detection as the source of records
+ * by acquisition on the samples (DESIGN.md section 8b): a differential preamble metric rho on the matched-filter output
+ * at every symbol position, which a carrier offset does not change, at most one packet per 1880-sample frame.  The
+ * batch that contains call n emits the packets whose grid starts in frame n-2.  The DD loop starts from the offset the
+ * metric measures.  Fields then: grid_sample (authoritative), call_index = 2 + floor(grid_sample / 1880), max_index =
+ * (grid_sample mod 1880) / 5, matches = training steps whose output agrees with the preamble, acq_metric, acq_freq_hz.
+ * Per-call results, per-call soft output and the bank state are those of a SC_FLAG_PACKET_DD bank.
  */
 typedef struct {
     uint64_t bits[8];       /* frame f: bit 2i = Q, bit 2i+1 = I of data symbol i, descrambled */
@@ -211,8 +222,10 @@ typedef struct {
     int16_t  max_index;
     int16_t  matches;       /* of the packet's own training pass (equals the call's) */
     float    cost;          /* sum of the 248 data_eq() returns (SC_FLAG_PACKET_DD: of |d - y|^2) */
-    uint32_t reserved0, reserved1;
-    uint64_t reserved2;
+    float    acq_metric;    /* SC_FLAG_PACKET_ACQ: rho on the record's grid, else 0 */
+    float    acq_freq_hz;   /* SC_FLAG_PACKET_ACQ: carrier offset estimate nu0 * 1600 / (2 pi), else 0 */
+    int64_t  grid_sample;   /* SC_FLAG_PACKET_ACQ: g, the stream's matched-filter sample of the grid's first symbol,
+                               counted from the cold start, else 0 */
 } sc_packet_result;         /* 96 bytes */
 
 /* packets: capacity records, appended in no particular order; *n_packets receives the number of packets found
@@ -413,7 +426,8 @@ int sc_ber_stats_dev(int device, const sc_frame_result *results, int64_t n_strea
  *   results, n_streams, result_stride, n_frames, tx_bits, n_packets, lead_in, gap_samples, group, n_groups: as for
  *             sc_ber_stats_dev (results: calls 0..n_frames-1 of a cold-started bank).
  * Alignment, the rule of sc_ber_stats_dev applied to the record: with n = call_index and
- * pos = (n-2)*1880 + 5*max_index + results[stream][n-2].rx_timing - 48 - lead_in[stream], the record is aligned to
+ * pos = (n-2)*1880 + 5*max_index + results[stream][n-2].rx_timing - 48 - lead_in[stream] -- or, when the record's
+ * grid_sample is not 0 (SC_FLAG_PACKET_ACQ banks), pos = grid_sample - 48 - lead_in[stream] -- the record is aligned to
  * transmitted packet j when |pos - j*(1880 + gap_samples)| <= 10 and 0 <= j < n_packets.  TX scrambles and RX
  * descrambles in packet mode, so the error pattern of data frame f (0..7) is (bits[f] ^ txword(f)) & (2^62 - 1), where
  * txword(f) packs tx_bits[stream][j][f][0..61] & 1 (no keystream term).

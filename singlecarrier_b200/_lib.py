@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libsinglecarrier_b200.so")
 
 SC_OK, SC_EINVAL, SC_ECUDA, SC_ENOMEM, SC_ESTATE = 0, -1, -2, -3, -4
-SC_FLAG_WIDE, SC_FLAG_DEBUG_EQ, SC_FLAG_PACKET, SC_FLAG_PACKET_DD = 0x1, 0x2, 0x4, 0x8
+SC_FLAG_WIDE, SC_FLAG_DEBUG_EQ, SC_FLAG_PACKET, SC_FLAG_PACKET_DD, SC_FLAG_PACKET_ACQ = 0x1, 0x2, 0x4, 0x8, 0x10
 
 
 class SingleCarrierError(RuntimeError):

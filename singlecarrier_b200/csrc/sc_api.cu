@@ -148,8 +148,12 @@ struct sc_modem {
     // snapshots and per-pipe scratch for the packet pass
     bool packet = false;
     bool packet_dd = false;                 // SC_FLAG_PACKET_DD: packets decoded by the decision-directed equalizer
+    bool packet_acq = false;                // SC_FLAG_PACKET_ACQ: packets found by acquisition on the samples
     DevBuf<int16_t> pk_hist2;               // frame call-2, [n][1880]
     DevBuf<float2> pk_mix_hist2;            // phasor table of frame call-2
+    DevBuf<int16_t> pk_hist3;               // SC_FLAG_PACKET_ACQ: frame call-3, [n][1880]
+    DevBuf<float2> pk_mix_hist3;            // and its phasor table
+    DevBuf<int4> acq_info[N_PIPE];          // SC_FLAG_PACKET_ACQ: per-pipe grid start, rho and nu0 of the listed packets
     DevBuf<int> pk_t_before[N_PIPE], pk_t_at[N_PIPE];         // [slab] rx_timing at entry of calls call0-1 / call0
     DevBuf<int2> pk_list[N_PIPE];
     DevBuf<int> pk_count[N_PIPE];
@@ -268,6 +272,8 @@ extern "C" int sc_create(sc_modem **out, int device, int64_t n_streams, uint32_t
     *out = nullptr;
     if ((flags & SC_FLAG_PACKET_DD) && !(flags & SC_FLAG_PACKET))
         return fail(SC_EINVAL, "sc_create: SC_FLAG_PACKET_DD needs SC_FLAG_PACKET");
+    if ((flags & SC_FLAG_PACKET_ACQ) && !((flags & SC_FLAG_PACKET) && (flags & SC_FLAG_PACKET_DD)))
+        return fail(SC_EINVAL, "sc_create: SC_FLAG_PACKET_ACQ needs SC_FLAG_PACKET and SC_FLAG_PACKET_DD");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
         cudaGetLastError();
@@ -284,6 +290,7 @@ extern "C" int sc_create(sc_modem **out, int device, int64_t n_streams, uint32_t
     m->debug_eq = (flags & SC_FLAG_DEBUG_EQ) != 0;
     m->packet = (flags & SC_FLAG_PACKET) != 0;
     m->packet_dd = (flags & SC_FLAG_PACKET_DD) != 0;
+    m->packet_acq = (flags & SC_FLAG_PACKET_ACQ) != 0;
     {
         uint16_t r = 0x4A80;                                             // scramble_init per packet
         for (int f = 0; f < 8; f++) m->pk_key.k[f] = keystream_next_word(r);
@@ -316,6 +323,12 @@ extern "C" int sc_create(sc_modem **out, int device, int64_t n_streams, uint32_t
             CU(m->pk_mix_hist2.reserve(FRAME));
             CU(cudaMemset(m->pk_mix_hist2, 0, (size_t) FRAME * sizeof(float2)));
             CU(m->pk_n_host_dev.reserve(1));
+        }
+        if (m->packet_acq) {
+            CU(m->pk_hist3.reserve((size_t) m->n * FRAME));
+            CU(cudaMemset(m->pk_hist3, 0, (size_t) m->n * FRAME * sizeof(int16_t)));
+            CU(m->pk_mix_hist3.reserve(FRAME));
+            CU(cudaMemset(m->pk_mix_hist3, 0, (size_t) FRAME * sizeof(float2)));
         }
         CU(m->unit_phase.reserve(1));
         {
@@ -475,6 +488,7 @@ static int packet_scratch(sc_modem *m) {
         CU(m->pk_list[i].reserve(PK_CAP));
         CU(m->pk_count[i].reserve(1));
         CU(m->pk_sym[i].reserve((size_t) (PK_CAP / 32) * PK_SYMS * 32));
+        if (m->packet_acq) CU(m->acq_info[i].reserve(PK_CAP));
         CU(m->pk_stream[i].create());
         CU(m->pk_ev_go[i].create());
         CU(m->pk_ev_done[i].create());
@@ -535,10 +549,20 @@ static const int16_t *fe_frame(const sc_modem *m, const Slab &s, int j, int64_t 
 }
 
 // The block's last frame becomes the history of the next block; in packet mode the one before it too (from this block
-// if it has two, else the frame the previous block saved).
+// if it has two, else the frame the previous block saved), and on ACQ banks the one before that (saved first: it may
+// come from the older history).
 static int store_history(sc_modem *m, const Slab &s) {
     const size_t pitch = FRAME * sizeof(int16_t), spitch = (size_t) s.stride * sizeof(int16_t);
     int16_t *hist = m->hist + (size_t) s.s0 * FRAME;
+    if (m->packet_acq) {
+        int16_t *h3 = m->pk_hist3 + (size_t) s.s0 * FRAME;
+        if (s.n_frames >= 3)
+            CU(cudaMemcpy2DAsync(h3, pitch, s.in + (size_t) (s.n_frames - 3) * FRAME, spitch, pitch, (size_t) s.ns,
+                                 cudaMemcpyDeviceToDevice, s.st));
+        else
+            CU(cudaMemcpyAsync(h3, (s.n_frames == 2 ? m->hist : m->pk_hist2) + (size_t) s.s0 * FRAME, (size_t) s.ns * pitch,
+                               cudaMemcpyDeviceToDevice, s.st));
+    }
     if (m->packet && s.n_frames >= 2)
         CU(cudaMemcpy2DAsync(m->pk_hist2 + (size_t) s.s0 * FRAME, pitch, s.in + (size_t) (s.n_frames - 2) * FRAME, spitch,
                              pitch, (size_t) s.ns, cudaMemcpyDeviceToDevice, s.st));
@@ -714,8 +738,10 @@ static int run_slab(sc_modem *m, const Slab &s) {
         psrc.stride = s.stride;
         psrc.hist1 = m->hist + (size_t) s0 * FRAME;
         psrc.hist2 = m->pk_hist2 + (size_t) s0 * FRAME;
+        psrc.hist3 = m->packet_acq ? m->pk_hist3 + (size_t) s0 * FRAME : nullptr;
         psrc.mix0 = mix0;
         psrc.mix_hist2 = slot0 >= 1 ? mix0 - FRAME : m->pk_mix_hist2;
+        psrc.mix_hist3 = slot0 >= 2 ? mix0 - 2 * FRAME : slot0 == 1 ? m->pk_mix_hist2 : m->pk_mix_hist3;
         psrc.timing_before_call0 = m->pk_t_before[pipe];
         psrc.timing_at_call0 = m->pk_t_at[pipe];
         psrc.call0 = call0;
@@ -763,13 +789,15 @@ static int run_slab(sc_modem *m, const Slab &s) {
             // The pass only READS what the calls up to j produced (results, frames, tables), so it runs on a side
             // stream beside the call chain: its 376-step serial kernel would otherwise sit on every call's critical path.
             NvtxRange range("sc:packet_pass");
-            int rcw = table_wait(m, st, slot0 + j, tab_waited);  // the pass reads the tables of frames up to call j-1
+            // the pass reads the tables of frames up to call j-1, acquisition up to call j
+            int rcw = table_wait(m, st, slot0 + j + (m->packet_acq ? 1 : 0), tab_waited);
             if (rcw != SC_OK) return rcw;
             CU(cudaEventRecord(m->pk_ev_go[pipe], st));
             CU(cudaStreamWaitEvent(m->pk_stream[pipe], m->pk_ev_go[pipe], 0));
+            const AcqScratch acq = {m->acq_info[pipe].p};
             CU(launch_packet_pass(psrc, ns, pk_done, j + 1, PK_CAP, m->pk_list[pipe], m->pk_count[pipe], m->pk_sym[pipe],
                                   m->pk_key, pk->packets, pk->capacity, pk->n_packets, pk->symbols, m->packet_dd,
-                                  m->pk_stream[pipe]));
+                                  m->packet_acq ? &acq : nullptr, m->pk_stream[pipe]));
             pk_done = j + 1;
         }
     }
@@ -818,7 +846,11 @@ static int start_tables(sc_modem *m, int n_frames) {
 }
 
 // the last frame's phasors become slot 0 of the next batch, and in packet mode the one before it the table of frame call-2
+// (on ACQ banks the one before that the table of frame call-3, taken first: it may be the older call-2 table)
 static int rotate_tables(sc_modem *m, int n_frames, cudaStream_t st) {
+    if (m->packet_acq)
+        CU(cudaMemcpyAsync(m->pk_mix_hist3, n_frames >= 2 ? m->mix_table + (size_t) (n_frames - 2) * FRAME : m->pk_mix_hist2,
+                           FRAME * sizeof(float2), cudaMemcpyDeviceToDevice, st));
     if (m->packet)
         CU(cudaMemcpyAsync(m->pk_mix_hist2, m->mix_table + (size_t) (n_frames - 1) * FRAME, FRAME * sizeof(float2),
                            cudaMemcpyDeviceToDevice, st));

@@ -117,19 +117,31 @@ struct PacketSrc {              // one block of calls [call0, call0 + nf) of a s
     const int16_t *in;          // block frames, stream s at in + s * stride
     long stride;
     const int16_t *hist1, *hist2;       // frames call0-1 and call0-2, [stream][1880]
+    const int16_t *hist3;       // frame call0-3 (SC_FLAG_PACKET_ACQ banks, else nullptr)
     const float2 *mix0;         // phasor table of frame call0-1; frames call0.. follow
     const float2 *mix_hist2;    // phasor table of frame call0-2
+    const float2 *mix_hist3;    // phasor table of frame call0-3 (SC_FLAG_PACKET_ACQ banks)
     const int *timing_before_call0, *timing_at_call0;   // rx_timing at entry of calls call0-1 and call0
     uint32_t call0;
     int stream0;                // bank index of the slab's first stream
     bool wide;
 };
+struct AcqScratch {             // per-pipe scratch of the acquisition pass, PK_CAP entries
+    int4 *info;
+};
 cudaError_t launch_packet_pass(const PacketSrc &src, int n_streams, int j_lo, int j_hi, int cap, int2 *list, int *count,
                                float2 *sym, const PacketKey &key, sc_packet_result *packets, long packet_capacity,
-                               unsigned long long *n_packets, float2 *packet_sym, bool dd, cudaStream_t st);
+                               unsigned long long *n_packets, float2 *packet_sym, bool dd, const AcqScratch *acq,
+                               cudaStream_t st);
 // packet_sym: nullptr, or the equalizer outputs of the 248 data steps of every packet, PK_DATA float2 per record slot
 // (record packets[k] <-> packet_sym[k * PK_DATA ..]); slots beyond packet_capacity are not written.
 // dd: decode with the decision-directed equalizer (SC_FLAG_PACKET_DD) instead of the reference's
+// acq: nullptr, or (SC_FLAG_PACKET_ACQ, with dd) the list comes from acquisition on the samples (sc_acq_kernels.cu)
+
+// sc_acq_kernels.cu: list[e] = (stream, j) and info[e] = (g - 1880 (call0 + j - 2), rho bits, nu0 bits, 0) for the
+// packets found in frame j-2 of calls [j_lo, j_hi)
+cudaError_t launch_acq_pass(const PacketSrc &src, int n_streams, int j_lo, int j_hi, int cap, int2 *list, int4 *info,
+                            int *count, cudaStream_t st);
 
 // sc_tx_kernels.cu
 struct TxArgs {

@@ -15,10 +15,13 @@
 //   packet_fir_kernel     (one warp per listed packet)    int16 -> mix -> 49-tap RRC at the 380 symbol instants
 //   packet_track_kernel   (one thread per listed packet)  the sequential loop, 128 + 248 steps
 //   packet_track_dd_kernel                                 the same with the decision-directed equalizer (SC_FLAG_PACKET_DD)
+//   packet_track_acq_kernel                                that equalizer on the grids acquisition found (SC_FLAG_PACKET_ACQ;
+//                                                          the list then comes from sc_acq_kernels.cu)
 #include "sc_common.cuh"
 #include "sc_tables.cuh"
 #include "sc_tracker.cuh"
 #include "sc_kernels.h"
+#include "sc_acq.cuh"
 
 namespace sc {
 
@@ -42,9 +45,12 @@ packet_list_kernel(const sc_frame_result *__restrict__ results, long result_stri
 constexpr int PK_NSAMP = NTAPS + CYC * (PK_SYMS - 1);                 // 1944 mixed samples
 constexpr int PK_FIR_WARPS = 2;
 
+// ACQ (SC_FLAG_PACKET_ACQ): the grid starts at g = 1880 (n-2) + info[e].x, which acquisition found; the samples
+// reach from frame n-3 to frame n.
+template <bool ACQ>
 __global__ void __launch_bounds__(PK_FIR_WARPS * 32)
 packet_fir_kernel(PacketSrc src, const int2 *__restrict__ list, const int *__restrict__ count, int cap,
-                  float2 *__restrict__ sym) {
+                  float2 *__restrict__ sym, const int4 *__restrict__ info) {
     __shared__ __align__(16) float2 smem[PK_FIR_WARPS][PK_NSAMP + 4];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int n_list = min(*count, cap);
@@ -52,6 +58,11 @@ packet_fir_kernel(PacketSrc src, const int2 *__restrict__ list, const int *__res
     for (int e = blockIdx.x * PK_FIR_WARPS + warp; e < n_list; e += gridDim.x * PK_FIR_WARPS) {
         const int2 ent = list[e];
         const int s = ent.x, j = ent.y;
+        if constexpr (ACQ) {
+            const int q0 = info[e].x - (NTAPS - 1);
+            __syncwarp();
+            for (int i = lane; i < PK_NSAMP; i += 32) mix[i] = acq_mix(src, s, j, q0 + i);
+        } else {
         const sc_frame_result *rec = src.results + (long) s * src.result_stride;
         const int mi = rec[j].max_index;
         int T;
@@ -77,6 +88,7 @@ packet_fir_kernel(PacketSrc src, const int2 *__restrict__ list, const int *__res
             const float v = (float) fr[k][qq];
             const float2 ph = __ldg(tb[k] + qq);
             mix[i] = make_float2(__fmul_rn(ph.x, v), __fmul_rn(ph.y, v));
+        }
         }
         __syncwarp();
         float2 *out = sym + ((long) (e >> 5) * PK_SYMS) * 32 + (e & 31);
@@ -167,9 +179,9 @@ packet_track_kernel(PacketSrc src, const int2 *__restrict__ list, const int *__r
     r.max_index = rec->max_index;
     r.matches = (int16_t) matches;
     r.cost = cost;
-    r.reserved0 = 0;
-    r.reserved1 = 0;
-    r.reserved2 = 0;
+    r.acq_metric = 0.0f;
+    r.acq_freq_hz = 0.0f;
+    r.grid_sample = 0;
     if (!SOFT) pos = atomicAdd(n_packets, 1ull);
     if ((long) pos < packet_capacity) packets[pos] = r;
 }
@@ -222,11 +234,14 @@ struct DdLoop {
     }
 };
 
-template <bool SOFT>
-__global__ void __launch_bounds__(128)
-packet_track_dd_kernel(PacketSrc src, const int2 *__restrict__ list, const int *__restrict__ count, int cap,
-                       const float2 *__restrict__ sym, PacketKey key, sc_packet_result *__restrict__ packets,
-                       long packet_capacity, unsigned long long *__restrict__ n_packets, float2 *__restrict__ psym) {
+// ACQ (SC_FLAG_PACKET_ACQ, packet_track_acq_kernel): the loop starts from nu = nu0 of info[e], matches counts the
+// training steps with (y.r + y.i) v_i > 0, and the record carries the grid's position, rho and the offset estimate.
+template <bool SOFT, bool ACQ>
+__device__ __forceinline__ void
+track_dd(PacketSrc src, const int2 *__restrict__ list, const int *__restrict__ count, int cap,
+         const float2 *__restrict__ sym, const PacketKey &key, sc_packet_result *__restrict__ packets,
+         long packet_capacity, unsigned long long *__restrict__ n_packets, float2 *__restrict__ psym,
+         const int4 *__restrict__ info) {
     const int n_list = min(*count, cap);
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n_list) return;
@@ -235,6 +250,12 @@ packet_track_dd_kernel(PacketSrc src, const int2 *__restrict__ list, const int *
 
     DdLoop dd;
     dd.reset();
+    int4 acq = make_int4(0, 0, 0, 0);
+    int acq_matches = 0;
+    if constexpr (ACQ) {
+        acq = info[e];
+        dd.nu = __int_as_float(acq.z);
+    }
     c32 x[EQ];
 #pragma unroll
     for (int i = 0; i < EQ - 1; i++) x[i] = from2(X[i * 32]);
@@ -243,8 +264,12 @@ packet_track_dd_kernel(PacketSrc src, const int2 *__restrict__ list, const int *
     for (int i = 0; i < PRE; i++) {
         x[EQ - 1] = nxt;
         nxt = from2(X[(i + EQ) * 32]);
-        const float a = ((c_pk_pre_neg[i >> 5] >> (i & 31)) & 1u) ? -DD_TRAIN_AMP : DD_TRAIN_AMP;
-        dd.step(x, dd.output(x), mk(a, a));
+        const bool neg = (c_pk_pre_neg[i >> 5] >> (i & 31)) & 1u;
+        const float a = neg ? -DD_TRAIN_AMP : DD_TRAIN_AMP;
+        const c32 y = dd.output(x);
+        if constexpr (ACQ)
+            if (__fmul_rn(__fadd_rn(y.r, y.i), neg ? -1.0f : 1.0f) > 0.0f) acq_matches++;
+        dd.step(x, y, mk(a, a));
 #pragma unroll
         for (int k = 0; k < EQ - 1; k++) x[k] = x[k + 1];
     }
@@ -275,35 +300,79 @@ packet_track_dd_kernel(PacketSrc src, const int2 *__restrict__ list, const int *
 #pragma unroll
         for (int kk = 0; kk < EQ - 1; kk++) x[kk] = x[kk + 1];
     }
-    const sc_frame_result *rec = src.results + (long) ent.x * src.result_stride + ent.y;
     r.stream = src.stream0 + ent.x;
-    r.call_index = src.call0 + (uint32_t) ent.y;
-    r.max_index = rec->max_index;
-    r.matches = rec->matches;
     r.cost = cost;
-    r.reserved0 = 0;
-    r.reserved1 = 0;
-    r.reserved2 = 0;
+    if constexpr (ACQ) {
+        const long long g = (long long) FRAME * ((long long) src.call0 + ent.y - 2) + acq.x;
+        const long long f = g >= 0 ? g / FRAME : -((-g + FRAME - 1) / FRAME);
+        r.call_index = (uint32_t) (2 + f);
+        r.max_index = (int16_t) ((g - f * FRAME) / CYC);
+        r.matches = (int16_t) acq_matches;
+        r.acq_metric = __int_as_float(acq.y);
+        r.acq_freq_hz = __fmul_rn(__int_as_float(acq.z), ACQ_HZ_PER_RAD);
+        r.grid_sample = g;
+    } else {
+        const sc_frame_result *rec = src.results + (long) ent.x * src.result_stride + ent.y;
+        r.call_index = src.call0 + (uint32_t) ent.y;
+        r.max_index = rec->max_index;
+        r.matches = rec->matches;
+        r.acq_metric = 0.0f;
+        r.acq_freq_hz = 0.0f;
+        r.grid_sample = 0;
+    }
     if (!SOFT) pos = atomicAdd(n_packets, 1ull);
     if ((long) pos < packet_capacity) packets[pos] = r;
 }
 
+template <bool SOFT>
+__global__ void __launch_bounds__(128)
+packet_track_dd_kernel(PacketSrc src, const int2 *__restrict__ list, const int *__restrict__ count, int cap,
+                       const float2 *__restrict__ sym, PacketKey key, sc_packet_result *__restrict__ packets,
+                       long packet_capacity, unsigned long long *__restrict__ n_packets, float2 *__restrict__ psym) {
+    track_dd<SOFT, false>(src, list, count, cap, sym, key, packets, packet_capacity, n_packets, psym, nullptr);
+}
+
+template <bool SOFT>
+__global__ void __launch_bounds__(128)
+packet_track_acq_kernel(PacketSrc src, const int2 *__restrict__ list, const int *__restrict__ count, int cap,
+                        const float2 *__restrict__ sym, PacketKey key, sc_packet_result *__restrict__ packets,
+                        long packet_capacity, unsigned long long *__restrict__ n_packets, float2 *__restrict__ psym,
+                        const int4 *__restrict__ info) {
+    track_dd<SOFT, true>(src, list, count, cap, sym, key, packets, packet_capacity, n_packets, psym, info);
+}
+
 cudaError_t launch_packet_pass(const PacketSrc &src, int n_streams, int j_lo, int j_hi, int cap, int2 *list, int *count,
                                float2 *sym, const PacketKey &key, sc_packet_result *packets, long packet_capacity,
-                               unsigned long long *n_packets, float2 *packet_sym, bool dd, cudaStream_t st) {
+                               unsigned long long *n_packets, float2 *packet_sym, bool dd, const AcqScratch *acq,
+                               cudaStream_t st) {
     cudaError_t e = cudaMemsetAsync(count, 0, sizeof(int), st);
     if (e != cudaSuccess) return e;
     const long total = (long) n_streams * (j_hi - j_lo);
     if (total <= 0) return cudaSuccess;
-    const int g1 = (int) std::min<long>((total + 255) / 256, 148L * 8);
-    packet_list_kernel<<<g1, 256, 0, st>>>(src.results, src.result_stride, n_streams, j_lo, j_hi, src.call0, cap, list, count);
+    if (acq) {
+        e = launch_acq_pass(src, n_streams, j_lo, j_hi, cap, list, acq->info, count, st);
+        if (e != cudaSuccess) return e;
+    } else {
+        const int g1 = (int) std::min<long>((total + 255) / 256, 148L * 8);
+        packet_list_kernel<<<g1, 256, 0, st>>>(src.results, src.result_stride, n_streams, j_lo, j_hi, src.call0, cap, list,
+                                               count);
+    }
     // the list length is only known on the device: size the grids for the worst case (every call valid), capped;
     // blocks beyond the list return at once
     const long worst = std::min<long>(total, cap);
     const int g2 = (int) std::min<long>((worst + PK_FIR_WARPS - 1) / PK_FIR_WARPS, 148L * 16);
-    packet_fir_kernel<<<g2, PK_FIR_WARPS * 32, 0, st>>>(src, list, count, cap, sym);
+    if (acq)
+        packet_fir_kernel<true><<<g2, PK_FIR_WARPS * 32, 0, st>>>(src, list, count, cap, sym, acq->info);
+    else
+        packet_fir_kernel<false><<<g2, PK_FIR_WARPS * 32, 0, st>>>(src, list, count, cap, sym, nullptr);
     const int g3 = (int) ((worst + 127) / 128);
-    if (dd && packet_sym)
+    if (acq && packet_sym)
+        packet_track_acq_kernel<true><<<g3, 128, 0, st>>>(src, list, count, cap, sym, key, packets, packet_capacity,
+                                                          n_packets, packet_sym, acq->info);
+    else if (acq)
+        packet_track_acq_kernel<false><<<g3, 128, 0, st>>>(src, list, count, cap, sym, key, packets, packet_capacity,
+                                                           n_packets, nullptr, acq->info);
+    else if (dd && packet_sym)
         packet_track_dd_kernel<true><<<g3, 128, 0, st>>>(src, list, count, cap, sym, key, packets, packet_capacity,
                                                          n_packets, packet_sym);
     else if (dd)
@@ -315,7 +384,7 @@ cudaError_t launch_packet_pass(const PacketSrc &src, int n_streams, int j_lo, in
     else
         packet_track_kernel<false><<<g3, 128, 0, st>>>(src, list, count, cap, sym, key, packets, packet_capacity,
                                                        n_packets, nullptr);
-    g_launch_count += 3;
+    g_launch_count += acq ? 4 : 3;
     return cudaGetLastError();
 }
 

@@ -209,8 +209,16 @@ packet_ber_stats_kernel(const sc_packet_result *__restrict__ packets, long capac
         if (g < 0 || g >= n_groups) continue;
         unsigned long long *c = acc + (long) g * SC_N_PACKET_BER_COUNTERS;
         atomicAdd(&c[0], 1ull);
-        const int t_prev = (int) __ldg(&results[s * result_stride + n - 2].rx_timing);
-        const long pos = (long) (n - 2) * FRAME + 5 * max_index + t_prev - BER_GROUP_DELAY - (lead_in ? lead_in[s] : 0);
+        // records of SC_FLAG_PACKET_ACQ banks carry their grid's position; the others 0
+        const long long gs = (long long) __ldg(reinterpret_cast<const unsigned long long *>(&packets[k].grid_sample));
+        const long lead = lead_in ? lead_in[s] : 0;
+        long pos;
+        if (gs != 0) {
+            pos = (long) gs - BER_GROUP_DELAY - lead;
+        } else {
+            const int t_prev = (int) __ldg(&results[s * result_stride + n - 2].rx_timing);
+            pos = (long) (n - 2) * FRAME + 5 * max_index + t_prev - BER_GROUP_DELAY - lead;
+        }
         long pkt = pos + period / 2;
         pkt = pkt >= 0 ? pkt / period : -((-pkt + period - 1) / period);          // floor division
         if (pkt < 0 || pkt >= n_packets) continue;

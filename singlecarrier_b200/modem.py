@@ -12,7 +12,7 @@ from typing import Optional
 
 import numpy as np
 
-from ._lib import SC_FLAG_DEBUG_EQ, SC_FLAG_PACKET, SC_FLAG_PACKET_DD, SC_FLAG_WIDE, Channel, check, lib
+from ._lib import SC_FLAG_DEBUG_EQ, SC_FLAG_PACKET, SC_FLAG_PACKET_ACQ, SC_FLAG_PACKET_DD, SC_FLAG_WIDE, Channel, check, lib
 
 FRAME_SIZE = 1880
 SYMBOLS_PER_FRAME = 376
@@ -36,8 +36,8 @@ RESULT_DTYPE = np.dtype([("bits", "<u8"), ("max_value", "<f4"), ("cost", "<f4"),
 assert RESULT_DTYPE.itemsize == 32
 # sc_packet_result (packet mode, an extension without a counterpart in the reference)
 PACKET_DTYPE = np.dtype([("bits", "<u8", (8,)), ("stream", "<i4"), ("call_index", "<u4"), ("max_index", "<i2"),
-                         ("matches", "<i2"), ("cost", "<f4"), ("reserved0", "<u4"), ("reserved1", "<u4"),
-                         ("reserved2", "<u8")])
+                         ("matches", "<i2"), ("cost", "<f4"), ("acq_metric", "<f4"), ("acq_freq_hz", "<f4"),
+                         ("grid_sample", "<i8")])
 assert PACKET_DTYPE.itemsize == 96
 
 
@@ -194,14 +194,16 @@ class ModemBank:
     """A bank of ``n_streams`` synchronized modems on one GPU (sc_modem handle)."""
 
     def __init__(self, n_streams: int, device: int = 0, wide: bool = False, foffset_hz: float = 0.0,
-                 debug_eq: bool = False, packet: bool = False, dd: bool = False):
+                 debug_eq: bool = False, packet: bool = False, dd: bool = False, acq: bool = False):
         """packet: packet mode (SC_FLAG_PACKET); dd: its packets decoded by the decision-directed equalizer
-        (SC_FLAG_PACKET_DD, needs packet=True)."""
+        (SC_FLAG_PACKET_DD, needs packet=True); acq: packets found by acquisition on the samples (SC_FLAG_PACKET_ACQ,
+        needs packet=True and dd=True)."""
         self._h = C.c_void_p()
         flags = (SC_FLAG_WIDE if wide else 0) | (SC_FLAG_DEBUG_EQ if debug_eq else 0) | (SC_FLAG_PACKET if packet else 0) \
-            | (SC_FLAG_PACKET_DD if dd else 0)
+            | (SC_FLAG_PACKET_DD if dd else 0) | (SC_FLAG_PACKET_ACQ if acq else 0)
         self.packet = packet
         self.dd = dd
+        self.acq = acq
         check(lib.sc_create(C.byref(self._h), device, n_streams, flags, foffset_hz))
         self.n_streams = n_streams
         self.device = device
