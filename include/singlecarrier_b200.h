@@ -446,6 +446,59 @@ int sc_packet_ber_stats_dev(int device, const sc_packet_result *packets, int64_t
                             const uint8_t *tx_bits, int n_packets, const int32_t *lead_in, int gap_samples,
                             const int32_t *group, int n_groups, uint64_t *counters, void *stream);
 
+/* ---- coded payload of packet-mode packets (DESIGN.md section 8c) -------------------------------------------------
+ *
+ * A fixed code on top of the packet format: SC_PACKET_PAYLOAD_BYTES bytes of payload, a CRC-16, a K = 7 rate-1/2
+ * convolutional code and a block interleaver fill the first SC_PACKET_CODED_BITS of a packet's SC_PACKET_BITS bits;
+ * the rest (the last ten data symbols, which the transmitter emits only in part) carry 0 and are never read.
+ *   crc      CRC-16/CCITT-FALSE over the payload (poly 0x1021, init 0xFFFF, MSB first, no reflection, no final XOR:
+ *            "123456789" -> 0x29B1), appended high byte first
+ *   info     u[0..231] = the 29 bytes MSB first, u[232..237] = 0 (the encoder ends in state 0)
+ *   encoder  s_t = (u[t-1] .. u[t-6]) with u[t-1] at bit 5, s_0 = 0; r = (u[t] << 6) | s_t;
+ *            c[2t] = parity(r & 0133), c[2t+1] = parity(r & 0171) (octal), s_{t+1} = r >> 1; t = 0..237
+ *   layout   packet bit p = 62 f + j (data frame f, bit j: the layout of sc_tx_*_dev's bits and of
+ *            sc_packet_result.bits): c[n] goes to p = 17 (n mod 28) + floor(n / 28); p = 476..495 carry 0
+ * All three entry points take a device, not a bank; pointers are device pointers.  SC_EINVAL before any CUDA call
+ * on a NULL pointer, n or capacity < 0, or a misaligned pointer. */
+#define SC_PACKET_PAYLOAD_BYTES 27
+#define SC_PACKET_CODED_BITS    476
+#define SC_PACKET_BITS          496
+
+typedef struct {
+    uint8_t  data[27];      /* the decoder's maximum-likelihood payload, also when crc_ok is 0 */
+    uint8_t  crc_ok;        /* 1 when the CRC of data equals the decoded CRC bits */
+    uint16_t flipped;       /* coded bits 0..475 whose LLR sign (L < 0: bit 1) disagrees with the decoded codeword */
+    uint16_t reserved;      /* 0 */
+} sc_packet_payload;        /* 32 bytes */
+
+/* payload [n][27] -> bits [n][8][62] of 0/1, the bits sc_tx_packets_dev / sc_tx_channel_dev take: payloads laid out
+ * [n_streams][n_packets][27] feed the transmitter directly.  n == 0 launches nothing. */
+int sc_packet_encode_dev(int device, const uint8_t *payload, int64_t n, uint8_t *bits, void *stream);
+
+/* Log-likelihood ratios of the 496 bits of every packet record, L > 0 favouring bit 0, from the packet symbols of
+ * sc_rx_packets_soft_*: for record k < min(*n_found, capacity), 496 floats at llr + k * 496 from the 248 complex
+ * floats at packet_symbols + k * 496 (the indexing of packet_symbols).  n_found is a DEVICE pointer read by the
+ * kernel, so the call queues behind sc_rx_packets_soft_dev without a host synchronisation; blocks at or beyond that
+ * count are not touched.  With y the record's block and d_i = (y_i.r < 0 ? -1 : 1) + j (y_i.i < 0 ? -1 : 1):
+ *   v = sum_i |y_i - d_i|^2 / 496 (float32, floored at 1e-6), a per-packet estimate of the noise variance per
+ *       dimension;
+ *   bit 2i of frame f: L = 2 Im(y[31 f + i]) / v, bit 2i+1: L = 2 Re(y[31 f + i]) / v, negated where bit 2i (2i+1)
+ *       of sc_packet_keystream_word(f) is 1; a non-finite L is written as 0.
+ * So bit == (L < 0) is the record's hard decision wherever L != 0.  The estimate v assumes the DD loop's output
+ * (SC_FLAG_PACKET_DD / SC_FLAG_PACKET_ACQ banks).  On a plain SC_FLAG_PACKET bank the symbols are the reference
+ * Kalman equalizer's and the LLRs are defined but useless.  The decoder below does not depend on their scale.
+ * packet_symbols and llr must be aligned to 8 bytes.  capacity == 0 launches nothing. */
+int sc_packet_llr_dev(int device, const float *packet_symbols, int64_t capacity, const uint64_t *n_found, float *llr,
+                      void *stream);
+
+/* Soft-decision Viterbi decoding of the packet code: for record k < min(*n_found, capacity) (n_found read on the
+ * device, as for sc_packet_llr_dev), the 496 LLRs at llr + k * 496 -> out[k].  Correlation metric, maximised, in
+ * float32 with adds and compares only: each LLR is first sanitised (non-finite -> 0, clamped to +-2^24); ties go to
+ * the predecessor whose newest-dropped bit is 0; traceback from state 0.  data holds the maximum-likelihood payload
+ * even when crc_ok is 0.  llr must be aligned to 8 bytes and out to 4.  capacity == 0 launches nothing. */
+int sc_packet_decode_dev(int device, const float *llr, int64_t capacity, const uint64_t *n_found,
+                         sc_packet_payload *out, void *stream);
+
 /* ---- multi-GPU reduction of the counters (SURVEY section 8e: the path's only collective) ------------------ */
 
 /* ncclAllReduce(sum) of n_counters uint64 in place on `stream`; nccl_comm is a ncclComm_t created by the

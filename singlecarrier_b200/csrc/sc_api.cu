@@ -1631,6 +1631,42 @@ extern "C" int sc_packet_ber_stats_dev(int device, const sc_packet_result *packe
     return SC_OK;
 }
 
+// ---- coded payload (DESIGN.md section 8c) -------------------------------------------------------
+extern "C" int sc_packet_encode_dev(int device, const uint8_t *payload, int64_t n, uint8_t *bits, void *stream) {
+    if (!payload || !bits || n < 0) return fail(SC_EINVAL, "sc_packet_encode_dev: bad arguments");
+    int rc = stage_device(device);
+    if (rc != SC_OK) return rc;
+    if (n == 0) return SC_OK;
+    CU(launch_packet_encode(payload, n, bits, (cudaStream_t) stream));
+    return SC_OK;
+}
+
+extern "C" int sc_packet_llr_dev(int device, const float *packet_symbols, int64_t capacity, const uint64_t *n_found,
+                                 float *llr, void *stream) {
+    if (!packet_symbols || !n_found || !llr || capacity < 0) return fail(SC_EINVAL, "sc_packet_llr_dev: bad arguments");
+    if (((uintptr_t) packet_symbols & 7) != 0 || ((uintptr_t) llr & 7) != 0)
+        return fail(SC_EINVAL, "sc_packet_llr_dev: packet_symbols and llr must be 8-byte aligned");
+    int rc = stage_device(device);
+    if (rc != SC_OK) return rc;
+    if (capacity == 0) return SC_OK;
+    PacketKey key;
+    for (int f = 0; f < 8; f++) key.k[f] = sc_packet_keystream_word(f);
+    CU(launch_packet_llr(packet_symbols, capacity, (const unsigned long long *) n_found, llr, key, (cudaStream_t) stream));
+    return SC_OK;
+}
+
+extern "C" int sc_packet_decode_dev(int device, const float *llr, int64_t capacity, const uint64_t *n_found,
+                                    sc_packet_payload *out, void *stream) {
+    if (!llr || !n_found || !out || capacity < 0) return fail(SC_EINVAL, "sc_packet_decode_dev: bad arguments");
+    if (((uintptr_t) llr & 7) != 0 || ((uintptr_t) out & 3) != 0)
+        return fail(SC_EINVAL, "sc_packet_decode_dev: llr must be 8-byte and out 4-byte aligned");
+    int rc = stage_device(device);
+    if (rc != SC_OK) return rc;
+    if (capacity == 0) return SC_OK;
+    CU(launch_packet_decode(llr, capacity, (const unsigned long long *) n_found, out, (cudaStream_t) stream));
+    return SC_OK;
+}
+
 // ---- checkpoint / resume ------------------------------------------------------------------------
 namespace {
 struct StateHeader {

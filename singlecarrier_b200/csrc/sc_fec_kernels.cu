@@ -1,0 +1,269 @@
+// sc_fec_kernels.cu -- the coded payload of packet-mode packets (DESIGN.md section 8c): encoder, LLRs and a
+// soft-decision Viterbi decoder.  The specification is tests/packet_fec_ref.c; every kernel here is bit-identical
+// to it.  The decoder uses adds and compares only (one rounding per add, no multiply that could be contracted).
+#include "sc_common.cuh"
+#include "sc_kernels.h"
+
+namespace sc {
+
+constexpr int FEC_STEPS = 238;                      // 232 info bits + 6 tail bits
+constexpr int FEC_CODED = SC_PACKET_CODED_BITS;     // 476
+constexpr int FEC_BITS = SC_PACKET_BITS;            // 496 floats / bits per packet
+constexpr int FEC_SYMS = FEC_BITS / 2;              // 248
+constexpr int FEC_WARPS = 8;                        // records per 256-thread block of the LLR and Viterbi kernels
+constexpr unsigned FEC_G0 = 0133, FEC_G1 = 0171;
+constexpr float FEC_CLAMP = 16777216.0f;            // 2^24: 476 x 2^24 keeps every path metric far below FLT_MAX
+
+// CRC-16/CCITT-FALSE byte table, built by the block in shared memory (no module-scope table: a new __constant__
+// symbol would move the constant-bank offsets of every other kernel of the library)
+__device__ __forceinline__ void fec_crc_table(unsigned *tab) {
+    for (int b = threadIdx.x; b < 256; b += blockDim.x) {
+        unsigned c = (unsigned) b << 8;
+        for (int i = 0; i < 8; i++) c = (c & 0x8000u) ? ((c << 1) ^ 0x1021u) & 0xffffu : (c << 1) & 0xffffu;
+        tab[b] = c;
+    }
+    __syncthreads();
+}
+
+__device__ __forceinline__ unsigned fec_crc_byte(const unsigned *tab, unsigned crc, unsigned byte) {
+    return ((crc << 8) ^ tab[((crc >> 8) ^ byte) & 0xffu]) & 0xffffu;
+}
+
+// Info bits are held as words: bit t of the 238 at bit t & 31 of word t >> 5.  Coded bit n reads the window
+// u[t-6 .. t] (t = n / 2, u of negative index 0), which is r = (u[t] << 6) | s_t bit for bit.
+__device__ __forceinline__ unsigned fec_code_bit(unsigned hi, unsigned lo, int n) {
+    const int t = n >> 1;
+    const unsigned long long x = ((unsigned long long) hi << 32) | lo;    // hi = word t >> 5, lo = the word before
+    const unsigned r = (unsigned) (x >> (26 + (t & 31))) & 127u;
+    return (unsigned) __popc(r & ((n & 1) ? FEC_G1 : FEC_G0)) & 1u;
+}
+
+// packet bit position p -> the coded bit n with pi(n) = p; the padding positions 476..495 map to themselves
+__device__ __forceinline__ int fec_coded_index(int p) { return p < FEC_CODED ? 28 * (p % 17) + p / 17 : p; }
+
+// 4 bytes, first at bits 0..7, MSB first -> the info-bit word (and back: the map is an involution)
+__device__ __forceinline__ unsigned fec_bytes_to_bits(unsigned w) { return __brev(__byte_perm(w, 0, 0x0123)); }
+
+__device__ __forceinline__ long fec_records(long capacity, const unsigned long long *n_found) {
+    const unsigned long long found = *n_found;
+    return found < (unsigned long long) capacity ? (long) found : capacity;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Encoder: one thread per packet.  Its info words live in a shared-memory column of its own.
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+packet_encode_kernel(const uint8_t *__restrict__ payload, long n, uint8_t *__restrict__ bits) {
+    __shared__ unsigned sh_u[8][256];
+    __shared__ unsigned sh_crc[256];
+    fec_crc_table(sh_crc);
+    const int tid = threadIdx.x;
+    for (long k = (long) blockIdx.x * blockDim.x + tid; k < n; k += (long) gridDim.x * blockDim.x) {
+        const uint8_t *p = payload + k * SC_PACKET_PAYLOAD_BYTES;
+        unsigned crc = 0xffffu, w = 0u;
+        for (int b = 0; b < 29; b++) {
+            unsigned byte;
+            if (b < SC_PACKET_PAYLOAD_BYTES) {
+                byte = __ldg(p + b);
+                crc = fec_crc_byte(sh_crc, crc, byte);
+            } else {
+                byte = b == SC_PACKET_PAYLOAD_BYTES ? crc >> 8 : crc & 0xffu;
+            }
+            w |= byte << (8 * (b & 3));
+            if ((b & 3) == 3 || b == 28) {
+                sh_u[b >> 2][tid] = fec_bytes_to_bits(w);
+                w = 0u;
+            }
+        }
+        uint8_t *out = bits + k * FEC_BITS;
+        const bool vec = ((uintptr_t) out & 15) == 0;
+        for (int q = 0; q < FEC_BITS / 16; q++) {
+            unsigned v[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+            for (int e = 0; e < 16; e++) {
+                const int pbit = 16 * q + e;
+                if (pbit < FEC_CODED) {
+                    const int nn = fec_coded_index(pbit);
+                    const int wt = nn >> 6;                                // word of t = nn / 2
+                    v[e >> 2] |= fec_code_bit(sh_u[wt][tid], wt ? sh_u[wt - 1][tid] : 0u, nn) << (8 * (e & 3));
+                }
+            }
+            if (vec) {
+                *reinterpret_cast<uint4 *>(out + 16 * q) = make_uint4(v[0], v[1], v[2], v[3]);
+            } else {
+#pragma unroll
+                for (int e = 0; e < 16; e++) out[16 * q + e] = (uint8_t) (v[e >> 2] >> (8 * (e & 3)));
+            }
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// LLRs: one warp per record.  Lane l loads symbols l, l + 32, ... (coalesced float2) and sums their squared
+// slicer errors in that order; an xor butterfly completes S in the order the specification writes out.
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+packet_llr_kernel(const float2 *__restrict__ sym, long capacity, const unsigned long long *__restrict__ n_found,
+                  float2 *__restrict__ llr, PacketKey key) {
+    __shared__ unsigned long long sh_ks[8];
+    if (threadIdx.x < 8) {                          // selects, not an index: the parameter stays out of local memory
+        unsigned long long v = key.k[0];
+#pragma unroll
+        for (int f = 1; f < 8; f++) v = threadIdx.x == f ? key.k[f] : v;
+        sh_ks[threadIdx.x] = v;
+    }
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const long n_rec = fec_records(capacity, n_found);
+    for (long k = (long) blockIdx.x * FEC_WARPS + (threadIdx.x >> 5); k < n_rec; k += (long) gridDim.x * FEC_WARPS) {
+        const float2 *y = sym + k * FEC_SYMS;
+        float acc = 0.0f;
+#pragma unroll
+        for (int i = 0; i < 8; i++) {
+            const int idx = lane + 32 * i;
+            if (idx < FEC_SYMS) {
+                const float2 v = __ldg(y + idx);
+                const float er = __fsub_rn(v.x, v.x < 0.0f ? -1.0f : 1.0f);
+                const float ei = __fsub_rn(v.y, v.y < 0.0f ? -1.0f : 1.0f);
+                acc = __fadd_rn(acc, __fadd_rn(__fmul_rn(er, er), __fmul_rn(ei, ei)));
+            }
+        }
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) acc = __fadd_rn(acc, __shfl_xor_sync(0xffffffffu, acc, off));
+        float var = __fdiv_rn(acc, 496.0f);
+        if (!(var >= 1e-6f)) var = 1e-6f;
+        float2 *out = llr + k * FEC_SYMS;
+#pragma unroll
+        for (int i = 0; i < 8; i++) {
+            const int idx = lane + 32 * i;
+            if (idx < FEC_SYMS) {
+                const int f = idx / SC_DATA_SYMBOLS, j = 2 * (idx - f * SC_DATA_SYMBOLS);
+                const unsigned long long w = sh_ks[f] >> j;
+                // loaded again (an L1 hit) rather than kept: live across the divide's out-of-line slow path, the
+                // block would be saved to the stack
+                const float2 v = __ldg(y + idx);
+                float lq = __fdiv_rn(__fmul_rn(2.0f, v.y), var), li = __fdiv_rn(__fmul_rn(2.0f, v.x), var);
+                if (w & 1ull) lq = -lq;
+                if (w & 2ull) li = -li;
+                out[idx] = make_float2(isfinite(lq) ? lq : 0.0f, isfinite(li) ? li : 0.0f);
+            }
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Viterbi: one warp per record, lane l owns states l and l + 32.  Both of its new states have the predecessors
+// 2l and 2l + 1, and the two generators share their first and last taps, so one metric M serves all four
+// branches: +M for (l <- 2l), (l + 32 <- 2l + 1), -M for the other two.  Two shuffles bring pm[2l], pm[2l + 1]:
+// even lanes offer (pm_l, pm_{l+32}), odd lanes the swapped pair.  Decisions go to shared memory by two ballots.
+// ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ float fec_sanitise(float x) {
+    return isfinite(x) ? fminf(fmaxf(x, -FEC_CLAMP), FEC_CLAMP) : 0.0f;
+}
+
+__global__ void __launch_bounds__(256)
+packet_viterbi_kernel(const float2 *__restrict__ llr, long capacity, const unsigned long long *__restrict__ n_found,
+                      sc_packet_payload *__restrict__ out) {
+    __shared__ __align__(8) float sh_l[FEC_WARPS][FEC_BITS];    // L'[pi(n)] at n: step t reads one float2
+    __shared__ uint2 sh_dec[FEC_WARPS][FEC_STEPS];
+    __shared__ unsigned sh_u[FEC_WARPS][8];
+    __shared__ unsigned sh_crc[256];
+    fec_crc_table(sh_crc);
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const bool hi = lane >= 16, odd = lane & 1;
+    const int src_a = (2 * lane + (hi ? 1 : 0)) & 31, src_b = (2 * lane + (hi ? 0 : 1)) & 31;
+    const bool neg0 = __popc((2u * lane) & FEC_G0) & 1, neg1 = __popc((2u * lane) & FEC_G1) & 1;
+    float *L = sh_l[w];
+    const long n_rec = fec_records(capacity, n_found);
+    for (long k = (long) blockIdx.x * FEC_WARPS + w; k < n_rec; k += (long) gridDim.x * FEC_WARPS) {
+        const float2 *src = llr + k * FEC_SYMS;
+#pragma unroll
+        for (int i = 0; i < 8; i++) {
+            const int idx = lane + 32 * i;
+            if (idx < FEC_SYMS) {
+                const float2 x = __ldg(src + idx);
+                L[fec_coded_index(2 * idx)] = fec_sanitise(x.x);
+                L[fec_coded_index(2 * idx + 1)] = fec_sanitise(x.y);
+            }
+        }
+        __syncwarp();
+        float pm0 = lane == 0 ? 0.0f : -INFINITY, pm1 = -INFINITY;
+        for (int t = 0; t < FEC_STEPS; t++) {
+            const float2 l = reinterpret_cast<const float2 *>(L)[t];
+            const float l0 = l.x, l1 = l.y;
+            const float m = __fadd_rn(neg0 ? -l0 : l0, neg1 ? -l1 : l1);
+            const float a = __shfl_sync(0xffffffffu, odd ? pm1 : pm0, src_a);
+            const float b = __shfl_sync(0xffffffffu, odd ? pm0 : pm1, src_b);
+            const float p0 = hi ? b : a, p1 = hi ? a : b;                 // pm[2l], pm[2l + 1]
+            const float c00 = __fadd_rn(p0, m), c01 = __fadd_rn(p1, -m);
+            const float c10 = __fadd_rn(p0, -m), c11 = __fadd_rn(p1, m);
+            const bool t0 = c01 > c00, t1 = c11 > c10;
+            pm0 = t0 ? c01 : c00;
+            pm1 = t1 ? c11 : c10;
+            const unsigned d0 = __ballot_sync(0xffffffffu, t0), d1 = __ballot_sync(0xffffffffu, t1);
+            if (lane == (t & 31)) sh_dec[w][t] = make_uint2(d0, d1);
+        }
+        __syncwarp();
+        // traceback, uniform over the warp: bit t of the decoded info goes to bit t & 31 of word t >> 5
+        unsigned s = 0u, word = 0u;
+        for (int t = FEC_STEPS - 1; t >= 0; t--) {
+            word = (word << 1) | (s >> 5);
+            if ((t & 31) == 0 && lane == 0) sh_u[w][t >> 5] = word;
+            const uint2 d = sh_dec[w][t];
+            s = ((s << 1) & 63u) | (((s & 32u) ? d.y : d.x) >> (s & 31u) & 1u);
+        }
+        __syncwarp();
+        unsigned flipped = 0u;
+        for (int n = lane; n < FEC_CODED; n += 32) {
+            const int wt = n >> 6;
+            const unsigned c = fec_code_bit(sh_u[w][wt], wt ? sh_u[w][wt - 1] : 0u, n);
+            flipped += (L[n] < 0.0f) != (c != 0u);
+        }
+        flipped = __reduce_add_sync(0xffffffffu, flipped);
+        unsigned crc = 0xffffu;
+        for (int q = 0; q < 7; q++) {
+            const unsigned by = fec_bytes_to_bits(sh_u[w][q]);           // payload bytes 4q .. 4q + 3
+            const int nb = q < 6 ? 4 : 3;
+            for (int e = 0; e < nb; e++) crc = fec_crc_byte(sh_crc, crc, (by >> (8 * e)) & 0xffu);
+        }
+        const unsigned b6 = fec_bytes_to_bits(sh_u[w][6]), b7 = fec_bytes_to_bits(sh_u[w][7]);
+        const unsigned rx_crc = ((b6 >> 24) << 8) | (b7 & 0xffu);
+        if (lane < 8) {
+            unsigned v;
+            if (lane < 6) v = fec_bytes_to_bits(sh_u[w][lane]);
+            else if (lane == 6) v = (b6 & 0x00ffffffu) | ((crc == rx_crc ? 1u : 0u) << 24);
+            else v = flipped;                                              // flipped, reserved = 0
+            reinterpret_cast<unsigned *>(out + k)[lane] = v;
+        }
+        __syncwarp();                                                      // L and sh_u are reused by the next record
+    }
+}
+
+// grid-stride loops: at most max_blocks CTAs (several per SM), each taking further records after its first
+static int fec_grid(long work, int per_block, int max_blocks) {
+    return (int) std::max<long>(1, std::min<long>((work + per_block - 1) / per_block, max_blocks));
+}
+
+cudaError_t launch_packet_encode(const uint8_t *payload, long n, uint8_t *bits, cudaStream_t st) {
+    packet_encode_kernel<<<fec_grid(n, 256, 148 * 2), 256, 0, st>>>(payload, n, bits);
+    g_launch_count++;
+    return cudaGetLastError();
+}
+
+cudaError_t launch_packet_llr(const float *packet_symbols, long capacity, const unsigned long long *n_found, float *llr,
+                              const PacketKey &key, cudaStream_t st) {
+    packet_llr_kernel<<<fec_grid(capacity, FEC_WARPS, 148 * 16), 32 * FEC_WARPS, 0, st>>>(
+        reinterpret_cast<const float2 *>(packet_symbols), capacity, n_found, reinterpret_cast<float2 *>(llr), key);
+    g_launch_count++;
+    return cudaGetLastError();
+}
+
+cudaError_t launch_packet_decode(const float *llr, long capacity, const unsigned long long *n_found,
+                                 sc_packet_payload *out, cudaStream_t st) {
+    packet_viterbi_kernel<<<fec_grid(capacity, FEC_WARPS, 148 * 16), 32 * FEC_WARPS, 0, st>>>(
+        reinterpret_cast<const float2 *>(llr), capacity, n_found, out);
+    g_launch_count++;
+    return cudaGetLastError();
+}
+
+}  // namespace sc

@@ -143,6 +143,13 @@ cudaError_t launch_packet_pass(const PacketSrc &src, int n_streams, int j_lo, in
 cudaError_t launch_acq_pass(const PacketSrc &src, int n_streams, int j_lo, int j_hi, int cap, int2 *list, int4 *info,
                             int *count, cudaStream_t st);
 
+// sc_fec_kernels.cu -- the coded payload (DESIGN.md section 8c); capacity >= 1, n_found read on the device
+cudaError_t launch_packet_encode(const uint8_t *payload, long n, uint8_t *bits, cudaStream_t st);
+cudaError_t launch_packet_llr(const float *packet_symbols, long capacity, const unsigned long long *n_found, float *llr,
+                              const PacketKey &key, cudaStream_t st);
+cudaError_t launch_packet_decode(const float *llr, long capacity, const unsigned long long *n_found,
+                                 sc_packet_payload *out, cudaStream_t st);
+
 // sc_tx_kernels.cu
 struct TxArgs {
     const uint8_t *bits;        // [n][n_packets][8][62] or nullptr

@@ -14,7 +14,8 @@ from typing import Optional
 
 import numpy as np
 
-from .modem import FRAME_SIZE, N_PACKET_BER_COUNTERS, REFERENCE_GAP, ModemBank, keystream_word
+from .modem import (FRAME_SIZE, N_PACKET_BER_COUNTERS, PACKET_CODED_BITS, PACKET_DTYPE, PAYLOAD_BYTES, PAYLOAD_DTYPE,
+                    REFERENCE_GAP, ModemBank, keystream_word)
 from .taps import modem_taps
 
 PERIOD = FRAME_SIZE + REFERENCE_GAP          # 2783 samples: one packet + dead air (qpsk.c:384,405,410-412)
@@ -34,6 +35,7 @@ class Workload:
     ebn0_db: Optional["object"]  # CUDA float [n_streams] or None
     n_packets: int
     channel: Optional[dict] = None   # the per-stream channel parameter tensors that were applied
+    payload: Optional["object"] = None   # CUDA uint8 [n_streams, n_packets, 27] when the packets carry coded payloads
 
 
 def awgn_sigma(ebn0_db, torch):
@@ -44,11 +46,13 @@ def awgn_sigma(ebn0_db, torch):
 
 
 def synthesize(bank: ModemBank, samples_per_stream: int, seed: int, *, config: int, gap: int = REFERENCE_GAP,
-               ebn0_db=None) -> Workload:
+               ebn0_db=None, payload=None) -> Workload:
     """config 2: clean channel, random df/phase, lead-in 80+5m (preamble lands on decimated index m).
     config 3: + AWGN at ebn0_db[s] (default: 13 points 0..12 dB, striped by stream index).
     config 4: bench workload (config 3 channel, random lead-in).
-    config 5: + linear drift (+-2 Hz/s) and a 2-tap echo (a 0.1..0.5, delay 1..10 samples) at 10 dB."""
+    config 5: + linear drift (+-2 Hz/s) and a 2-tap echo (a 0.1..0.5, delay 1..10 samples) at 10 dB.
+    payload: None (random bits), or CUDA uint8 [n_streams, n_packets, 27]: the packets carry these payloads through the
+    packet code (sc_packet_encode_dev); n_packets must be the number the stream's length gives."""
     import torch
     dev = torch.device("cuda", bank.device)
     n = bank.n_streams
@@ -78,9 +82,15 @@ def synthesize(bank: ModemBank, samples_per_stream: int, seed: int, *, config: i
         ch["echo_delay"] = torch.randint(1, 11, (n,), generator=g, device=dev, dtype=torch.int32)
     out = torch.empty((n, samples_per_stream), dtype=torch.int16, device=dev)
     bits = torch.empty((n, n_packets, 8, 62), dtype=torch.uint8, device=dev)
-    bank.tx_packets_dev(out, n_packets, gap_samples=gap, seed=seed, bits_out=bits, lead_in=lead, channel=ch)
+    if payload is None:
+        bank.tx_packets_dev(out, n_packets, gap_samples=gap, seed=seed, bits_out=bits, lead_in=lead, channel=ch)
+    else:
+        assert tuple(payload.shape) == (n, n_packets, PAYLOAD_BYTES) and payload.dtype == torch.uint8, "payload shape"
+        payload = payload.to(dev).contiguous()
+        bank.packet_encode(payload, bits)
+        bank.tx_packets_dev(out, n_packets, gap_samples=gap, seed=seed, bits=bits, lead_in=lead, channel=ch)
     torch.cuda.synchronize(dev)
-    return Workload(out, bits, lead, gap, eb, n_packets, ch)
+    return Workload(out, bits, lead, gap, eb, n_packets, ch, payload)
 
 
 def demodulate(bank: ModemBank, samples, n_frames: int):
@@ -179,3 +189,68 @@ def packet_ber_dev(bank: ModemBank, packets, n_found, res, n_frames: int, wl: Wo
         comm.all_reduce_counters(cnt)
     torch.cuda.synchronize(res.device)
     return packet_counters(cnt.cpu().numpy())
+
+
+def _host(x):
+    return x.cpu().numpy() if hasattr(x, "cpu") else np.asarray(x)
+
+
+def _packed_words(tx_bits, chunk: int = 8192):
+    """uint8 [n, n_packets, 8, 62] of 0/1 -> uint64 [n, n_packets, 8], bit k of word f = bit k of frame f"""
+    n = tx_bits.shape[0]
+    out = np.zeros(tuple(tx_bits.shape[:3]), np.uint64)
+    for a in range(0, n, chunk):
+        t = _host(tx_bits[a:a + chunk])
+        t = np.concatenate([t, np.zeros(t.shape[:3] + (2,), np.uint8)], axis=-1)
+        out[a:a + chunk] = np.packbits(t, axis=-1, bitorder="little").view("<u8")[..., 0]
+    return out
+
+
+def packet_fec(packets, n_found: int, decoded, res, n_frames: int, wl: Workload, group=None, n_groups: int = 1):
+    """Host recount of the coded payloads of packet records against the workload's payloads (wl.payload).
+
+    packets: the records (PACKET_DTYPE, or the CUDA uint8 buffer rx_packets_*_dev filled), n_found: their number (the
+    first min(n_found, capacity) are counted), decoded: the matching sc_packet_payload records (PAYLOAD_DTYPE or a
+    CUDA uint8 buffer), res: the batch's results (CUDA uint8 [n_streams, >= n_frames * 32] or RESULT_DTYPE).
+    Records are counted and aligned to transmitted packet j by the rule of sc_packet_ber_stats_dev (grid_sample when it
+    is not 0, else call index, max_index and rx_timing).  Returns numpy int64 arrays per group: records, aligned,
+    crc_ok (aligned records whose CRC checks), correct (aligned, crc_ok and the payload transmitted), undetected
+    (aligned, crc_ok and another payload), raw_errors (hard-decision errors over the coded bits 0..475 of aligned
+    records) and raw_packet_errors (aligned records with at least one)."""
+    assert wl.payload is not None, "the workload carries no coded payload"
+    pay = _host(wl.payload).reshape(-1, wl.n_packets, PAYLOAD_BYTES)
+    pk = _host(packets).view(PACKET_DTYPE).reshape(-1)
+    dec = _host(decoded).view(PAYLOAD_DTYPE).reshape(-1)
+    kept = min(int(n_found), pk.size, dec.size)
+    pk, dec = pk[:kept], dec[:kept]
+    r = _host(res)
+    n_streams = pay.shape[0]
+    timing = r.view(np.uint8).reshape(n_streams, -1, 32)[:, :, 20:22].copy().view("<i2")[..., 0].astype(np.int64)
+    lead = _host(wl.lead).astype(np.int64)
+    grp = np.zeros(n_streams, np.int64) if group is None else _host(group).astype(np.int64)
+    s = pk["stream"].astype(np.int64)
+    n = pk["call_index"].astype(np.int64)
+    ok = (s >= 0) & (s < n_streams) & (n >= 2) & (n < n_frames)
+    s, n = np.where(ok, s, 0), np.where(ok, n, 2)
+    g = grp[s]
+    ok &= (g >= 0) & (g < n_groups)
+    gs = pk["grid_sample"].astype(np.int64)
+    pos = np.where(gs != 0, gs, (n - 2) * FRAME_SIZE + 5 * pk["max_index"].astype(np.int64) + timing[s, n - 2]) \
+        - GROUP_DELAY - lead[s]
+    period = FRAME_SIZE + wl.gap
+    j = np.floor_divide(pos + period // 2, period)
+    al = ok & (j >= 0) & (j < wl.n_packets) & (np.abs(pos - j * period) <= 10)
+    j = np.clip(j, 0, wl.n_packets - 1)
+    crc = dec["crc_ok"] != 0
+    same = (dec["data"] == pay[s, j]).all(axis=1)
+    # hard decisions against the transmitted bits, packed like the records' words (bit k of word f = bit 62 f + k)
+    txw = _packed_words(wl.tx_bits)[s, j]
+    mask = np.array([(1 << 62) - 1] * 7 + [(1 << (PACKET_CODED_BITS - 7 * 62)) - 1], np.uint64)
+    raw = np.bitwise_count((pk["bits"] ^ txw) & mask).sum(axis=1).astype(np.int64)
+    out = {k: np.zeros(n_groups, np.int64) for k in ("records", "aligned", "crc_ok", "correct", "undetected",
+                                                      "raw_errors", "raw_packet_errors")}
+    for name, m, w in (("records", ok, None), ("aligned", al, None), ("crc_ok", al & crc, None),
+                       ("correct", al & crc & same, None), ("undetected", al & crc & ~same, None),
+                       ("raw_errors", al, raw), ("raw_packet_errors", al & (raw > 0), None)):
+        np.add.at(out[name], g[m], 1 if w is None else w[m])
+    return out

@@ -39,6 +39,10 @@ PACKET_DTYPE = np.dtype([("bits", "<u8", (8,)), ("stream", "<i4"), ("call_index"
                          ("matches", "<i2"), ("cost", "<f4"), ("acq_metric", "<f4"), ("acq_freq_hz", "<f4"),
                          ("grid_sample", "<i8")])
 assert PACKET_DTYPE.itemsize == 96
+# sc_packet_payload: one decoded packet of the coded payload (DESIGN.md section 8c)
+PAYLOAD_BYTES, PACKET_CODED_BITS, PACKET_BITS = 27, 476, 496
+PAYLOAD_DTYPE = np.dtype([("data", "u1", (PAYLOAD_BYTES,)), ("crc_ok", "u1"), ("flipped", "<u2"), ("reserved", "<u2")])
+assert PAYLOAD_DTYPE.itemsize == 32
 
 
 def keystream_word(call_index: int) -> int:
@@ -262,6 +266,31 @@ class ModemBank:
                                           results.data_ptr(), self.n_streams, results.stride(0) // 32, n_frames,
                                           tx_bits.data_ptr(), tx_bits.shape[1], _ptr(lead_in), gap, _ptr(group),
                                           n_groups, counters.data_ptr(), stream))
+
+    def packet_encode(self, payload, bits, stream: int = 0) -> None:
+        """Encode payloads (CUDA uint8 [..., 27]) into packet bits (CUDA uint8 [..., 8, 62], e.g. [n, n_packets, 8, 62]),
+        the bits tx_packets_dev takes (sc_packet_encode_dev)."""
+        n = payload.numel() // PAYLOAD_BYTES
+        assert payload.is_contiguous() and bits.is_contiguous() and bits.numel() == n * PACKET_BITS
+        check(lib.sc_packet_encode_dev(self.device, payload.data_ptr(), n, bits.data_ptr(), stream))
+
+    def packet_llr(self, packet_symbols, n_found, llr, stream: int = 0) -> None:
+        """LLRs (L > 0: bit 0) of the 496 bits of every record rx_packets_soft_dev left (sc_packet_llr_dev):
+        packet_symbols as filled (496 floats per record, its size sets the capacity), n_found = CUDA int64[1] (read on
+        the device), llr a CUDA float32 tensor of the same number of floats."""
+        capacity = packet_symbols.numel() * packet_symbols.element_size() // (PACKET_BITS * 4)
+        assert llr.numel() * llr.element_size() >= capacity * PACKET_BITS * 4, "capacity"
+        check(lib.sc_packet_llr_dev(self.device, packet_symbols.data_ptr(), capacity, n_found.data_ptr(),
+                                    llr.data_ptr(), stream))
+
+    def packet_decode(self, llr, n_found, out, stream: int = 0) -> None:
+        """Viterbi-decode the records' LLRs (CUDA float32, 496 per record, its size sets the capacity) into out (CUDA
+        uint8 [capacity * 32], viewable as PAYLOAD_DTYPE) for the first min(n_found, capacity) records
+        (sc_packet_decode_dev)."""
+        capacity = llr.numel() * llr.element_size() // (PACKET_BITS * 4)
+        assert out.numel() * out.element_size() >= capacity * PAYLOAD_DTYPE.itemsize, "capacity"
+        check(lib.sc_packet_decode_dev(self.device, llr.data_ptr(), capacity, n_found.data_ptr(), out.data_ptr(),
+                                       stream))
 
     def transfer_bytes(self):
         out = (C.c_uint64 * 2)()
