@@ -77,7 +77,7 @@ acq_detect_kernel(PacketSrc src, int n_streams, int j_lo, int j_hi, int cap, int
         const int s = (int) (e / nj), j = j_lo + (int) (e - (long) s * nj);
         if (src.call0 + (uint32_t) j < 2u) continue;                 // call n decides frame n-2
         __syncthreads();
-        for (int i = tid; i < ACQ_NMIX + ACQ_PHASE; i += ACQ_THREADS) mix[i] = acq_mix(src, s, j, ACQ_Q0 + i);
+        for (int i = tid; i < ACQ_NMIX + ACQ_PHASE; i += ACQ_THREADS) mix[i] = packet_mix(src, s, j, ACQ_Q0 + i);
 #pragma unroll 1
         for (int ph = 0; ph <= ACQ_PHASE; ph += ACQ_PHASE) {          // the grids 5 k and 5 k + 2
             __syncthreads();

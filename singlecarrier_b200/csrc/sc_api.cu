@@ -120,11 +120,13 @@ struct sc_modem {
     DevBuf<float2> win;                     // tracker windows, tiles of 32 streams x WIN_ROWS
     DevBuf<int> max_index;
     DevBuf<float> max_value;
-    DevBuf<int16_t> hist;                   // last frame of the previous batch, [n][1880]
+    // frames before the batch that the receiver reads: call-1 (the front-end), call-2 (packet mode), call-3 (ACQ)
+    int hist_depth = 1;                     // H
+    DevBuf<int16_t> hist;                   // frames call-H .. call-1, [H][n][1880]
 
     // shared tables
     DevBuf<float2> rx_phase;                // fbb_rx_phase (device scalar)
-    DevBuf<float2> mix_table;               // slot 0 = frame of call-1, slots 1.. = this batch
+    DevBuf<float2> mix_table;               // phasors of frames call-H .., this batch's from table_slot(m, 1)
     DevBuf<float2> unit_phase;              // constant 1+0i: the cold phasor of a transmission (qpsk.c:375)
     float *state_dbg = nullptr;             // drop-in shim: full tracker state after the last call, [n][48] (not owned)
     std::vector<uint64_t> kw;               // keystream words of the batch being queued
@@ -144,15 +146,10 @@ struct sc_modem {
     DevBuf<float> stage_eq[N_PIPE];
     DevBuf<float> stage_sym[N_PIPE];
 
-    // packet mode (SC_FLAG_PACKET, extension): the frame before the saved one, its phasor table, the rx_timing
-    // snapshots and per-pipe scratch for the packet pass
+    // packet mode (SC_FLAG_PACKET, extension): the rx_timing snapshots and per-pipe scratch for the packet pass
     bool packet = false;
     bool packet_dd = false;                 // SC_FLAG_PACKET_DD: packets decoded by the decision-directed equalizer
     bool packet_acq = false;                // SC_FLAG_PACKET_ACQ: packets found by acquisition on the samples
-    DevBuf<int16_t> pk_hist2;               // frame call-2, [n][1880]
-    DevBuf<float2> pk_mix_hist2;            // phasor table of frame call-2
-    DevBuf<int16_t> pk_hist3;               // SC_FLAG_PACKET_ACQ: frame call-3, [n][1880]
-    DevBuf<float2> pk_mix_hist3;            // and its phasor table
     DevBuf<int4> acq_info[N_PIPE];          // SC_FLAG_PACKET_ACQ: per-pipe grid start, rho and nu0 of the listed packets
     DevBuf<int> pk_t_before[N_PIPE], pk_t_at[N_PIPE];         // [slab] rx_timing at entry of calls call0-1 / call0
     DevBuf<int2> pk_list[N_PIPE];
@@ -291,6 +288,7 @@ extern "C" int sc_create(sc_modem **out, int device, int64_t n_streams, uint32_t
     m->packet = (flags & SC_FLAG_PACKET) != 0;
     m->packet_dd = (flags & SC_FLAG_PACKET_DD) != 0;
     m->packet_acq = (flags & SC_FLAG_PACKET_ACQ) != 0;
+    m->hist_depth = 1 + m->packet + m->packet_acq;
     {
         uint16_t r = 0x4A80;                                             // scramble_init per packet
         for (int f = 0; f < 8; f++) m->pk_key.k[f] = keystream_next_word(r);
@@ -314,22 +312,11 @@ extern "C" int sc_create(sc_modem **out, int device, int64_t n_streams, uint32_t
         CU(m->win.reserve((size_t) (np / 32) * WIN_ROWS * 32));
         CU(m->max_index.reserve(np));
         CU(m->max_value.reserve(np));
-        CU(m->hist.reserve((size_t) m->n * FRAME));
-        CU(cudaMemset(m->hist, 0, (size_t) m->n * FRAME * sizeof(int16_t)));
+        const size_t hist_len = (size_t) m->hist_depth * m->n * FRAME;
+        CU(m->hist.reserve(hist_len));
+        CU(cudaMemset(m->hist, 0, hist_len * sizeof(int16_t)));
         CU(m->rx_phase.reserve(1));
-        if (m->packet) {
-            CU(m->pk_hist2.reserve((size_t) m->n * FRAME));
-            CU(cudaMemset(m->pk_hist2, 0, (size_t) m->n * FRAME * sizeof(int16_t)));
-            CU(m->pk_mix_hist2.reserve(FRAME));
-            CU(cudaMemset(m->pk_mix_hist2, 0, (size_t) FRAME * sizeof(float2)));
-            CU(m->pk_n_host_dev.reserve(1));
-        }
-        if (m->packet_acq) {
-            CU(m->pk_hist3.reserve((size_t) m->n * FRAME));
-            CU(cudaMemset(m->pk_hist3, 0, (size_t) m->n * FRAME * sizeof(int16_t)));
-            CU(m->pk_mix_hist3.reserve(FRAME));
-            CU(cudaMemset(m->pk_mix_hist3, 0, (size_t) FRAME * sizeof(float2)));
-        }
+        if (m->packet) CU(m->pk_n_host_dev.reserve(1));
         CU(m->unit_phase.reserve(1));
         {
             const float2 one = make_float2(1.0f, 0.0f);
@@ -416,17 +403,24 @@ struct OvTrace {
 };
 static OvTrace g_trace;
 
-// Make sure the mix table can hold slot 0 + n_frames frames and generate this batch's phasors
+// The phasor table of batch slot `slot`: slot 0 is frame call-1, slots 1.. this batch's frames; the history's older
+// frames precede slot 0, so the table of frame call-1-k is table_slot(m, -k) for k < H.
+static float2 *table_slot(const sc_modem *m, int slot) {
+    return m->mix_table + (size_t) (m->hist_depth - 1 + slot) * FRAME;
+}
+
+// Make sure the mix table can hold the H history slots + n_frames frames and generate this batch's phasors
 // (calls call .. call+n_frames-1 into slots 1..n_frames) on stream st.
 static int prepare_tables(sc_modem *m, int n_frames, cudaStream_t st) {
-    if (m->mix_table.cap < (size_t) (n_frames + 1) * FRAME) {          // a larger table, keeping slot 0
+    const size_t hist_bytes = (size_t) m->hist_depth * FRAME * sizeof(float2);
+    if (m->mix_table.cap < (size_t) (m->hist_depth + n_frames) * FRAME) {     // a larger table, keeping the history
         DevBuf<float2> nt;
-        CU(nt.reserve((size_t) (n_frames + 1) * FRAME));
+        CU(nt.reserve((size_t) (m->hist_depth + n_frames) * FRAME));
         if (m->mix_table) {
-            CU(cudaMemcpyAsync(nt, m->mix_table, (size_t) FRAME * sizeof(float2), cudaMemcpyDeviceToDevice, st));
+            CU(cudaMemcpyAsync(nt, m->mix_table, hist_bytes, cudaMemcpyDeviceToDevice, st));
             CU(cudaStreamSynchronize(st));
         } else {
-            CU(cudaMemsetAsync(nt, 0, (size_t) FRAME * sizeof(float2), st));
+            CU(cudaMemsetAsync(nt, 0, hist_bytes, st));
         }
         m->mix_table = std::move(nt);                                   // the old table goes with nt
     }
@@ -435,7 +429,7 @@ static int prepare_tables(sc_modem *m, int n_frames, cudaStream_t st) {
     // that holds its frame: one thread generates a frame in ~12 us, a small bank consumes one in ~40 us, and a single
     // tail kernel (~0.5 ms for 42 frames) would stall the chain right after the head.
     const int head = std::min(n_frames, TAB_HEAD);
-    CU(launch_nco_table(m->rx_phase, m->rx_rect, NCO_RX, 0, head, 1.0f / 16384.0f, m->mix_table + FRAME, st));
+    CU(launch_nco_table(m->rx_phase, m->rx_rect, NCO_RX, 0, head, 1.0f / 16384.0f, table_slot(m, 1), st));
     CU(cudaEventRecord(m->ev_tab1, st));
     g_trace.mark("tabhead", (uint32_t) head, 0, st);
     CU(cudaStreamWaitEvent(m->tab_stream, m->ev_tab1, 0));
@@ -443,7 +437,7 @@ static int prepare_tables(sc_modem *m, int n_frames, cudaStream_t st) {
         if ((int) m->ev_tabc.size() <= c) m->ev_tabc.emplace_back();
         CU(m->ev_tabc[c].create());
         CU(launch_nco_table(m->rx_phase, m->rx_rect, NCO_RX, 0, std::min(TAB_CHUNK, n_frames - f), 1.0f / 16384.0f,
-                            m->mix_table + (size_t) (f + 1) * FRAME, m->tab_stream));
+                            table_slot(m, f + 1), m->tab_stream));
         CU(cudaEventRecord(m->ev_tabc[c], m->tab_stream));
         g_trace.mark("table", (uint32_t) (f + TAB_CHUNK), 9, m->tab_stream);
     }
@@ -542,34 +536,30 @@ struct Slab {
     const PacketSink *pk;
 };
 
+// slot k of stream s0's sample history: frame c-H+k, c the first call of the block that reads it
+static int16_t *hist_slot(const sc_modem *m, int k, int64_t s0) {
+    return m->hist + ((size_t) k * m->n + s0) * FRAME;
+}
+
 // the frame fe(n) filters, for call n = call0 + j: frame j-1 of the block, or the last one of the previous block
 static const int16_t *fe_frame(const sc_modem *m, const Slab &s, int j, int64_t &fstride) {
     fstride = j >= 1 ? s.stride : FRAME;
-    return j >= 1 ? s.in + (size_t) (j - 1) * FRAME : m->hist + (size_t) s.s0 * FRAME;
+    return j >= 1 ? s.in + (size_t) (j - 1) * FRAME : hist_slot(m, m->hist_depth - 1, s.s0);
 }
 
-// The block's last frame becomes the history of the next block; in packet mode the one before it too (from this block
-// if it has two, else the frame the previous block saved), and on ACQ banks the one before that (saved first: it may
-// come from the older history).
+// The block's last H frames become the history of the next block: slot k takes block frame nf-H+k, or, when the block
+// is shorter than that, the frame the previous block saved in slot nf+k (above k, so read before it is overwritten).
 static int store_history(sc_modem *m, const Slab &s) {
-    const size_t pitch = FRAME * sizeof(int16_t), spitch = (size_t) s.stride * sizeof(int16_t);
-    int16_t *hist = m->hist + (size_t) s.s0 * FRAME;
-    if (m->packet_acq) {
-        int16_t *h3 = m->pk_hist3 + (size_t) s.s0 * FRAME;
-        if (s.n_frames >= 3)
-            CU(cudaMemcpy2DAsync(h3, pitch, s.in + (size_t) (s.n_frames - 3) * FRAME, spitch, pitch, (size_t) s.ns,
-                                 cudaMemcpyDeviceToDevice, s.st));
+    const size_t pitch = FRAME * sizeof(int16_t);
+    for (int k = 0; k < m->hist_depth; k++) {
+        const int f = s.n_frames - m->hist_depth + k;
+        if (f >= 0)
+            CU(cudaMemcpy2DAsync(hist_slot(m, k, s.s0), pitch, s.in + (size_t) f * FRAME, (size_t) s.stride * sizeof(int16_t),
+                                 pitch, (size_t) s.ns, cudaMemcpyDeviceToDevice, s.st));
         else
-            CU(cudaMemcpyAsync(h3, (s.n_frames == 2 ? m->hist : m->pk_hist2) + (size_t) s.s0 * FRAME, (size_t) s.ns * pitch,
+            CU(cudaMemcpyAsync(hist_slot(m, k, s.s0), hist_slot(m, s.n_frames + k, s.s0), (size_t) s.ns * pitch,
                                cudaMemcpyDeviceToDevice, s.st));
     }
-    if (m->packet && s.n_frames >= 2)
-        CU(cudaMemcpy2DAsync(m->pk_hist2 + (size_t) s.s0 * FRAME, pitch, s.in + (size_t) (s.n_frames - 2) * FRAME, spitch,
-                             pitch, (size_t) s.ns, cudaMemcpyDeviceToDevice, s.st));
-    else if (m->packet)
-        CU(cudaMemcpyAsync(m->pk_hist2 + (size_t) s.s0 * FRAME, hist, (size_t) s.ns * pitch, cudaMemcpyDeviceToDevice, s.st));
-    CU(cudaMemcpy2DAsync(hist, pitch, s.in + (size_t) (s.n_frames - 1) * FRAME, spitch, pitch, (size_t) s.ns,
-                         cudaMemcpyDeviceToDevice, s.st));
     return SC_OK;
 }
 
@@ -595,7 +585,7 @@ static int run_slab_overlapped(sc_modem *m, const Slab &s, bool coop) {
     const int64_t s0 = s.s0;
     const uint32_t call0 = m->call + (uint32_t) slot0;
     const uint64_t *kw = m->kw.data() + slot0;
-    const float2 *mix0 = m->mix_table + (size_t) slot0 * FRAME;
+    const float2 *mix0 = table_slot(m, slot0);
     cudaStream_t C[2];
     const Stream *Dn = m->ov_data[pipe];
     C[call0 & 1] = st;
@@ -712,8 +702,7 @@ static int run_slab_overlapped(sc_modem *m, const Slab &s, bool coop) {
     return SC_OK;
 }
 
-// The call loop of one slab; afterwards the block's last frame (and in packet mode the one before it) is saved for the
-// block that follows.
+// The call loop of one slab; afterwards the block's last frames are saved for the block that follows.
 static int run_slab(sc_modem *m, const Slab &s) {
     const cudaStream_t st = s.st;
     const int pipe = s.pipe, ns = s.ns, n_frames = s.n_frames, slot0 = s.slot0;
@@ -722,7 +711,7 @@ static int run_slab(sc_modem *m, const Slab &s) {
     float *eq_dbg = s.eq_dbg;
     const uint32_t call0 = m->call + (uint32_t) slot0;
     const uint64_t *kw = m->kw.data() + slot0;
-    const float2 *mix0 = m->mix_table + (size_t) slot0 * FRAME;
+    const float2 *mix0 = table_slot(m, slot0);
     float2 *win = m->win + (size_t) (s0 / 32) * WIN_ROWS * 32;
     int tab_waited = -1;
     PacketSrc psrc;
@@ -736,12 +725,9 @@ static int run_slab(sc_modem *m, const Slab &s) {
         psrc.result_stride = s.result_stride;
         psrc.in = s.in;
         psrc.stride = s.stride;
-        psrc.hist1 = m->hist + (size_t) s0 * FRAME;
-        psrc.hist2 = m->pk_hist2 + (size_t) s0 * FRAME;
-        psrc.hist3 = m->packet_acq ? m->pk_hist3 + (size_t) s0 * FRAME : nullptr;
+        psrc.hist = hist_slot(m, m->hist_depth - 1, s0);
+        psrc.hist_pitch = m->n * FRAME;
         psrc.mix0 = mix0;
-        psrc.mix_hist2 = slot0 >= 1 ? mix0 - FRAME : m->pk_mix_hist2;
-        psrc.mix_hist3 = slot0 >= 2 ? mix0 - 2 * FRAME : slot0 == 1 ? m->pk_mix_hist2 : m->pk_mix_hist3;
         psrc.timing_before_call0 = m->pk_t_before[pipe];
         psrc.timing_at_call0 = m->pk_t_at[pipe];
         psrc.call0 = call0;
@@ -845,17 +831,12 @@ static int start_tables(sc_modem *m, int n_frames) {
     return SC_OK;
 }
 
-// the last frame's phasors become slot 0 of the next batch, and in packet mode the one before it the table of frame call-2
-// (on ACQ banks the one before that the table of frame call-3, taken first: it may be the older call-2 table)
+// The tables of the batch's last H frames become the next batch's history: history slot k (frame call-H+k) takes the
+// table n_frames slots above it, from this batch or, when the batch is shorter than H-k, from a higher history slot.
 static int rotate_tables(sc_modem *m, int n_frames, cudaStream_t st) {
-    if (m->packet_acq)
-        CU(cudaMemcpyAsync(m->pk_mix_hist3, n_frames >= 2 ? m->mix_table + (size_t) (n_frames - 2) * FRAME : m->pk_mix_hist2,
+    for (int k = 0; k < m->hist_depth; k++)
+        CU(cudaMemcpyAsync(m->mix_table + (size_t) k * FRAME, m->mix_table + (size_t) (n_frames + k) * FRAME,
                            FRAME * sizeof(float2), cudaMemcpyDeviceToDevice, st));
-    if (m->packet)
-        CU(cudaMemcpyAsync(m->pk_mix_hist2, m->mix_table + (size_t) (n_frames - 1) * FRAME, FRAME * sizeof(float2),
-                           cudaMemcpyDeviceToDevice, st));
-    CU(cudaMemcpyAsync(m->mix_table, m->mix_table + (size_t) n_frames * FRAME, FRAME * sizeof(float2),
-                       cudaMemcpyDeviceToDevice, st));
     return SC_OK;
 }
 

@@ -116,11 +116,9 @@ struct PacketSrc {              // one block of calls [call0, call0 + nf) of a s
     long result_stride;
     const int16_t *in;          // block frames, stream s at in + s * stride
     long stride;
-    const int16_t *hist1, *hist2;       // frames call0-1 and call0-2, [stream][1880]
-    const int16_t *hist3;       // frame call0-3 (SC_FLAG_PACKET_ACQ banks, else nullptr)
-    const float2 *mix0;         // phasor table of frame call0-1; frames call0.. follow
-    const float2 *mix_hist2;    // phasor table of frame call0-2
-    const float2 *mix_hist3;    // phasor table of frame call0-3 (SC_FLAG_PACKET_ACQ banks)
+    const int16_t *hist;        // frame call0-1, [stream][1880]; frame call0-1-k lies k * hist_pitch before it, k < H
+    long hist_pitch;
+    const float2 *mix0;         // phasor table of frame call0-1; that of block frame f >= -H at mix0 + (f + 1) * 1880
     const int *timing_before_call0, *timing_at_call0;   // rx_timing at entry of calls call0-1 and call0
     uint32_t call0;
     int stream0;                // bank index of the slab's first stream

@@ -58,38 +58,21 @@ packet_fir_kernel(PacketSrc src, const int2 *__restrict__ list, const int *__res
     for (int e = blockIdx.x * PK_FIR_WARPS + warp; e < n_list; e += gridDim.x * PK_FIR_WARPS) {
         const int2 ent = list[e];
         const int s = ent.x, j = ent.y;
+        int q0;                                                       // first raw sample, relative to frame n-2
         if constexpr (ACQ) {
-            const int q0 = info[e].x - (NTAPS - 1);
-            __syncwarp();
-            for (int i = lane; i < PK_NSAMP; i += 32) mix[i] = acq_mix(src, s, j, q0 + i);
+            q0 = info[e].x - (NTAPS - 1);
         } else {
-        const sc_frame_result *rec = src.results + (long) s * src.result_stride;
-        const int mi = rec[j].max_index;
-        int T;
-        if (j >= 2) T = rec[j - 2].rx_timing;                         // rx_timing after call n-2 = at entry of call n-1
-        else T = (j == 1 ? src.timing_at_call0 : src.timing_before_call0)[s];
-        T = min(max(T, NTAPS - 1), 2 * PRE - 1);
-        const int q0 = CYC * mi + T - (NTAPS - 1);                    // first raw sample, relative to frame n-2
-        // frames n-2 and n-1: block frames j-2, j-1; -1 / -2 are the two frames kept from the previous block
-        const int16_t *fr[2];
-        const float2 *tb[2];
-#pragma unroll
-        for (int k = 0; k < 2; k++) {
-            const int fj = j - 2 + k;
-            if (fj >= 0) fr[k] = src.in + (long) s * src.stride + (long) fj * FRAME;
-            else fr[k] = (fj == -1 ? src.hist1 : src.hist2) + (long) s * FRAME;
-            tb[k] = fj >= -1 ? src.mix0 + (long) (fj + 1) * FRAME : src.mix_hist2;
+            const sc_frame_result *rec = src.results + (long) s * src.result_stride;
+            const int mi = rec[j].max_index;
+            int T;
+            if (j >= 2) T = rec[j - 2].rx_timing;                     // rx_timing after call n-2 = at entry of call n-1
+            else T = (j == 1 ? src.timing_at_call0 : src.timing_before_call0)[s];
+            T = min(max(T, NTAPS - 1), 2 * PRE - 1);
+            q0 = CYC * mi + T - (NTAPS - 1);                          // 0 .. 842: samples of frames n-2 and n-1 only
         }
         __syncwarp();
-        for (int i = lane; i < PK_NSAMP; i += 32) {                   // mixer, qpsk.c:138-145 (table = phasor / 16384)
-            const int q = q0 + i;
-            const int k = q >= FRAME ? 1 : 0;
-            const int qq = q - k * FRAME;
-            const float v = (float) fr[k][qq];
-            const float2 ph = __ldg(tb[k] + qq);
-            mix[i] = make_float2(__fmul_rn(ph.x, v), __fmul_rn(ph.y, v));
-        }
-        }
+        // mixer, qpsk.c:138-145 (table = phasor / 16384)
+        for (int i = lane; i < PK_NSAMP; i += 32) mix[i] = packet_mix(src, s, j, q0 + i);
         __syncwarp();
         float2 *out = sym + ((long) (e >> 5) * PK_SYMS) * 32 + (e & 31);
         for (int o = lane; o < PK_SYMS; o += 32) {                    // src/fir.c:36-42 at sample 5 o + 48 of the window
