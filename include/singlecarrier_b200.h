@@ -499,6 +499,54 @@ int sc_packet_llr_dev(int device, const float *packet_symbols, int64_t capacity,
 int sc_packet_decode_dev(int device, const float *llr, int64_t capacity, const uint64_t *n_found,
                          sc_packet_payload *out, void *stream);
 
+/* ---- code rates of the coded payload (DESIGN.md section 8c, "Code rates") ----------------------------------------
+ *
+ * The same mother code, punctured per stream to rate 2/3 or 3/4 with the IEEE 802.11a patterns; the packet layout,
+ * the interleaver and the LLRs (sc_packet_llr_dev) do not change.  Each stream has one code, set at both ends of its
+ * link (a device uint8 table stream_code[n_streams], the same for the encoder and the decoder):
+ *   code  payload B  steps T = 8 B + 22  mother bits kept per period  transmitted bits N  free distance
+ *   0     27         238                 c0 c1                        476                 10  (today's code)
+ *   1     36         310                 c0 c1 | c0                   465                 6
+ *   2     41         350                 c0 c1 | c0 | c1              467                 5
+ *   info      u = B payload bytes, their CRC-16 (as above, high byte first), MSB first: 8 B + 16 bits; then 6 zeros
+ *   encoder   the rate-1/2 encoder above over t = 0..T-1 -> mother bits c[2t] (0133), c[2t+1] (0171)
+ *   puncture  transmitted bit n < N is mother bit m(n): code 0: m = n; code 1: m = 4 floor(n/3) + (0, 1, 2)[n mod 3];
+ *             code 2: m = 6 floor(n/4) + (0, 1, 2, 5)[n mod 4]
+ *   layout    transmitted bit n goes to packet bit p = 17 (n mod 28) + floor(n / 28); every other p of the 496 is 0
+ *   decoder   L'[m(n)] = the sanitised LLR at p(n) for n < N, L'[m] = 0 for every punctured m; then the recursion of
+ *             sc_packet_decode_dev over T steps and the traceback from state 0
+ * For code 0 this is exactly the code of sc_packet_encode_dev / sc_packet_decode_dev. */
+#define SC_PACKET_CODE_R12 0
+#define SC_PACKET_CODE_R23 1
+#define SC_PACKET_CODE_R34 2
+#define SC_PACKET_PAYLOAD_MAX 41
+int sc_packet_payload_bytes(int code);          /* 27, 36, 41; 0 for any other value (host function) */
+
+typedef struct {
+    uint8_t  data[41];      /* the first sc_packet_payload_bytes(code) bytes: the maximum-likelihood payload; the rest 0 */
+    uint8_t  code;          /* the code the record was decoded with, as read from stream_code (255: stream out of range) */
+    uint8_t  crc_ok;        /* 1 when the CRC of the payload equals the decoded CRC bits */
+    uint8_t  reserved0;     /* 0 */
+    uint16_t flipped;       /* of the code's N transmitted bits, those whose LLR sign disagrees with the decoded codeword */
+    uint16_t reserved1;     /* 0 */
+} sc_packet_payload_ex;     /* 48 bytes */
+
+/* payload [n_streams][n_packets][41] (bytes past the stream's B are ignored), stream_code device uint8[n_streams]
+ *   -> bits [n_streams][n_packets][8][62], the layout sc_tx_packets_dev / sc_tx_channel_dev take.  A stream whose code
+ *   is not 0..2 gets all-zero bits.  SC_EINVAL before any CUDA call on a NULL pointer, n_streams < 0 or
+ *   n_packets < 1; n_streams == 0 launches nothing. */
+int sc_packet_encode_ex_dev(int device, const uint8_t *payload, int64_t n_streams, int n_packets,
+                            const uint8_t *stream_code, uint8_t *bits, void *stream);
+
+/* Record k < min(*n_found, capacity) (n_found read on the device, as for sc_packet_decode_dev): its code is
+ *   stream_code[packets[k].stream]; the 496 LLRs at llr + 496 k (sc_packet_llr_dev's output) -> out[k].  A stream
+ *   outside 0..n_streams-1, or a code that is not 0..2: data 0, crc_ok 0, flipped 0, code as read (255 for the
+ *   stream).  Records at or past that count are not touched.  SC_EINVAL before any CUDA call on a NULL pointer, a
+ *   negative capacity or n_streams, llr not aligned to 8 bytes or out not to 4; capacity == 0 launches nothing. */
+int sc_packet_decode_ex_dev(int device, const float *llr, const sc_packet_result *packets, int64_t capacity,
+                            const uint64_t *n_found, const uint8_t *stream_code, int64_t n_streams,
+                            sc_packet_payload_ex *out, void *stream);
+
 /* ---- multi-GPU reduction of the counters (SURVEY section 8e: the path's only collective) ------------------ */
 
 /* ncclAllReduce(sum) of n_counters uint64 in place on `stream`; nccl_comm is a ncclComm_t created by the

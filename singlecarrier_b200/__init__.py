@@ -7,12 +7,14 @@ fir / equalizer / kalman / scramble primitives underneath), processing thousands
 and ``bench.py``.  PyTorch is used only for device memory, streams and ``torch.distributed``.
 """
 from ._lib import LIB_PATH, SingleCarrierError, lib  # noqa: F401
-from .modem import (BITS_PER_CALL, DATA_SYMBOLS, FRAME_SIZE, PACKET_DATA_SYMBOLS, PACKET_DTYPE, PAYLOAD_DTYPE,  # noqa: F401
-                    RESULT_DTYPE,
+from .modem import (BITS_PER_CALL, CODE_R12, CODE_R23, CODE_R34, DATA_SYMBOLS, FRAME_SIZE,  # noqa: F401
+                    PACKET_DATA_SYMBOLS, PACKET_DTYPE, PAYLOAD_DTYPE, PAYLOAD_EX_DTYPE, PAYLOAD_MAX, RESULT_DTYPE,
+                    payload_bytes,
                     SYMBOLS_PER_FRAME, ModemBank, NcclComm, PinnedBuffer, h2d_probe, keystream_word, launch_count,
                     packet_keystream_word, packet_soft_bits, soft_bits, unpack_bits, unpack_packet_bits)
 
 __all__ = ["ModemBank", "NcclComm", "PinnedBuffer", "h2d_probe", "RESULT_DTYPE", "PACKET_DTYPE", "PAYLOAD_DTYPE",
            "unpack_packet_bits", "FRAME_SIZE", "BITS_PER_CALL",
            "SYMBOLS_PER_FRAME", "DATA_SYMBOLS", "PACKET_DATA_SYMBOLS", "unpack_bits", "soft_bits", "packet_soft_bits",
-           "keystream_word", "packet_keystream_word", "launch_count", "SingleCarrierError", "lib", "LIB_PATH"]
+           "keystream_word", "packet_keystream_word", "launch_count", "SingleCarrierError", "lib", "LIB_PATH",
+           "PAYLOAD_EX_DTYPE", "PAYLOAD_MAX", "CODE_R12", "CODE_R23", "CODE_R34", "payload_bytes"]

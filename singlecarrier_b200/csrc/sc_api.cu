@@ -1648,6 +1648,36 @@ extern "C" int sc_packet_decode_dev(int device, const float *llr, int64_t capaci
     return SC_OK;
 }
 
+extern "C" int sc_packet_payload_bytes(int code) {
+    return code == SC_PACKET_CODE_R12 ? 27 : code == SC_PACKET_CODE_R23 ? 36 : code == SC_PACKET_CODE_R34 ? 41 : 0;
+}
+
+extern "C" int sc_packet_encode_ex_dev(int device, const uint8_t *payload, int64_t n_streams, int n_packets,
+                                       const uint8_t *stream_code, uint8_t *bits, void *stream) {
+    if (!payload || !stream_code || !bits || n_streams < 0 || n_packets < 1)
+        return fail(SC_EINVAL, "sc_packet_encode_ex_dev: bad arguments");
+    int rc = stage_device(device);
+    if (rc != SC_OK) return rc;
+    if (n_streams == 0) return SC_OK;
+    CU(launch_packet_encode_ex(payload, n_streams, n_packets, stream_code, bits, (cudaStream_t) stream));
+    return SC_OK;
+}
+
+extern "C" int sc_packet_decode_ex_dev(int device, const float *llr, const sc_packet_result *packets, int64_t capacity,
+                                       const uint64_t *n_found, const uint8_t *stream_code, int64_t n_streams,
+                                       sc_packet_payload_ex *out, void *stream) {
+    if (!llr || !packets || !n_found || !stream_code || !out || capacity < 0 || n_streams < 0)
+        return fail(SC_EINVAL, "sc_packet_decode_ex_dev: bad arguments");
+    if (((uintptr_t) llr & 7) != 0 || ((uintptr_t) out & 3) != 0)
+        return fail(SC_EINVAL, "sc_packet_decode_ex_dev: llr must be 8-byte and out 4-byte aligned");
+    int rc = stage_device(device);
+    if (rc != SC_OK) return rc;
+    if (capacity == 0) return SC_OK;
+    CU(launch_packet_decode_ex(llr, packets, capacity, (const unsigned long long *) n_found, stream_code, n_streams, out,
+                               (cudaStream_t) stream));
+    return SC_OK;
+}
+
 // ---- checkpoint / resume ------------------------------------------------------------------------
 namespace {
 struct StateHeader {

@@ -147,6 +147,11 @@ cudaError_t launch_packet_llr(const float *packet_symbols, long capacity, const 
                               const PacketKey &key, cudaStream_t st);
 cudaError_t launch_packet_decode(const float *llr, long capacity, const unsigned long long *n_found,
                                  sc_packet_payload *out, cudaStream_t st);
+cudaError_t launch_packet_encode_ex(const uint8_t *payload, long n_streams, int n_packets, const uint8_t *stream_code,
+                                    uint8_t *bits, cudaStream_t st);
+cudaError_t launch_packet_decode_ex(const float *llr, const sc_packet_result *packets, long capacity,
+                                    const unsigned long long *n_found, const uint8_t *stream_code, long n_streams,
+                                    sc_packet_payload_ex *out, cudaStream_t st);
 
 // sc_tx_kernels.cu
 struct TxArgs {

@@ -15,7 +15,7 @@ from typing import Optional
 import numpy as np
 
 from .modem import (FRAME_SIZE, N_PACKET_BER_COUNTERS, PACKET_CODED_BITS, PACKET_DTYPE, PAYLOAD_BYTES, PAYLOAD_DTYPE,
-                    REFERENCE_GAP, ModemBank, keystream_word)
+                    PAYLOAD_EX_DTYPE, PAYLOAD_MAX, REFERENCE_GAP, ModemBank, keystream_word, payload_bytes)
 from .taps import modem_taps
 
 PERIOD = FRAME_SIZE + REFERENCE_GAP          # 2783 samples: one packet + dead air (qpsk.c:384,405,410-412)
@@ -36,6 +36,7 @@ class Workload:
     n_packets: int
     channel: Optional[dict] = None   # the per-stream channel parameter tensors that were applied
     payload: Optional["object"] = None   # CUDA uint8 [n_streams, n_packets, 27] when the packets carry coded payloads
+    stream_code: Optional["object"] = None   # CUDA uint8 [n_streams] with per-stream code rates (payload [.., 41])
 
 
 def awgn_sigma(ebn0_db, torch):
@@ -46,13 +47,15 @@ def awgn_sigma(ebn0_db, torch):
 
 
 def synthesize(bank: ModemBank, samples_per_stream: int, seed: int, *, config: int, gap: int = REFERENCE_GAP,
-               ebn0_db=None, payload=None) -> Workload:
+               ebn0_db=None, payload=None, stream_code=None) -> Workload:
     """config 2: clean channel, random df/phase, lead-in 80+5m (preamble lands on decimated index m).
     config 3: + AWGN at ebn0_db[s] (default: 13 points 0..12 dB, striped by stream index).
     config 4: bench workload (config 3 channel, random lead-in).
     config 5: + linear drift (+-2 Hz/s) and a 2-tap echo (a 0.1..0.5, delay 1..10 samples) at 10 dB.
     payload: None (random bits), or CUDA uint8 [n_streams, n_packets, 27]: the packets carry these payloads through the
-    packet code (sc_packet_encode_dev); n_packets must be the number the stream's length gives."""
+    packet code (sc_packet_encode_dev); n_packets must be the number the stream's length gives.
+    stream_code: None, or CUDA uint8 [n_streams]: each stream's code rate; payload is then [n_streams, n_packets, 41]
+    and goes through sc_packet_encode_ex_dev."""
     import torch
     dev = torch.device("cuda", bank.device)
     n = bank.n_streams
@@ -85,12 +88,18 @@ def synthesize(bank: ModemBank, samples_per_stream: int, seed: int, *, config: i
     if payload is None:
         bank.tx_packets_dev(out, n_packets, gap_samples=gap, seed=seed, bits_out=bits, lead_in=lead, channel=ch)
     else:
-        assert tuple(payload.shape) == (n, n_packets, PAYLOAD_BYTES) and payload.dtype == torch.uint8, "payload shape"
+        width = PAYLOAD_BYTES if stream_code is None else PAYLOAD_MAX
+        assert tuple(payload.shape) == (n, n_packets, width) and payload.dtype == torch.uint8, "payload shape"
         payload = payload.to(dev).contiguous()
-        bank.packet_encode(payload, bits)
+        if stream_code is None:
+            bank.packet_encode(payload, bits)
+        else:
+            stream_code = stream_code.to(dev, torch.uint8).contiguous()
+            assert stream_code.numel() == n, "stream_code shape"
+            bank.packet_encode_ex(payload, stream_code, bits)
         bank.tx_packets_dev(out, n_packets, gap_samples=gap, seed=seed, bits=bits, lead_in=lead, channel=ch)
     torch.cuda.synchronize(dev)
-    return Workload(out, bits, lead, gap, eb, n_packets, ch, payload)
+    return Workload(out, bits, lead, gap, eb, n_packets, ch, payload, stream_code)
 
 
 def demodulate(bank: ModemBank, samples, n_frames: int):
@@ -216,11 +225,16 @@ def packet_fec(packets, n_found: int, decoded, res, n_frames: int, wl: Workload,
     is not 0, else call index, max_index and rx_timing).  Returns numpy int64 arrays per group: records, aligned,
     crc_ok (aligned records whose CRC checks), correct (aligned, crc_ok and the payload transmitted), undetected
     (aligned, crc_ok and another payload), raw_errors (hard-decision errors over the coded bits 0..475 of aligned
-    records) and raw_packet_errors (aligned records with at least one)."""
+    records) and raw_packet_errors (aligned records with at least one).
+
+    A workload with per-stream codes (wl.stream_code) takes the sc_packet_payload_ex records (PAYLOAD_EX_DTYPE) of
+    sc_packet_decode_ex_dev: the payloads compare over the first payload_bytes(code) bytes, raw errors count over the
+    code's N transmitted positions only, and payload_bytes (the sum of the payload bytes of correct records) is added."""
     assert wl.payload is not None, "the workload carries no coded payload"
-    pay = _host(wl.payload).reshape(-1, wl.n_packets, PAYLOAD_BYTES)
+    coded = wl.stream_code is not None
+    pay = _host(wl.payload).reshape(-1, wl.n_packets, PAYLOAD_MAX if coded else PAYLOAD_BYTES)
     pk = _host(packets).view(PACKET_DTYPE).reshape(-1)
-    dec = _host(decoded).view(PAYLOAD_DTYPE).reshape(-1)
+    dec = _host(decoded).view(PAYLOAD_EX_DTYPE if coded else PAYLOAD_DTYPE).reshape(-1)
     kept = min(int(n_found), pk.size, dec.size)
     pk, dec = pk[:kept], dec[:kept]
     r = _host(res)
@@ -242,15 +256,34 @@ def packet_fec(packets, n_found: int, decoded, res, n_frames: int, wl: Workload,
     al = ok & (j >= 0) & (j < wl.n_packets) & (np.abs(pos - j * period) <= 10)
     j = np.clip(j, 0, wl.n_packets - 1)
     crc = dec["crc_ok"] != 0
-    same = (dec["data"] == pay[s, j]).all(axis=1)
     # hard decisions against the transmitted bits, packed like the records' words (bit k of word f = bit 62 f + k)
     txw = _packed_words(wl.tx_bits)[s, j]
-    mask = np.array([(1 << 62) - 1] * 7 + [(1 << (PACKET_CODED_BITS - 7 * 62)) - 1], np.uint64)
+    if coded:
+        n_bytes = np.array([payload_bytes(c) for c in range(256)], np.int64)[_host(wl.stream_code).astype(np.int64)[s]]
+        same = ((dec["data"] == pay[s, j]) | (np.arange(PAYLOAD_MAX) >= n_bytes[:, None])).all(axis=1)
+        mask = coded_position_masks()[np.minimum(_host(wl.stream_code).astype(np.int64)[s], 3)]
+    else:
+        same = (dec["data"] == pay[s, j]).all(axis=1)
+        mask = np.array([(1 << 62) - 1] * 7 + [(1 << (PACKET_CODED_BITS - 7 * 62)) - 1], np.uint64)
     raw = np.bitwise_count((pk["bits"] ^ txw) & mask).sum(axis=1).astype(np.int64)
-    out = {k: np.zeros(n_groups, np.int64) for k in ("records", "aligned", "crc_ok", "correct", "undetected",
-                                                      "raw_errors", "raw_packet_errors")}
-    for name, m, w in (("records", ok, None), ("aligned", al, None), ("crc_ok", al & crc, None),
-                       ("correct", al & crc & same, None), ("undetected", al & crc & ~same, None),
-                       ("raw_errors", al, raw), ("raw_packet_errors", al & (raw > 0), None)):
+    names = ("records", "aligned", "crc_ok", "correct", "undetected", "raw_errors", "raw_packet_errors")
+    out = {k: np.zeros(n_groups, np.int64) for k in names + (("payload_bytes",) if coded else ())}
+    rows = [("records", ok, None), ("aligned", al, None), ("crc_ok", al & crc, None),
+            ("correct", al & crc & same, None), ("undetected", al & crc & ~same, None),
+            ("raw_errors", al, raw), ("raw_packet_errors", al & (raw > 0), None)]
+    if coded:
+        rows.append(("payload_bytes", al & crc & same, n_bytes))
+    for name, m, w in rows:
         np.add.at(out[name], g[m], 1 if w is None else w[m])
+    return out
+
+
+def coded_position_masks() -> np.ndarray:
+    """uint64 [4, 8]: row c (code 0..2) has the packet bit positions pi(n), n < N(c), that carry transmitted bits, in
+    the records' word layout (bit k of word f = bit 62 f + k); row 3 (any other code) is empty."""
+    out = np.zeros((4, 8), np.uint64)
+    for c, n_coded in enumerate((476, 465, 467)):
+        for n in range(n_coded):
+            p = 17 * (n % 28) + n // 28
+            out[c, p // 62] |= np.uint64(1 << (p % 62))
     return out

@@ -43,6 +43,17 @@ assert PACKET_DTYPE.itemsize == 96
 PAYLOAD_BYTES, PACKET_CODED_BITS, PACKET_BITS = 27, 476, 496
 PAYLOAD_DTYPE = np.dtype([("data", "u1", (PAYLOAD_BYTES,)), ("crc_ok", "u1"), ("flipped", "<u2"), ("reserved", "<u2")])
 assert PAYLOAD_DTYPE.itemsize == 32
+# code rates (DESIGN.md section 8c, "Code rates"): one code per stream; sc_packet_payload_ex records
+CODE_R12, CODE_R23, CODE_R34 = 0, 1, 2
+PAYLOAD_MAX = 41
+PAYLOAD_EX_DTYPE = np.dtype([("data", "u1", (PAYLOAD_MAX,)), ("code", "u1"), ("crc_ok", "u1"), ("reserved0", "u1"),
+                             ("flipped", "<u2"), ("reserved1", "<u2")])
+assert PAYLOAD_EX_DTYPE.itemsize == 48
+
+
+def payload_bytes(code: int) -> int:
+    """Payload bytes of a packet at code rate ``code`` (27, 36, 41; 0 for any other value)."""
+    return int(lib.sc_packet_payload_bytes(int(code)))
 
 
 def keystream_word(call_index: int) -> int:
@@ -291,6 +302,29 @@ class ModemBank:
         assert out.numel() * out.element_size() >= capacity * PAYLOAD_DTYPE.itemsize, "capacity"
         check(lib.sc_packet_decode_dev(self.device, llr.data_ptr(), capacity, n_found.data_ptr(), out.data_ptr(),
                                        stream))
+
+    def packet_encode_ex(self, payload, stream_code, bits, stream: int = 0) -> None:
+        """Encode payloads (CUDA uint8 [n_streams, n_packets, 41]; bytes past the stream's payload_bytes are ignored)
+        at each stream's code (stream_code: CUDA uint8 [n_streams]) into packet bits (CUDA uint8
+        [n_streams, n_packets, 8, 62]) (sc_packet_encode_ex_dev).  A stream whose code is not 0..2 gets zero bits."""
+        n_streams, n_packets = payload.shape[0], payload.shape[1]
+        assert payload.is_contiguous() and bits.is_contiguous() and stream_code.is_contiguous()
+        assert payload.numel() == n_streams * n_packets * PAYLOAD_MAX and stream_code.numel() == n_streams
+        assert bits.numel() == n_streams * n_packets * PACKET_BITS
+        check(lib.sc_packet_encode_ex_dev(self.device, payload.data_ptr(), n_streams, n_packets,
+                                          stream_code.data_ptr(), bits.data_ptr(), stream))
+
+    def packet_decode_ex(self, llr, packets, n_found, stream_code, out, stream: int = 0) -> None:
+        """Viterbi-decode the records' LLRs (CUDA float32, 496 per record, its size sets the capacity) at the code of
+        each record's stream (stream_code: CUDA uint8 [n_streams], packets: the records as rx_packets_soft_dev left
+        them) into out (CUDA uint8 [capacity * 48], viewable as PAYLOAD_EX_DTYPE) for the first min(n_found, capacity)
+        records (sc_packet_decode_ex_dev)."""
+        capacity = llr.numel() * llr.element_size() // (PACKET_BITS * 4)
+        assert packets.numel() * packets.element_size() >= capacity * PACKET_DTYPE.itemsize, "capacity"
+        assert out.numel() * out.element_size() >= capacity * PAYLOAD_EX_DTYPE.itemsize, "capacity"
+        assert stream_code.is_contiguous()
+        check(lib.sc_packet_decode_ex_dev(self.device, llr.data_ptr(), packets.data_ptr(), capacity, n_found.data_ptr(),
+                                          stream_code.data_ptr(), stream_code.numel(), out.data_ptr(), stream))
 
     def transfer_bytes(self):
         out = (C.c_uint64 * 2)()
