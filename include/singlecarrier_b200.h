@@ -547,6 +547,25 @@ int sc_packet_decode_ex_dev(int device, const float *llr, const sc_packet_result
                             const uint64_t *n_found, const uint8_t *stream_code, int64_t n_streams,
                             sc_packet_payload_ex *out, void *stream);
 
+/* Per-packet codes.  sc_packet_encode_ex_dev takes one code per packet when each packet is given as a stream of its
+ * own: payload [n_streams * n_packets][1][41], n_streams * n_packets "streams" of n_packets = 1, and a code table
+ * uint8[n_streams * n_packets] (packet j of stream s at s * n_packets + j).  The bits come out in exactly the
+ * [n_streams][n_packets][8][62] layout the transmitter takes.
+ *
+ * Blind code detection (DESIGN.md section 8c, "Blind code detection"): the receiver needs no code table.  Record
+ * k < min(*n_found, capacity) (n_found read on the device, as above) is decoded at every code c of code_mask (bit c
+ * set, c = 0..2), each exactly as sc_packet_decode_ex_dev decodes it at c, and one of those records is returned
+ * unchanged in out[k] (its code field says which):
+ *   better(a, b)  flipped_a * N_b < flipped_b * N_a (N = 476, 465, 467); equal: the lower code
+ *   choose        the best of the candidates whose CRC passes; when none passes, the best of all (crc_ok 0)
+ * The CRC identifies the code (a record decoded at the wrong code passes with probability about 2^-16); flipped / N
+ * only breaks ties.  A one-code mask 1 << c gives exactly the records of sc_packet_decode_ex_dev with every stream at c.
+ * Records at or past the count are not touched.  SC_EINVAL before any CUDA call on a NULL pointer, a negative
+ * capacity, code_mask 0 or with a bit above bit 2, llr not aligned to 8 bytes or out not to 4; capacity == 0 launches
+ * nothing. */
+int sc_packet_decode_blind_dev(int device, const float *llr, int64_t capacity, const uint64_t *n_found,
+                               unsigned code_mask, sc_packet_payload_ex *out, void *stream);
+
 /* ---- multi-GPU reduction of the counters (SURVEY section 8e: the path's only collective) ------------------ */
 
 /* ncclAllReduce(sum) of n_counters uint64 in place on `stream`; nccl_comm is a ncclComm_t created by the

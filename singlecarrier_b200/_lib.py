@@ -90,6 +90,7 @@ def _load() -> C.CDLL:
     sig("sc_packet_payload_bytes", i32, i32)
     sig("sc_packet_encode_ex_dev", i32, i32, vp, i64, i32, vp, vp, vp)
     sig("sc_packet_decode_ex_dev", i32, i32, vp, vp, i64, vp, vp, i64, vp, vp)
+    sig("sc_packet_decode_blind_dev", i32, i32, vp, i64, vp, u32, vp, vp)
     sig("sc_reduce_stats", i32, vp, i32, vp, vp)
     sig("sc_comm_unique_id", i32, vp)
     sig("sc_comm_init_rank", i32, C.POINTER(vp), i32, i32, vp, i32)

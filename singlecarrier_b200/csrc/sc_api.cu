@@ -1678,6 +1678,20 @@ extern "C" int sc_packet_decode_ex_dev(int device, const float *llr, const sc_pa
     return SC_OK;
 }
 
+extern "C" int sc_packet_decode_blind_dev(int device, const float *llr, int64_t capacity, const uint64_t *n_found,
+                                          unsigned code_mask, sc_packet_payload_ex *out, void *stream) {
+    if (!llr || !n_found || !out || capacity < 0 || code_mask == 0u || (code_mask & ~7u) != 0u)
+        return fail(SC_EINVAL, "sc_packet_decode_blind_dev: bad arguments");
+    if (((uintptr_t) llr & 7) != 0 || ((uintptr_t) out & 3) != 0)
+        return fail(SC_EINVAL, "sc_packet_decode_blind_dev: llr must be 8-byte and out 4-byte aligned");
+    int rc = stage_device(device);
+    if (rc != SC_OK) return rc;
+    if (capacity == 0) return SC_OK;
+    CU(launch_packet_decode_blind(llr, capacity, (const unsigned long long *) n_found, code_mask, out,
+                                  (cudaStream_t) stream));
+    return SC_OK;
+}
+
 // ---- checkpoint / resume ------------------------------------------------------------------------
 namespace {
 struct StateHeader {

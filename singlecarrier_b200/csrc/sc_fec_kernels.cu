@@ -346,6 +346,50 @@ packet_code_encode_kernel(const uint8_t *__restrict__ payload, long n_streams, i
     }
 }
 
+// One record's 496 LLRs at src decoded at code (0..2, uniform over the warp), with the warp's buffers L (2 T floats),
+// dec (T steps) and u (the info words) -> word `lane` of its sc_packet_payload_ex record (lanes 0..11; 0 on the
+// others), and crc_ok and flipped, uniform over the warp.  The caller syncs the warp before L or u is written again.
+__device__ __forceinline__ unsigned fec_decode_code(const float2 *src, unsigned code, const FecLane &q, int lane, float *L,
+                                                    uint2 *dec, unsigned *u, const unsigned *tab, bool &crc_ok,
+                                                    unsigned &flipped) {
+    const auto words = [&](int i) { return u[i]; };
+    const int n_bytes = fec_code_bytes(code), steps = 8 * n_bytes + 22, n_coded = fec_code_coded(code);
+    for (int m = lane; m < 2 * steps; m += 32) L[m] = 0.0f;
+    __syncwarp();
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+        const int idx = lane + 32 * i;
+        if (idx < FEC_SYMS) {
+            const float2 x = __ldg(src + idx);
+            const int n0 = fec_coded_index(2 * idx), n1 = fec_coded_index(2 * idx + 1);
+            if (n0 < n_coded) L[fec_mother_index(code, n0)] = fec_sanitise(x.x);
+            if (n1 < n_coded) L[fec_mother_index(code, n1)] = fec_sanitise(x.y);
+        }
+    }
+    __syncwarp();
+    float pm0 = lane == 0 ? 0.0f : -INFINITY, pm1 = -INFINITY;
+    for (int t = 0; t < steps; t++) {
+        const uint2 d = fec_acs(q, reinterpret_cast<const float2 *>(L)[t], pm0, pm1);
+        if (lane == (t & 31)) dec[t] = d;
+    }
+    __syncwarp();
+    fec_traceback(dec, steps, u, lane);
+    __syncwarp();
+    flipped = 0u;
+    for (int n = lane; n < n_coded; n += 32) flipped += fec_flip(words, L, fec_mother_index(code, n));
+    flipped = __reduce_add_sync(0xffffffffu, flipped);
+    const unsigned crc = fec_crc_info(tab, u, n_bytes);
+    const unsigned rx_crc = (fec_info_byte(u, n_bytes) << 8) | fec_info_byte(u, n_bytes + 1);
+    crc_ok = crc == rx_crc;
+    const int keep = n_bytes - 4 * lane;                                   // payload bytes in word lane of data
+    unsigned v = 0u;
+    if (lane < FEC_WORDS_MAX && keep > 0)
+        v = fec_bytes_to_bits(u[lane]) & (keep >= 4 ? 0xffffffffu : (1u << (8 * keep)) - 1u);
+    if (lane == 10) v |= (code << 8) | ((crc_ok ? 1u : 0u) << 16);        // data[40], code, crc_ok, 0
+    if (lane == 11) v = flipped;                                           // flipped, reserved1 = 0
+    return v;
+}
+
 // one warp per record, as packet_viterbi_kernel; the record's code is read once, so every branch on it is uniform
 __global__ void __launch_bounds__(32 * FEC_WARPS, 4)
 packet_code_viterbi_kernel(const float2 *__restrict__ llr, const sc_packet_result *__restrict__ packets, long capacity,
@@ -358,50 +402,58 @@ packet_code_viterbi_kernel(const float2 *__restrict__ llr, const sc_packet_resul
     fec_crc_table(sh_crc);
     const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const FecLane q = fec_lane(lane);
-    float *L = sh_l[w];
-    const auto words = [&](int i) { return sh_u[w][i]; };
     const long n_rec = fec_records(capacity, n_found);
     for (long k = (long) blockIdx.x * FEC_WARPS + w; k < n_rec; k += (long) gridDim.x * FEC_WARPS) {
         const int s = __ldg(&packets[k].stream);
         const unsigned code = s >= 0 && s < n_streams ? __ldg(stream_code + s) : 255u;
         unsigned v = lane == 10 ? code << 8 : 0u;                         // the record not decoded: data 0, crc_ok 0
         if (code < FEC_CODES) {
-            const int n_bytes = fec_code_bytes(code), steps = 8 * n_bytes + 22, n_coded = fec_code_coded(code);
-            for (int m = lane; m < 2 * steps; m += 32) L[m] = 0.0f;
-            __syncwarp();
-            const float2 *src = llr + k * FEC_SYMS;
-#pragma unroll
-            for (int i = 0; i < 8; i++) {
-                const int idx = lane + 32 * i;
-                if (idx < FEC_SYMS) {
-                    const float2 x = __ldg(src + idx);
-                    const int n0 = fec_coded_index(2 * idx), n1 = fec_coded_index(2 * idx + 1);
-                    if (n0 < n_coded) L[fec_mother_index(code, n0)] = fec_sanitise(x.x);
-                    if (n1 < n_coded) L[fec_mother_index(code, n1)] = fec_sanitise(x.y);
-                }
-            }
-            __syncwarp();
-            float pm0 = lane == 0 ? 0.0f : -INFINITY, pm1 = -INFINITY;
-            for (int t = 0; t < steps; t++) {
-                const uint2 d = fec_acs(q, reinterpret_cast<const float2 *>(L)[t], pm0, pm1);
-                if (lane == (t & 31)) sh_dec[w][t] = d;
-            }
-            __syncwarp();
-            fec_traceback(sh_dec[w], steps, sh_u[w], lane);
-            __syncwarp();
-            unsigned flipped = 0u;
-            for (int n = lane; n < n_coded; n += 32) flipped += fec_flip(words, L, fec_mother_index(code, n));
-            flipped = __reduce_add_sync(0xffffffffu, flipped);
-            const unsigned crc = fec_crc_info(sh_crc, sh_u[w], n_bytes);
-            const unsigned rx_crc = (fec_info_byte(sh_u[w], n_bytes) << 8) | fec_info_byte(sh_u[w], n_bytes + 1);
-            const int keep = n_bytes - 4 * lane;                           // payload bytes in word lane of data
-            if (lane < FEC_WORDS_MAX && keep > 0)
-                v = fec_bytes_to_bits(sh_u[w][lane]) & (keep >= 4 ? 0xffffffffu : (1u << (8 * keep)) - 1u);
-            if (lane == 10) v |= (code << 8) | ((crc == rx_crc ? 1u : 0u) << 16);   // data[40], code, crc_ok, 0
-            if (lane == 11) v = flipped;                                   // flipped, reserved1 = 0
+            bool crc_ok;
+            unsigned flipped;
+            v = fec_decode_code(llr + k * FEC_SYMS, code, q, lane, sh_l[w], sh_dec[w], sh_u[w], sh_crc, crc_ok, flipped);
         }
         if (lane < 12) reinterpret_cast<unsigned *>(out + k)[lane] = v;
         __syncwarp();                                                      // L and sh_u are reused by the next record
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Blind code detection (DESIGN.md section 8c, "Blind code detection"): each record decoded at every code of the mask,
+// in code order, through the same buffers.  A candidate replaces the kept one when it passes its CRC and the kept one
+// does not, or when both agree on the CRC and its flipped / N is smaller (flipped_a N_b < flipped_b N_a, integers; a
+// tie keeps the lower code).  Lanes 0..11 keep the kept record's words in a register; the record is written once.
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(32 * FEC_WARPS, 4)
+packet_blind_decode_kernel(const float2 *__restrict__ llr, long capacity, const unsigned long long *__restrict__ n_found,
+                           unsigned code_mask, sc_packet_payload_ex *__restrict__ out) {
+    __shared__ __align__(8) float sh_l[FEC_WARPS][2 * FEC_STEPS_MAX];
+    __shared__ uint2 sh_dec[FEC_WARPS][FEC_STEPS_MAX];
+    __shared__ unsigned sh_u[FEC_WARPS][FEC_WORDS_MAX];
+    __shared__ unsigned sh_crc[256];
+    fec_crc_table(sh_crc);
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const FecLane q = fec_lane(lane);
+    const long n_rec = fec_records(capacity, n_found);
+    for (long k = (long) blockIdx.x * FEC_WARPS + w; k < n_rec; k += (long) gridDim.x * FEC_WARPS) {
+        unsigned best_v = 0u, best_flipped = 0u, best_n = 0u;             // best_n 0: no candidate kept yet
+        bool best_ok = false;
+#pragma unroll 1
+        for (unsigned code = 0; code < FEC_CODES; code++) {
+            if (!((code_mask >> code) & 1u)) continue;
+            bool crc_ok;
+            unsigned flipped;
+            const unsigned v = fec_decode_code(llr + k * FEC_SYMS, code, q, lane, sh_l[w], sh_dec[w], sh_u[w], sh_crc,
+                                               crc_ok, flipped);
+            const unsigned n = fec_code_coded(code);
+            if (best_n == 0u || (crc_ok && !best_ok) || (crc_ok == best_ok && flipped * best_n < best_flipped * n)) {
+                best_v = v;
+                best_ok = crc_ok;
+                best_flipped = flipped;
+                best_n = n;
+            }
+            __syncwarp();                                                  // L and sh_u are reused by the next code
+        }
+        if (lane < 12) reinterpret_cast<unsigned *>(out + k)[lane] = best_v;
     }
 }
 
@@ -445,6 +497,14 @@ cudaError_t launch_packet_decode_ex(const float *llr, const sc_packet_result *pa
                                     sc_packet_payload_ex *out, cudaStream_t st) {
     packet_code_viterbi_kernel<<<fec_grid(capacity, FEC_WARPS, 148 * 16), 32 * FEC_WARPS, 0, st>>>(
         reinterpret_cast<const float2 *>(llr), packets, capacity, n_found, stream_code, n_streams, out);
+    g_launch_count++;
+    return cudaGetLastError();
+}
+
+cudaError_t launch_packet_decode_blind(const float *llr, long capacity, const unsigned long long *n_found,
+                                       unsigned code_mask, sc_packet_payload_ex *out, cudaStream_t st) {
+    packet_blind_decode_kernel<<<fec_grid(capacity, FEC_WARPS, 148 * 16), 32 * FEC_WARPS, 0, st>>>(
+        reinterpret_cast<const float2 *>(llr), capacity, n_found, code_mask, out);
     g_launch_count++;
     return cudaGetLastError();
 }

@@ -152,6 +152,8 @@ cudaError_t launch_packet_encode_ex(const uint8_t *payload, long n_streams, int 
 cudaError_t launch_packet_decode_ex(const float *llr, const sc_packet_result *packets, long capacity,
                                     const unsigned long long *n_found, const uint8_t *stream_code, long n_streams,
                                     sc_packet_payload_ex *out, cudaStream_t st);
+cudaError_t launch_packet_decode_blind(const float *llr, long capacity, const unsigned long long *n_found,
+                                       unsigned code_mask, sc_packet_payload_ex *out, cudaStream_t st);
 
 // sc_tx_kernels.cu
 struct TxArgs {

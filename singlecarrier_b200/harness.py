@@ -37,6 +37,7 @@ class Workload:
     channel: Optional[dict] = None   # the per-stream channel parameter tensors that were applied
     payload: Optional["object"] = None   # CUDA uint8 [n_streams, n_packets, 27] when the packets carry coded payloads
     stream_code: Optional["object"] = None   # CUDA uint8 [n_streams] with per-stream code rates (payload [.., 41])
+    packet_code: Optional["object"] = None   # CUDA uint8 [n_streams, n_packets] with per-packet code rates (the same)
 
 
 def awgn_sigma(ebn0_db, torch):
@@ -47,7 +48,7 @@ def awgn_sigma(ebn0_db, torch):
 
 
 def synthesize(bank: ModemBank, samples_per_stream: int, seed: int, *, config: int, gap: int = REFERENCE_GAP,
-               ebn0_db=None, payload=None, stream_code=None) -> Workload:
+               ebn0_db=None, payload=None, stream_code=None, packet_code=None) -> Workload:
     """config 2: clean channel, random df/phase, lead-in 80+5m (preamble lands on decimated index m).
     config 3: + AWGN at ebn0_db[s] (default: 13 points 0..12 dB, striped by stream index).
     config 4: bench workload (config 3 channel, random lead-in).
@@ -55,7 +56,9 @@ def synthesize(bank: ModemBank, samples_per_stream: int, seed: int, *, config: i
     payload: None (random bits), or CUDA uint8 [n_streams, n_packets, 27]: the packets carry these payloads through the
     packet code (sc_packet_encode_dev); n_packets must be the number the stream's length gives.
     stream_code: None, or CUDA uint8 [n_streams]: each stream's code rate; payload is then [n_streams, n_packets, 41]
-    and goes through sc_packet_encode_ex_dev."""
+    and goes through sc_packet_encode_ex_dev.
+    packet_code: None, or CUDA uint8 [n_streams, n_packets]: each packet's code rate (not with stream_code); payload is
+    [n_streams, n_packets, 41] and goes through sc_packet_encode_ex_dev with one packet per stream."""
     import torch
     dev = torch.device("cuda", bank.device)
     n = bank.n_streams
@@ -88,18 +91,24 @@ def synthesize(bank: ModemBank, samples_per_stream: int, seed: int, *, config: i
     if payload is None:
         bank.tx_packets_dev(out, n_packets, gap_samples=gap, seed=seed, bits_out=bits, lead_in=lead, channel=ch)
     else:
-        width = PAYLOAD_BYTES if stream_code is None else PAYLOAD_MAX
+        assert stream_code is None or packet_code is None, "stream_code and packet_code are exclusive"
+        width = PAYLOAD_BYTES if stream_code is None and packet_code is None else PAYLOAD_MAX
         assert tuple(payload.shape) == (n, n_packets, width) and payload.dtype == torch.uint8, "payload shape"
         payload = payload.to(dev).contiguous()
-        if stream_code is None:
-            bank.packet_encode(payload, bits)
-        else:
+        if stream_code is not None:
             stream_code = stream_code.to(dev, torch.uint8).contiguous()
             assert stream_code.numel() == n, "stream_code shape"
             bank.packet_encode_ex(payload, stream_code, bits)
+        elif packet_code is not None:
+            packet_code = packet_code.to(dev, torch.uint8).contiguous()
+            assert tuple(packet_code.shape) == (n, n_packets), "packet_code shape"
+            # each packet a stream of its own: the bits land in the [n_streams][n_packets][8][62] layout all the same
+            bank.packet_encode_ex(payload.view(n * n_packets, 1, PAYLOAD_MAX), packet_code.view(-1), bits)
+        else:
+            bank.packet_encode(payload, bits)
         bank.tx_packets_dev(out, n_packets, gap_samples=gap, seed=seed, bits=bits, lead_in=lead, channel=ch)
     torch.cuda.synchronize(dev)
-    return Workload(out, bits, lead, gap, eb, n_packets, ch, payload, stream_code)
+    return Workload(out, bits, lead, gap, eb, n_packets, ch, payload, stream_code, packet_code)
 
 
 def demodulate(bank: ModemBank, samples, n_frames: int):
@@ -229,53 +238,76 @@ def packet_fec(packets, n_found: int, decoded, res, n_frames: int, wl: Workload,
 
     A workload with per-stream codes (wl.stream_code) takes the sc_packet_payload_ex records (PAYLOAD_EX_DTYPE) of
     sc_packet_decode_ex_dev: the payloads compare over the first payload_bytes(code) bytes, raw errors count over the
-    code's N transmitted positions only, and payload_bytes (the sum of the payload bytes of correct records) is added."""
+    code's N transmitted positions only, and payload_bytes (the sum of the payload bytes of correct records) is added.
+
+    A workload with per-packet codes (wl.packet_code, records of sc_packet_decode_blind_dev) does the same with the
+    code of the aligned packet j; correct also needs the record's code to be that code, and wrong_code (aligned records
+    whose CRC passes at another code, counted in undetected as well) is added."""
     assert wl.payload is not None, "the workload carries no coded payload"
-    coded = wl.stream_code is not None
+    per_packet = wl.packet_code is not None
+    coded = wl.stream_code is not None or per_packet
     pay = _host(wl.payload).reshape(-1, wl.n_packets, PAYLOAD_MAX if coded else PAYLOAD_BYTES)
     pk = _host(packets).view(PACKET_DTYPE).reshape(-1)
     dec = _host(decoded).view(PAYLOAD_EX_DTYPE if coded else PAYLOAD_DTYPE).reshape(-1)
     kept = min(int(n_found), pk.size, dec.size)
     pk, dec = pk[:kept], dec[:kept]
+    s, j, ok, al = packet_alignment(pk, kept, res, n_frames, wl)
+    grp = np.zeros(pay.shape[0], np.int64) if group is None else _host(group).astype(np.int64)
+    g = grp[s]
+    ok &= (g >= 0) & (g < n_groups)
+    al &= ok
+    crc = dec["crc_ok"] != 0
+    # hard decisions against the transmitted bits, packed like the records' words (bit k of word f = bit 62 f + k)
+    txw = _packed_words(wl.tx_bits)[s, j]
+    if coded:
+        code = _host(wl.packet_code).astype(np.int64)[s, j] if per_packet else _host(wl.stream_code).astype(np.int64)[s]
+        n_bytes = np.array([payload_bytes(c) for c in range(256)], np.int64)[code]
+        same = ((dec["data"] == pay[s, j]) | (np.arange(PAYLOAD_MAX) >= n_bytes[:, None])).all(axis=1)
+        mask = coded_position_masks()[np.minimum(code, 3)]
+        if per_packet:
+            wrong = dec["code"].astype(np.int64) != code
+            same &= ~wrong
+    else:
+        same = (dec["data"] == pay[s, j]).all(axis=1)
+        mask = np.array([(1 << 62) - 1] * 7 + [(1 << (PACKET_CODED_BITS - 7 * 62)) - 1], np.uint64)
+    raw = np.bitwise_count((pk["bits"] ^ txw) & mask).sum(axis=1).astype(np.int64)
+    names = ("records", "aligned", "crc_ok", "correct", "undetected", "raw_errors", "raw_packet_errors")
+    names += (("payload_bytes",) if coded else ()) + (("wrong_code",) if per_packet else ())
+    out = {k: np.zeros(n_groups, np.int64) for k in names}
+    rows = [("records", ok, None), ("aligned", al, None), ("crc_ok", al & crc, None),
+            ("correct", al & crc & same, None), ("undetected", al & crc & ~same, None),
+            ("raw_errors", al, raw), ("raw_packet_errors", al & (raw > 0), None)]
+    if coded:
+        rows.append(("payload_bytes", al & crc & same, n_bytes))
+    if per_packet:
+        rows.append(("wrong_code", al & crc & wrong, None))
+    for name, m, w in rows:
+        np.add.at(out[name], g[m], 1 if w is None else w[m])
+    return out
+
+
+def packet_alignment(packets, n_found: int, res, n_frames: int, wl: Workload):
+    """The rule of sc_packet_ber_stats_dev for the first min(n_found, len) packet records: their stream s and packet j
+    (int64, both 0 and clipped into range where not counted), counted (a stream in range and a call 2..n_frames-1) and
+    aligned (counted, and within +-10 samples of packet j of its stream; j from grid_sample when it is not 0, else from
+    call index, max_index and rx_timing)."""
+    pk = _host(packets).view(PACKET_DTYPE).reshape(-1)
+    pk = pk[:min(int(n_found), pk.size)]
+    n_streams = wl.tx_bits.shape[0]
     r = _host(res)
-    n_streams = pay.shape[0]
     timing = r.view(np.uint8).reshape(n_streams, -1, 32)[:, :, 20:22].copy().view("<i2")[..., 0].astype(np.int64)
     lead = _host(wl.lead).astype(np.int64)
-    grp = np.zeros(n_streams, np.int64) if group is None else _host(group).astype(np.int64)
     s = pk["stream"].astype(np.int64)
     n = pk["call_index"].astype(np.int64)
     ok = (s >= 0) & (s < n_streams) & (n >= 2) & (n < n_frames)
     s, n = np.where(ok, s, 0), np.where(ok, n, 2)
-    g = grp[s]
-    ok &= (g >= 0) & (g < n_groups)
     gs = pk["grid_sample"].astype(np.int64)
     pos = np.where(gs != 0, gs, (n - 2) * FRAME_SIZE + 5 * pk["max_index"].astype(np.int64) + timing[s, n - 2]) \
         - GROUP_DELAY - lead[s]
     period = FRAME_SIZE + wl.gap
     j = np.floor_divide(pos + period // 2, period)
     al = ok & (j >= 0) & (j < wl.n_packets) & (np.abs(pos - j * period) <= 10)
-    j = np.clip(j, 0, wl.n_packets - 1)
-    crc = dec["crc_ok"] != 0
-    # hard decisions against the transmitted bits, packed like the records' words (bit k of word f = bit 62 f + k)
-    txw = _packed_words(wl.tx_bits)[s, j]
-    if coded:
-        n_bytes = np.array([payload_bytes(c) for c in range(256)], np.int64)[_host(wl.stream_code).astype(np.int64)[s]]
-        same = ((dec["data"] == pay[s, j]) | (np.arange(PAYLOAD_MAX) >= n_bytes[:, None])).all(axis=1)
-        mask = coded_position_masks()[np.minimum(_host(wl.stream_code).astype(np.int64)[s], 3)]
-    else:
-        same = (dec["data"] == pay[s, j]).all(axis=1)
-        mask = np.array([(1 << 62) - 1] * 7 + [(1 << (PACKET_CODED_BITS - 7 * 62)) - 1], np.uint64)
-    raw = np.bitwise_count((pk["bits"] ^ txw) & mask).sum(axis=1).astype(np.int64)
-    names = ("records", "aligned", "crc_ok", "correct", "undetected", "raw_errors", "raw_packet_errors")
-    out = {k: np.zeros(n_groups, np.int64) for k in names + (("payload_bytes",) if coded else ())}
-    rows = [("records", ok, None), ("aligned", al, None), ("crc_ok", al & crc, None),
-            ("correct", al & crc & same, None), ("undetected", al & crc & ~same, None),
-            ("raw_errors", al, raw), ("raw_packet_errors", al & (raw > 0), None)]
-    if coded:
-        rows.append(("payload_bytes", al & crc & same, n_bytes))
-    for name, m, w in rows:
-        np.add.at(out[name], g[m], 1 if w is None else w[m])
-    return out
+    return s, np.clip(j, 0, wl.n_packets - 1), ok, al
 
 
 def coded_position_masks() -> np.ndarray:

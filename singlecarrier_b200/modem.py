@@ -326,6 +326,17 @@ class ModemBank:
         check(lib.sc_packet_decode_ex_dev(self.device, llr.data_ptr(), packets.data_ptr(), capacity, n_found.data_ptr(),
                                           stream_code.data_ptr(), stream_code.numel(), out.data_ptr(), stream))
 
+    def packet_decode_blind(self, llr, n_found, out, code_mask: int = 7, stream: int = 0) -> None:
+        """Viterbi-decode the records' LLRs (CUDA float32, 496 per record, its size sets the capacity) at every code of
+        code_mask (bit c for code c) and keep, per record, the best whose CRC passes (fewest flipped bits per
+        transmitted bit, then the lower code), or the best of all when none passes, into out (CUDA uint8
+        [capacity * 48], viewable as PAYLOAD_EX_DTYPE) for the first min(n_found, capacity) records
+        (sc_packet_decode_blind_dev).  No code table is needed: each record's code field says which code it is."""
+        capacity = llr.numel() * llr.element_size() // (PACKET_BITS * 4)
+        assert out.numel() * out.element_size() >= capacity * PAYLOAD_EX_DTYPE.itemsize, "capacity"
+        check(lib.sc_packet_decode_blind_dev(self.device, llr.data_ptr(), capacity, n_found.data_ptr(), int(code_mask),
+                                             out.data_ptr(), stream))
+
     def transfer_bytes(self):
         out = (C.c_uint64 * 2)()
         check(lib.sc_transfer_bytes(self._h, out))
