@@ -143,17 +143,17 @@ def grids64(x: np.ndarray, pk, foffset: float = 0.0, wide: bool = False) -> np.n
 
 
 # ---- loop-back streams with known bits ----------------------------------------------------------------------------
-def loop_streams(oracle, rng, n_streams, n_packets, sigma=0.0, gap=903):
-    """Loop-back streams from the spec's packet-mode transmitter (pyoracle.ext_tx_packet, scrambled): random lead-in,
-    gap zeros after every packet, AWGN of sigma LSB -> (int16 [n, n_frames * 1880], tx bits uint8 [n, n_packets, 496],
-    packet starts int [n, n_packets])"""
+def loop_streams(oracle, rng, n_streams, n_packets, sigma=0.0, gap=903, lead_max=2000):
+    """Loop-back streams from the spec's packet-mode transmitter (pyoracle.ext_tx_packet, scrambled): random lead-in
+    of 0 .. lead_max - 1 samples, gap zeros after every packet, AWGN of sigma LSB -> (int16 [n, n_frames * 1880],
+    tx bits uint8 [n, n_packets, 496], packet starts int [n, n_packets])"""
     total = ((n_packets * (1880 + gap) + 2000 + 2 * 1880) // 1880) * 1880
     out = np.zeros((n_streams, total), np.int16)
     txb = np.zeros((n_streams, n_packets, 496), np.uint8)
     starts = np.zeros((n_streams, n_packets), np.int64)
     for s in range(n_streams):
         st = oracle.new_state()
-        lead = int(rng.integers(0, 2000))
+        lead = int(rng.integers(0, lead_max))
         parts = [np.zeros(lead, np.int16)]
         for j in range(n_packets):
             txb[s, j] = rng.integers(0, 2, 496).astype(np.uint8)

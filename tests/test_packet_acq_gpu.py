@@ -24,13 +24,14 @@ def sc():
     return m
 
 
-def acq_streams(sc, ns, n_packets, seed, gap=903):
-    """Streams from the library's packet-mode TX and channel: offsets uniform in +-40 Hz, AWGN 0..1500 LSB, a 2-tap
-    echo on every third stream -> (int16 [ns, n], tx bits [ns, n_packets, 8, 62], lead-in [ns])"""
+def acq_streams(sc, ns, n_packets, seed, gap=903, lead_max=2783):
+    """Streams from the library's packet-mode TX and channel: lead-ins of 0 .. lead_max - 1 samples, offsets uniform in
+    +-40 Hz, AWGN 0..1500 LSB, a 2-tap echo on every third stream -> (int16 [ns, n], tx bits [ns, n_packets, 8, 62],
+    lead-in [ns])"""
     import torch
     bank = sc.ModemBank(ns, packet=True)
     g = torch.Generator(device="cuda").manual_seed(seed)
-    lead = torch.randint(0, 2783, (ns,), generator=g, device="cuda", dtype=torch.int32)
+    lead = torch.randint(0, lead_max, (ns,), generator=g, device="cuda", dtype=torch.int32)
     echo = (torch.arange(ns, device="cuda") % 3 == 0).float()
     ch = {"df_hz": (torch.rand(ns, generator=g, device="cuda") * 80 - 40).float(),
           "phi_rad": (torch.rand(ns, generator=g, device="cuda") * 6.283).float(),
